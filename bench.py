@@ -4,6 +4,8 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo (torchrun launches N ranks for N > 1)
   python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm's CPU path (oracle port)
+  python bench.py --steps K --dump-outputs DIR              # + each workload's last timed step as DIR/*.npy (seeded inputs:
+                                                            #   two builds can be compared array for array)
 
 A "step" = one pass of the hot path over one batch: HR uint8 truncation, DRCT forward (uint8 truncation fused into
 the last kernel), one scoring launch (13 SSIM window sizes + MSE + PSNR per image) and, when sharded, the NCCL
@@ -46,7 +48,12 @@ def parse():
     p.add_argument("--no-sub-workloads", action="store_true", help="skip the sub-records of the other BASELINE configs")
     p.add_argument("--cpu-sample", type=int, default=4, help="images per CPU-baseline step")
     p.add_argument("--no-cpu-baseline", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write each workload's results of its last timed step to DIR/<workload>_<array>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def synthetic_pairs(n: int, seed: int = 1234, hr: int = 128):
@@ -294,6 +301,22 @@ WORKLOADS = {
 }
 
 
+DUMP_SR_SAMPLES = 1 << 20                      # SR pixels kept per workload (4 MiB as float32)
+
+
+def dump_outputs(dump_dir: str, workload: str, scores: np.ndarray, sr_u8: torch.Tensor) -> None:
+    """What the evaluator handed back in the last timed step: the fp64 score table [images, n_ws + 2] (ordered by image id)
+    and a fixed sample (seed 0, ascending flat NHWC indices) of the uint8 SR pixels as float32."""
+    os.makedirs(dump_dir, exist_ok=True)
+    name = workload.replace("-", "_")
+    np.save(os.path.join(dump_dir, f"{name}_scores.npy"), np.asarray(scores, dtype=np.float64))
+    flat = sr_u8.reshape(-1)
+    n = flat.numel()
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SR_SAMPLES), replace=False))
+    sample = flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy()
+    np.save(os.path.join(dump_dir, f"{name}_sr_sample.npy"), sample)
+
+
 def build_model(mods, workload: str, batch: int, dev):
     model_kind, lr_side, _, _, _, _ = WORKLOADS[workload]
     main_mod = mods["main"]
@@ -315,7 +338,7 @@ def build_model(mods, workload: str, batch: int, dev):
 
 
 def run_workload(mods, workload: str, B: int, steps: int, warmup: int, dev, rank: int, world: int, local_rank: int,
-                 with_roofline: bool = True) -> dict:
+                 with_roofline: bool = True, dump_dir: str = None) -> dict:
     """One workload, timed twice: `value` with the inputs resident in HBM (CUDA events, L2 flushed between steps, max over
     ranks) and `e2e` through the public evaluator API from pinned host tensors (H2D copies + D2H read of the score table in
     the timed region).  Returns the fields of a bench record."""
@@ -370,6 +393,9 @@ def run_workload(mods, workload: str, B: int, steps: int, warmup: int, dev, rank
         barrier()
     ms = e0.elapsed_time(e1)
     launches = ops.LAUNCHES - launches0
+    if dump_dir is not None and rank == 0:
+        table = evaluate.scores_table(out, world * B) if world > 1 else out.cpu().numpy()
+        dump_outputs(dump_dir, workload, table, ev.last_sr_u8)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -498,21 +524,22 @@ def main():
     mods = {n: importlib.import_module(f"{PKG}.{n}") for n in ("ops", "drct", "drn", "evaluate", "metrics", "main")}
 
     B = args.batch if args.batch is not None else WORKLOADS[args.workload][2]
-    head = run_workload(mods, args.workload, B, args.steps, args.warmup, dev, rank, world, local_rank)
+    head = run_workload(mods, args.workload, B, args.steps, args.warmup, dev, rank, world, local_rank,
+                        dump_dir=args.dump_outputs)
 
-    # ---- the other BASELINE configurations ride in the same line as sub-records (same timing rules, fewer steps)
+    # ---- the other BASELINE configurations ride in the same line as sub-records (same timing rules)
     subs = {}
     if not args.no_sub_workloads:
-        sub_steps = max(2, min(args.steps, 5))
         for name, key in (("drn-l", "drn_l_b64"), ("drct-l-64", "drct_l_64px_b128"), ("drct-l", "drct_l_b256")):
             if name == args.workload:
                 continue
-            r = run_workload(mods, name, WORKLOADS[name][2], sub_steps, 3, dev, rank, world, local_rank)
+            r = run_workload(mods, name, WORKLOADS[name][2], args.steps, 3, dev, rank, world, local_rank,
+                             dump_dir=args.dump_outputs)
             r.pop("clocks", None)
             subs[key] = r
         if world > 1 and args.workload == "drct-l" and 256 % world == 0:
             # strong scaling: the SAME 256 images split over the ranks (SURVEY.md 8d)
-            r = run_workload(mods, "drct-l", 256 // world, sub_steps, 3, dev, rank, world, local_rank, with_roofline=False)
+            r = run_workload(mods, "drct-l", 256 // world, args.steps, 3, dev, rank, world, local_rank, with_roofline=False)
             subs["strong_scaling_global256"] = {"value": r["value"], "unit": "images/s", "ms_per_step": r["ms_per_step"],
                                                 "batch_per_gpu": 256 // world, "global_batch": 256, "e2e": r["e2e"],
                                                 "scaling": "strong"}
