@@ -258,20 +258,9 @@ extern "C" int adsr_swin_mlp_conv_res_bf16(const void* y, int64_t ldy, int M, in
 static long long* g_attn_trace = nullptr;
 extern "C" void adsr_debug_set_attn_trace(void* device_buffer) { g_attn_trace = static_cast<long long*>(device_buffer); }
 
-extern "C" void adsr_debug_set_mlp_acc1(int max_buffers) { g_mlp_acc1_max = max_buffers; }
-extern "C" void adsr_debug_set_attn_pipe(int enabled) { g_attn_pipe = enabled; }
-
-static int g_swin_attn2 = 1;
-extern "C" void adsr_debug_set_swin_attn2(int enabled) { g_swin_attn2 = enabled; }
-
 extern "C" int adsr_swin_attn_mode(int C, int heads, int head_dim_padded, int allow_proj) {
     SwinAttnParams p{};
     return swin_attn_plan(p, C, heads, head_dim_padded, allow_proj);
-}
-
-extern "C" int adsr_swin_attn2_covers(int C, int heads, int head_dim_padded) {
-    SwinAttnParams p{};
-    return g_swin_attn2 ? swin_attn2_plan(p, C, heads, head_dim_padded) : 0;
 }
 
 extern "C" int adsr_swin_attn_bf16(const void* x, int64_t ldx, int B, int H, int W, int C, int shift, int heads, int head_dim,
@@ -285,9 +274,7 @@ extern "C" int adsr_swin_attn_bf16(const void* x, int64_t ldx, int B, int H, int
         w1_packed == nullptr || bias_qkv == nullptr || colsum_qkv == nullptr || bias_table == nullptr)
         return ADSR_ERR_BAD_SHAPE;
     SwinAttnParams p{};
-    // attention only: the two-heads-in-flight kernel where its two TMEM regions / k|v panel sets fit
-    const bool two = fuse_proj == 0 && g_swin_attn2 != 0 && swin_attn2_plan(p, C, heads, head_dim_padded) == 1;
-    const int mode = two ? 1 : swin_attn_plan(p, C, heads, head_dim_padded, fuse_proj);
+    const int mode = swin_attn_plan(p, C, heads, head_dim_padded, fuse_proj);
     if (mode == 0 || (fuse_proj != 0) != (mode == 2)) return ADSR_ERR_BAD_SHAPE;
     if (mode == 2 && (w2_packed == nullptr || bias_proj == nullptr)) return ADSR_ERR_BAD_SHAPE;
     if (stats_out != nullptr && (mode != 2 || stats_out_slot0 >= stats_out_stride)) return ADSR_ERR_BAD_SHAPE;
@@ -303,7 +290,6 @@ extern "C" int adsr_swin_attn_bf16(const void* x, int64_t ldx, int B, int H, int
     p.scale_log2e = (1.0f / sqrtf(static_cast<float>(head_dim))) * 1.4426950408889634f;
     p.B = B; p.H = H; p.W = W; p.shift = shift;
     p.trace = g_attn_trace;
-    if (two) return launch_swin_attn2(p, num_sms, static_cast<cudaStream_t>(stream));
     return launch_swin_attn(p, num_sms, static_cast<cudaStream_t>(stream));
 }
 

@@ -158,8 +158,6 @@ struct SwinMlpParams {
     int adj_stats_vec4;   // the two slots of a row form one aligned 16-byte store (set by the launcher)
 };
 int swin_mlp_fixed_smem_bytes(int hidden_padded, int n2);
-extern int g_mlp_acc1_max;
-extern int g_attn_pipe;
 int launch_swin_mlp(SwinMlpParams& p, const void* y, long long ldy, void* z, long long ldz, int num_sms, cudaStream_t stream);
 
 // ---- fused attention half of a Swin block (swin_attn.cu)
@@ -204,9 +202,6 @@ int encode_tmap_nhwc_box3_bf16(CUtensorMap* map, const void* base, int B, int H,
                                int box_h);
 int swin_attn_plan(SwinAttnParams& p, int C, int nH, int hdp, int allow_proj);   // 0 = not covered, 1 = qkv + attention, 2 = + proj
 int launch_swin_attn(SwinAttnParams& p, int num_sms, cudaStream_t stream);
-// two heads in flight (swin_attn2.cu): qkv + attention only, the 16 epilogue warps split into two groups that own the even / odd heads
-int swin_attn2_plan(SwinAttnParams& p, int C, int nH, int hdp);                   // 1 = covered, 0 = use swin_attn.cu
-int launch_swin_attn2(SwinAttnParams& p, int num_sms, cudaStream_t stream);
 
 // ---- halo-tile 3x3 conv with resident weights (conv_halo.cu)
 struct ConvHaloParams {

@@ -998,8 +998,6 @@ int round16(int v) { return (v + 15) / 16 * 16; }
 
 }  // namespace
 
-int g_attn_pipe = 1;                           // debug switch (adsr_debug_set_attn_pipe): 0 = heads one after the other
-
 // Static plan of the fused kernel for one block shape.  Returns 0 = not covered (use the separate kernels),
 // 1 = qkv + attention fused (out = attention rows [M, nH * hdp], proj by the row-tile GEMM), 2 = whole attention half.
 int swin_attn_plan(SwinAttnParams& p, int C, int nH, int hdp, int allow_proj) {
@@ -1023,7 +1021,7 @@ int swin_attn_plan(SwinAttnParams& p, int C, int nH, int hdp, int allow_proj) {
     p.early_setup = p.col_acc >= 0 ? 1 : 0;
     // ... and then the heads are pipelined: the conversion of head h + 1 runs under P V of head h (second v panel), the
     // normalisation of head h under S of head h + 1
-    p.pipe = (p.col_acc >= 0 && g_attn_pipe != 0) ? 1 : 0;
+    p.pipe = p.col_acc >= 0 ? 1 : 0;
     // a [3 hdp x 64] qkv slab is one ring slot and one issue step (every step costs ~400 cycles of wait / commit bookkeeping on
     // top of its MMAs, so steps are kept as large as the MMA N limit of 256 allows); 3 hdp > 256: two N pieces
     const int n3 = 3 * hdp;

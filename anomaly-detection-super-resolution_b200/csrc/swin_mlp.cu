@@ -21,8 +21,6 @@
 
 namespace adsr {
 
-int g_mlp_acc1_max = 3;                        // debug switch (adsr_debug_set_mlp_acc1): 2 = never use a third chunk accumulator
-
 namespace {
 
 constexpr int kEpiWarps = 16;                 // warps 0..15: epilogue (TMEM lane quadrant = warp % 4)
@@ -713,7 +711,7 @@ int launch_swin_mlp(SwinMlpParams& p, const void* y, long long ldy, void* z, lon
     if (p.n2 + 2 * p.hc > 512 || p.acc1_col[0] < (p.fuse_adj ? 2 : 1) * p.n2 || p.acc1_col[1] < p.acc1_col[0] + p.hc || p.acc1_col[1] + p.hc > 512)
         return ADSR_ERR_BAD_SHAPE;
     p.acc1_col[2] = p.acc1_col[1] + p.hc;
-    p.n_acc1 = (p.acc1_col[2] + p.hc <= 512 && g_mlp_acc1_max >= 3) ? 3 : 2;
+    p.n_acc1 = p.acc1_col[2] + p.hc <= 512 ? 3 : 2;
     if (p.ks1 <= 0 || p.ks1 > 5 || p.k1steps <= 4 * (p.ks1 - 1) || p.k1steps > 4 * p.ks1) return ADSR_ERR_BAD_SHAPE;
     if (p.w1_slots < 2 || p.w1_slots > 8 || p.w2_slots < 2 || p.w2_slots > 8 || (p.w1_slot_bytes % 1024) || (p.w2_slot_bytes % 1024))
         return ADSR_ERR_BAD_SHAPE;

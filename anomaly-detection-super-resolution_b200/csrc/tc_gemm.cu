@@ -12,13 +12,12 @@
 // (folded LayerNorm, bias, GELU / LeakyReLU / ReLU, alpha, residual), rounds once to bf16 and can emit the row's
 // (sum, sum of squares) for the NEXT LayerNorm.
 //
-// Two epilogue variants (template EPI_TMA):
-//   * TMA epilogue (row-major outputs at 16-byte aligned columns): every warp owns a double-buffered 32x32 bf16
-//     staging tile in the 64-byte-swizzle layout.  The residual tile is TMA-LOADED into it (one chunk ahead), the row
-//     owner adds it from shared memory and writes the result back in place, one lane TMA-STORES the box.  No address
-//     arithmetic, predicates or global load/store instructions in the hot loop; M / N edges are clipped by the TMA unit.
-//   * manual epilogue (PixelShuffle(2) stores, slab slices at 8-byte aligned columns): staged tile, coalesced 64-byte
-//     row segments written with ordinary stores, residual added in the write-out mapping.
+// This kernel has the TMA epilogue (row-major outputs with a residual, at 16-byte aligned columns, BN % 32 == 0): every
+// warp owns a double-buffered 32x32 bf16 staging tile in the 64-byte-swizzle layout.  The residual tile is TMA-LOADED
+// into it (one chunk ahead), the row owner adds it from shared memory and writes the result back in place, one lane
+// TMA-STORES the box.  No address arithmetic, predicates or global load/store instructions in the hot loop; M / N edges
+// are clipped by the TMA unit.  Every other output (no residual, PixelShuffle(2) stores, slab slices at 8-byte aligned
+// columns) goes to the manual-epilogue kernel of tc_gemm_manual.cu; launch_tc_gemm below picks one of the two.
 //
 // Replaces (reference call sites): nn.Linear qkv/proj/fc1/fc2 (src/drct.py:278,300,185-188) with the LayerNorms in front
 // of qkv / fc1 (src/drct.py:481,510), the 1x1 adjust convs (src/drct.py:334-374, 389-393), conv_after_body /
@@ -98,13 +97,7 @@ __device__ __forceinline__ void bulk_wait_read() {      // <= N most recent grou
 }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
-__device__ __forceinline__ uint32_t add_bf16x2_f32(uint32_t a, uint32_t b, bool lo_ok, bool hi_ok) {
-    const float l = bf16_lo(a) + (lo_ok ? bf16_lo(b) : 0.f);
-    const float h = bf16_hi(a) + (hi_ok ? bf16_hi(b) : 0.f);
-    return pack_bf16x2(l, h);
-}
-
-template <int ACT, bool EPI_TMA, bool STATS>
+template <int ACT, bool STATS>
 __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_constant__ TcGemmParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     uint8_t* smem_a = smem;
@@ -242,7 +235,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
             mbar_arrive_expect_tx(bar, kStageTileBytes);
             tma_load_2d(stg + bufi * kStageTileBytes, &p.tmap_res, nt * p.BN + ch * 32, mt * 128 + quad * 32, bar);
         };
-        if (EPI_TMA && has_res && lane == 0) {
+        if (has_res && lane == 0) {
             int it0, ch0;
             if (next_chunk(0, half, it0, ch0)) issue_res_load(it0, ch0, 0);
         }
@@ -279,50 +272,28 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
                 const int c0 = ch * 32;
                 const int n0 = n_base + c0;
                 if (n0 >= n_lim) continue;                      // warp-uniform: nothing of this chunk is stored
-                const bool wide = c0 + 32 <= p.BN;             // BN % 32 == 16 (manual epilogue only): 16-column tail
                 uint8_t* sbuf = stg + (g & 1) * kStageTileBytes;
                 const uint32_t sbuf_row = smem_u32(sbuf) + static_cast<uint32_t>(lane * 64);
 
-                // manual epilogue: residual prefetch in the coalesced (write-out) mapping
-                uint4 rres[4];
-                if (!EPI_TMA && has_res) {
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int r = row0 + i * 8 + (lane >> 2);
-                        const int col = n0 + (lane & 3) * 8;
-                        rres[i] = (r < p.M && col < n_lim)
-                                      ? __ldg(reinterpret_cast<const uint4*>(p.res + static_cast<long long>(r) * p.ldres + col))
-                                      : make_uint4(0, 0, 0, 0);
-                    }
-                }
                 uint32_t raw[32];
                 __syncwarp();                                   // tcgen05.ld is .sync.aligned
-                if (wide) {
-                    tmem_ld32(taddr + static_cast<uint32_t>(c0), raw);
-                } else {
-                    uint32_t lo[16];
-                    tmem_ld16(taddr + static_cast<uint32_t>(c0), lo);
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) { raw[j] = lo[j]; raw[16 + j] = 0; }
-                }
+                tmem_ld32(taddr + static_cast<uint32_t>(c0), raw);
                 tmem_ld_wait();
 
-                if (EPI_TMA) {
-                    if (has_res) {
-                        // prefetch the residual tile of my NEXT chunk into the other staging buffer; the store that last
-                        // used that buffer (chunk g-1) must have finished reading it
-                        if (lane == 0) {
-                            int it2, ch2;
-                            if (next_chunk(it, ch + 2, it2, ch2)) {
-                                bulk_wait_read<0>();
-                                issue_res_load(it2, ch2, (g + 1) & 1);
-                            }
+                if (has_res) {
+                    // prefetch the residual tile of my NEXT chunk into the other staging buffer; the store that last
+                    // used that buffer (chunk g-1) must have finished reading it
+                    if (lane == 0) {
+                        int it2, ch2;
+                        if (next_chunk(it, ch + 2, it2, ch2)) {
+                            bulk_wait_read<0>();
+                            issue_res_load(it2, ch2, (g + 1) & 1);
                         }
-                        mbar_wait(&bars->res_full[ew][g & 1], static_cast<uint32_t>(g >> 1) & 1);   // my residual tile landed
-                    } else {
-                        if (lane == 0) bulk_wait_read<1>();     // the store of chunk g-2 has finished reading this buffer
-                        __syncwarp();
                     }
+                    mbar_wait(&bars->res_full[ew][g & 1], static_cast<uint32_t>(g >> 1) & 1);   // my residual tile landed
+                } else {
+                    if (lane == 0) bulk_wait_read<1>();         // the store of chunk g-2 has finished reading this buffer
+                    __syncwarp();
                 }
 
                 // ---- fp32 math per element, one rounding to bf16; logical 16-byte chunk j of my row holds columns 8j..8j+7
@@ -330,7 +301,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     uint32_t rw[4] = {0u, 0u, 0u, 0u};
-                    if (EPI_TMA && has_res) {
+                    if (has_res) {
                         asm volatile("ld.shared.v4.b32 {%0,%1,%2,%3}, [%4];"
                                      : "=r"(rw[0]), "=r"(rw[1]), "=r"(rw[2]), "=r"(rw[3])
                                      : "r"(sbuf_row + static_cast<uint32_t>((j ^ wsw) << 4)));
@@ -352,7 +323,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
                             v[e] = apply_act<ACT>(a[e] + bv[e], p.slope) * p.alpha;
-                            if (EPI_TMA && has_res) {
+                            if (has_res) {
                                 const uint32_t w2 = rw[2 * h2 + (e >> 1)];
                                 v[e] += (e & 1) ? bf16_hi(w2) : bf16_lo(w2);
                             }
@@ -360,24 +331,9 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
                             //  residual make them exact zeros, and act(0) = 0 for every activation used)
                             if (STATS) { st_sum += v[e]; st_sq = fmaf(v[e], v[e], st_sq); }
                         }
-                        if (p.out_mode == ADSR_OUT_ROWS) {
-                            pk[2 * q4] = pack_bf16x2(v[0], v[1]);
-                            pk[2 * q4 + 1] = pack_bf16x2(v[2], v[3]);
-                        } else {
-                            // PixelShuffle(2): column 4c+sub -> staging position sub*8 + c (8 channels per chunk);
-                            // permuted below from the float values kept in raw[]
-                            raw[4 * q4 + 0] = __float_as_uint(v[0]); raw[4 * q4 + 1] = __float_as_uint(v[1]);
-                            raw[4 * q4 + 2] = __float_as_uint(v[2]); raw[4 * q4 + 3] = __float_as_uint(v[3]);
-                        }
+                        pk[2 * q4] = pack_bf16x2(v[0], v[1]);
+                        pk[2 * q4 + 1] = pack_bf16x2(v[2], v[3]);
                     }
-                }
-                if (p.out_mode != ADSR_OUT_ROWS) {
-#pragma unroll
-                    for (int sub = 0; sub < 4; ++sub)
-#pragma unroll
-                        for (int c = 0; c < 4; ++c)
-                            pk[sub * 4 + c] = pack_bf16x2(__uint_as_float(raw[(2 * c) * 4 + sub]),
-                                                          __uint_as_float(raw[(2 * c + 1) * 4 + sub]));
                 }
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -386,57 +342,11 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
                                  : "memory");
                 }
 
-                if (EPI_TMA) {
-                    fence_proxy_async_smem();                   // my st.shared must be visible to the TMA (async proxy)
-                    __syncwarp();
-                    if (lane == 0) {
-                        tma_store_2d(&p.tmap_out, sbuf, p.ocol0 + n0, row0);   // rows >= M / columns >= ocol0+n_store clipped
-                        bulk_commit();
-                    }
-                } else {
-                    __syncwarp();
-                    // ---- coalesced write-out: lane -> (row = i*8 + lane/4, 16-byte chunk = lane%4)
-                    const bool st16 = (p.ocol0 & 7) == 0;
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int rl = i * 8 + (lane >> 2);
-                        const int cc = lane & 3;
-                        const uint4 val = *reinterpret_cast<const uint4*>(sbuf + rl * 64 + ((cc ^ ((rl >> 1) & 3)) << 4));
-                        const int r = row0 + rl;
-                        if (r >= p.M) continue;
-                        if (p.out_mode == ADSR_OUT_ROWS) {
-                            const int col = n0 + cc * 8;
-                            if (col >= n_lim) continue;
-                            uint4 o = val;
-                            if (has_res) {
-                                o.x = add_bf16x2_f32(val.x, rres[i].x, col + 0 < p.N, col + 1 < p.N);
-                                o.y = add_bf16x2_f32(val.y, rres[i].y, col + 2 < p.N, col + 3 < p.N);
-                                o.z = add_bf16x2_f32(val.z, rres[i].z, col + 4 < p.N, col + 5 < p.N);
-                                o.w = add_bf16x2_f32(val.w, rres[i].w, col + 6 < p.N, col + 7 < p.N);
-                            }
-                            __nv_bfloat16* dst = p.out + static_cast<long long>(r) * p.ldo + p.ocol0 + col;
-                            if (col + 8 > n_lim) {              // n_store % 8 == 4: only the first 4 columns belong to us
-                                reinterpret_cast<uint2*>(dst)[0] = make_uint2(o.x, o.y);
-                            } else if (st16) {
-                                *reinterpret_cast<uint4*>(dst) = o;
-                            } else {                            // slab slices start at 8-byte aligned columns
-                                reinterpret_cast<uint2*>(dst)[0] = make_uint2(o.x, o.y);
-                                reinterpret_cast<uint2*>(dst)[1] = make_uint2(o.z, o.w);
-                            }
-                        } else {
-                            // staging chunk cc = sub-pixel (i2, j2); 8 channels n0/4 .. n0/4+7
-                            const int hw = p.Hout * p.Wout;
-                            const int b = r / hw;
-                            const int rem = r - b * hw;
-                            const int y = rem / p.Wout;
-                            const int x = rem - y * p.Wout;
-                            const int i2 = cc >> 1, j2 = cc & 1;
-                            __nv_bfloat16* dst = p.out +
-                                ((static_cast<long long>(b) * (2 * p.Hout) + 2 * y + i2) * (2 * p.Wout) + 2 * x + j2) * p.ldo + (n0 >> 2);
-                            *reinterpret_cast<uint4*>(dst) = val;
-                        }
-                    }
-                    __syncwarp();                               // the staging tile is reused two chunks later
+                fence_proxy_async_smem();                       // my st.shared must be visible to the TMA (async proxy)
+                __syncwarp();
+                if (lane == 0) {
+                    tma_store_2d(&p.tmap_out, sbuf, p.ocol0 + n0, row0);   // rows >= M / columns >= ocol0+n_store clipped
+                    bulk_commit();
                 }
                 ++g;
             }
@@ -448,7 +358,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) tc_gemm_kernel(const __grid_co
             tc_fence_before_sync();
             mbar_arrive(&bars->tmem_empty[buf]);
         }
-        if (EPI_TMA && lane == 0) bulk_wait_all();              // all my stores have left shared memory and are complete
+        if (lane == 0) bulk_wait_all();                         // all my stores have left shared memory and are complete
     } else if (warp >= 4 + kEpiWarps && !p.use_tma) {
         // ================================ conv mode: A producers (4 warps, 128 threads) ===============
         const int pw = warp - (4 + kEpiWarps);
@@ -655,10 +565,10 @@ int launch_tc_gemm(TcGemmParams& p, int num_sms, cudaStream_t stream) {
     if (!p.epi_tma) return launch_tc_gemm_manual(p, grid, stream);
     const bool st = p.stats_out != nullptr;
     switch (p.act) {
-        case ADSR_ACT_NONE: return st ? launch(tc_gemm_kernel<ADSR_ACT_NONE, true, true>) : launch(tc_gemm_kernel<ADSR_ACT_NONE, true, false>);
-        case ADSR_ACT_LRELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_LRELU, true, true>) : launch(tc_gemm_kernel<ADSR_ACT_LRELU, true, false>);
-        case ADSR_ACT_GELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_GELU, true, true>) : launch(tc_gemm_kernel<ADSR_ACT_GELU, true, false>);
-        case ADSR_ACT_RELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_RELU, true, true>) : launch(tc_gemm_kernel<ADSR_ACT_RELU, true, false>);
+        case ADSR_ACT_NONE: return st ? launch(tc_gemm_kernel<ADSR_ACT_NONE, true>) : launch(tc_gemm_kernel<ADSR_ACT_NONE, false>);
+        case ADSR_ACT_LRELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_LRELU, true>) : launch(tc_gemm_kernel<ADSR_ACT_LRELU, false>);
+        case ADSR_ACT_GELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_GELU, true>) : launch(tc_gemm_kernel<ADSR_ACT_GELU, false>);
+        case ADSR_ACT_RELU: return st ? launch(tc_gemm_kernel<ADSR_ACT_RELU, true>) : launch(tc_gemm_kernel<ADSR_ACT_RELU, false>);
     }
     return ADSR_ERR_BAD_SHAPE;
 }

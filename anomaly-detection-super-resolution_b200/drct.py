@@ -18,7 +18,6 @@ Evaluation semantics only (DropPath = identity, as `model.eval()`); see DESIGN.m
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional, Tuple
 
 import torch
@@ -28,17 +27,6 @@ from . import ops, pack
 from .pack import PackedWeight, round_up
 
 RGB_MEAN = (0.4488, 0.4371, 0.4040)   # src/drct.py:774
-_FUSED_ADJUST = os.environ.get("ADSR_FUSED_ADJUST", "1") != "0"  # A/B switch: 0 = adjust convs as separate GEMMs
-_FOLD_ADJUST5 = os.environ.get("ADSR_FOLD_ADJUST5", "1") != "0"  # A/B switch: 0 = adjust5 + the RDG residual as a row-tile GEMM
-if os.environ.get("ADSR_ATTN_PIPE", "1") == "0":                # A/B switch: 0 = the fused attention kernel takes its heads one after the other
-    import ctypes as _ct
-    from . import _abi as _abi_dbg
-    _f = _abi_dbg.lib().adsr_debug_set_attn_pipe
-    _f.restype, _f.argtypes = None, [_ct.c_int]
-    _f(0)
-_ALT_TILE_ORDER = os.environ.get("ADSR_ALT_TILE_ORDER", "1") != "0"  # A/B switch: 0 = every kernel walks its row tiles front to back
-_FUSED_ATTN = os.environ.get("ADSR_FUSED_ATTN", "1") != "0"
-_PREFER_ATTN2 = os.environ.get("ADSR_PREFER_ATTN2", "0") != "0"  # A/B switch: 1 = swin_attn2 (+ proj GEMM) wherever it covers the block shape    # A/B switch for profiling: 0 = separate qkv / attention / proj kernels
 
 
 def _heads_for(dim: int, k: int, nh: int) -> int:
@@ -210,14 +198,12 @@ class DRCT(nn.Module):
                 b.proj = up(pack.pack_proj_weight(proj_w, proj_b, b.heads))
                 # fused attention half (csrc/swin_attn.cu): 2 = qkv + attention + proj + residual in one kernel,
                 # 1 = qkv + attention (proj stays a row-tile GEMM), 0 = shape not covered (separate kernels)
-                b.attn_mode = ops.swin_attn_mode(b.dim, b.heads, b.hdp) if (b.ws == 8 and _FUSED_ATTN) else 0
-                if b.attn_mode == 2 and _PREFER_ATTN2 and ops.swin_attn2_covers(b.dim, b.heads, b.hdp):
-                    b.attn_mode = 1           # two-heads-in-flight attention kernel + proj as a row-tile GEMM
+                b.attn_mode = ops.swin_attn_mode(b.dim, b.heads, b.hdp) if b.ws == 8 else 0
                 b.attn = up(pack.pack_swin_attn(qkv_w, qkv_b, n1w, n1b, sw.norm1.eps, proj_w, proj_b, b.heads)) if b.attn_mode else None
                 # the 32-channel adjust convs ride in the MLP kernel's last epilogue where its tiling leaves room (z is then never
                 # written); otherwise (and for adjust5) the adjust conv stays a GEMM of its own
                 b.mlp = None
-                if k < 4 and adj.out_channels == 32 and _FUSED_ADJUST:
+                if k < 4 and adj.out_channels == 32:
                     try:
                         b.mlp = up(pack.pack_swin_mlp(fc1_w, fc1_b, n2w, n2b, sw.norm2.eps, fc2_w, fc2_b, adj_w, adj_b))
                     except ValueError:
@@ -226,7 +212,7 @@ class DRCT(nn.Module):
                     b.mlp = up(pack.pack_swin_mlp(fc1_w, fc1_b, n2w, n2b, sw.norm2.eps, fc2_w, fc2_b))
                 # adjust5 and the group's residual (`x5 * 0.2 + x`, src/drct.py:394-396) fold into the last block's MLP kernel the same way
                 b.mlp_res = None
-                if k == 4 and _FOLD_ADJUST5:
+                if k == 4:
                     try:
                         b.mlp_res = up(pack.pack_swin_mlp_conv_res(fc1_w, fc1_b, n2w, n2b, sw.norm2.eps, fc2_w, fc2_b, adj_w, adj_b, 0.2))
                     except ValueError:
@@ -316,10 +302,9 @@ class DRCT(nn.Module):
         ops.drct_head(x, P["cf_w"], P["cf_b"], P["mean"], float(self.img_range), P["pe_w"], P["pe_b"], D, ws["x0"], slab,
                       stats_out=st_slab)
 
-        # Tile order: the persistent row-tile kernels (proj / adjust GEMMs, fused MLP) can walk their 128-row tiles backwards.  A batch-256
-        # activation (94 - 168 MB) does not fit the 126 MB L2 next to everything else, but the rows its producer wrote LAST are still
-        # there: each of these kernels runs opposite to the kernel that produced its input (the attention kernels always run forward).
-        rev = _ALT_TILE_ORDER
+        # Tile order: the persistent row-tile kernels (proj / adjust GEMMs, fused MLP) walk their 128-row tiles in either direction.  A
+        # batch-256 activation (94 - 168 MB) does not fit the 126 MB L2 next to everything else, but the rows its producer wrote LAST are
+        # still there: each of these kernels runs opposite to the kernel that produced its input (the attention kernels always run forward).
         slab_fwd = True                                   # direction in which the current slab contents were written
         for blocks in P["blocks"]:
             # st_slab: x owns the first xs slots (written by adjust5: four partial slots from the folded kernel), each x_j two more
@@ -336,16 +321,16 @@ class DRCT(nn.Module):
                     y_fwd = True
                 elif fused == 1:
                     ops.swin_attn(slab, b.attn, b.table, att, B, H, W, b.shift, (st_slab, xs + 2 * k), False)
-                    ops.tc_gemm(att, b.heads * b.hdp, b.proj, y, res=slab, stats_out=(st_y, 0), reverse=rev)
-                    y_fwd = not rev
+                    ops.tc_gemm(att, b.heads * b.hdp, b.proj, y, res=slab, stats_out=(st_y, 0), reverse=True)
+                    y_fwd = False
                 else:
-                    ops.tc_gemm(slab, C, b.qkv, qkv, stats_in=(st_slab, xs + 2 * k), reverse=rev and slab_fwd)
+                    ops.tc_gemm(slab, C, b.qkv, qkv, stats_in=(st_slab, xs + 2 * k), reverse=slab_fwd)
                     ops.window_attention(qkv, att, b.table, B, H, W, b.ws, b.shift, b.heads, b.hd, b.hdp)
-                    ops.tc_gemm(att, b.heads * b.hdp, b.proj, y, res=slab, stats_out=(st_y, 0), reverse=rev)
-                    y_fwd = not rev
+                    ops.tc_gemm(att, b.heads * b.hdp, b.proj, y, res=slab, stats_out=(st_y, 0), reverse=True)
+                    y_fwd = False
                 # ---- MLP half (src/drct.py:510, 185-189): norm2 + fc1 + GELU + fc2 + residual in ONE kernel, the hidden
                 #      activations never leave the SM
-                mlp_rev = rev and y_fwd
+                mlp_rev = y_fwd
                 if b.mlp.wadj is not None:
                     # ... and the adjust 1x1 conv (+LeakyReLU 0.2) into the slab slice (src/drct.py:389-393) in the same kernel
                     ops.swin_mlp_adjust(y, C, b.mlp, slab, C, stats_in=(st_y, y_slots), stats_out=(st_slab, xs + 2 * k), reverse=mlp_rev)
@@ -358,7 +343,7 @@ class DRCT(nn.Module):
                     continue
                 ops.swin_mlp(y, C, b.mlp, z, stats_in=(st_y, y_slots), reverse=mlp_rev)
                 # ---- adjust 1x1 conv (+LeakyReLU 0.2) into the slab slice / 0.2*x5 + x  (src/drct.py:389-396)
-                adj_rev = rev and not mlp_rev
+                adj_rev = not mlp_rev
                 if not b.last:
                     ops.tc_gemm(z, C, b.adjust, slab, act=ops.ACT_LRELU, slope=0.2, ocol0=C, n_store=b.adjust_out,
                                 stats_out=(st_slab, xs + 2 * k), reverse=adj_rev)

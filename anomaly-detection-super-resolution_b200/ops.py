@@ -7,7 +7,6 @@ module (bench.py reports it as `gpu_launches`).
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import Optional, Sequence
 
 import torch
@@ -17,7 +16,7 @@ from ._abi import ACT_GELU, ACT_LRELU, ACT_NONE, ACT_RELU, OUT_PIXEL_SHUFFLE2, O
 from .pack import PackedWeight
 
 LAUNCHES = 0
-_HALO_CONV = os.environ.get("ADSR_HALO_CONV", "1") != "0"   # narrow 3x3 convs through csrc/conv_halo.cu (0 = streaming implicit GEMM)
+_HALO_CONV = True   # narrow 3x3 convs through csrc/conv_halo.cu; tests and tools/conv_bench.py clear it to run the implicit GEMM instead
 PROFILE = None      # set to a list to collect (kind, algorithmic_flops, start_event, end_event) per launch (bench.py)
 
 
@@ -130,11 +129,6 @@ def swin_mlp_conv_res(y: torch.Tensor, c: int, pm, res: torch.Tensor, out: torch
 def swin_attn_mode(c: int, heads: int, hdp: int, allow_proj: bool = True) -> int:
     """What adsr_swin_attn_bf16 covers for this block shape: 2 = whole attention half, 1 = qkv + attention, 0 = nothing."""
     return int(lib().adsr_swin_attn_mode(c, heads, hdp, int(allow_proj)))
-
-
-def swin_attn2_covers(c: int, heads: int, hdp: int) -> bool:
-    """True when the two-heads-in-flight attention kernel (csrc/swin_attn2.cu) covers this block shape."""
-    return bool(lib().adsr_swin_attn2_covers(c, heads, hdp))
 
 
 def swin_attn(x: torch.Tensor, pa, table: torch.Tensor, out: torch.Tensor, b: int, h: int, w: int, shift: int, stats_in: tuple,

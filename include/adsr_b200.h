@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 13
+#define ADSR_ABI_VERSION 14
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -131,10 +131,6 @@ int adsr_swin_mlp_conv_res_bf16(const void* y, int64_t ldy, int M, int C,
  *   0 = shape not covered (use adsr_tc_gemm_bf16 + adsr_window_attention).
  * Requires H % 8 == W % 8 == 0 and an even number of windows; x and out must not alias. */
 int adsr_swin_attn_mode(int C, int heads, int head_dim_padded, int allow_proj);
-/* 1 when the attention-only call (fuse_proj = 0) of this block shape runs the two-heads-in-flight kernel (csrc/swin_attn2.cu: the 16
- * epilogue warps form two groups that own the even / odd heads, each with its own TMEM region and k / v panels): two regions of
- * max(3 hdp, hdp + 128) columns and two k/v panel sets must fit; otherwise 0 (one head at a time). */
-int adsr_swin_attn2_covers(int C, int heads, int head_dim_padded);
 int adsr_swin_attn_bf16(const void* x, int64_t ldx, int B, int H, int W, int C, int shift, int heads, int head_dim,
                         int head_dim_padded, const void* w1_packed, const void* w2_packed,
                         const float* bias_qkv, const float* colsum_qkv, const float* bias_proj, const float* bias_table,

@@ -108,27 +108,13 @@ def test_swin_attn_many_tiles_per_cta_and_rect():
     _case(1, 8, 16, 276, 6, 0, True, seed=9)            # a single tile
 
 
-def _set_attn2(enabled: int):
-    import ctypes
-    abi = mod("_abi")
-    f = abi.lib().adsr_debug_set_swin_attn2
-    f.restype, f.argtypes = None, [ctypes.c_int]
-    f(enabled)
-
-
 @pytest.mark.parametrize("C,heads", [(180, 6), (212, 4), (276, 6)])
-@pytest.mark.parametrize("shift", [0, 4])
-@pytest.mark.parametrize("variant", [1, 0])
-def test_swin_attn2_two_heads_in_flight(C, heads, shift, variant):
-    """qkv + attention only (proj stays a GEMM): the two-heads-in-flight kernel of csrc/swin_attn2.cu (variant 1: two epilogue
-    groups own the even / odd heads) and the one-head-at-a-time kernel of csrc/swin_attn.cu (variant 0) on the DRCT-L block
-    shapes whose two TMEM regions + two k/v panel sets fit, several tiles per CTA."""
-    abi, pack = mod("_abi"), mod("pack")
-    assert abi.lib().adsr_swin_attn2_covers(C, heads, pack.head_pad(C // heads)) == 1
-    _set_attn2(variant)
-    try:
-        _case(40, 32, 32, C, heads, shift, False, seed=C + shift + variant)
-        _case(1, 8, 16, C, heads, 0, False, seed=3)            # a single tile: only one head per group in flight at the end
-        _case(3, 16, 24, C, heads, shift, False, seed=5)       # 9 tiles on 148 SMs: one tile per CTA, rectangular
-    finally:
-        _set_attn2(1)
+@pytest.mark.parametrize("B,H,W,shift", [
+    (40, 32, 32, 0), (40, 32, 32, 4),        # 320 window pairs on 148 SMs: several tiles per CTA
+    (1, 8, 16, 0),                           # a single tile
+    (3, 16, 24, 0), (3, 16, 24, 4),          # 9 tiles on 148 SMs: one tile per CTA, rectangular
+])
+def test_swin_attn_qkv_attention_only_geometries(C, heads, B, H, W, shift):
+    """qkv + attention only (proj stays a GEMM) on the DRCT-L block shapes the model runs with proj fused, over tile counts
+    from one to several per CTA: the fused kernel with two TMEM head regions (the next head's q|k|v runs one head ahead)."""
+    _case(B, H, W, C, heads, shift, False, seed={40: C + shift, 1: 3, 3: 5}[B])

@@ -6,10 +6,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 PKG = "anomaly-detection-super-resolution_b200"
 ops = importlib.import_module(PKG + ".ops"); pack = importlib.import_module(PKG + ".pack")
 dev = "cuda"
-if os.environ.get("PIPE"):      # PIPE=0: heads one after the other in the fused kernel (A/B of the pipelined head order)
-    import ctypes
-    _abi = importlib.import_module(PKG + "._abi"); _f = _abi.lib().adsr_debug_set_attn_pipe; _f.restype = None; _f.argtypes = [ctypes.c_int]
-    _f(int(os.environ["PIPE"]))
 B = int(os.environ.get("B", 256)); H = W = 32
 M = B * H * W
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
@@ -68,20 +64,9 @@ for (C, heads, shift) in shapes:
     bs, as_ = timeit(separate)
     line = (f"attn half C={C} heads={heads} hd={hd:3d} shift={shift} mode={mode}: fused {bf*1e3:7.1f} us (avg {af*1e3:7.1f}) "
             f"{fl/bf/1e9:6.1f} TFLOP/s   separate {bs*1e3:7.1f} us")
-    import ctypes
-    lib = importlib.import_module(PKG + "._abi").lib()
-    has2 = hasattr(lib, "adsr_debug_set_swin_attn2")
-    if has2:
-        lib.adsr_debug_set_swin_attn2.restype, lib.adsr_debug_set_swin_attn2.argtypes = None, [ctypes.c_int]
     fa = 2.0 * M * C * 3 * C + 4.0 * M * 64 * C
-    for variant in ((1, 0) if has2 else (0,)):
-        if has2:
-            lib.adsr_debug_set_swin_attn2(variant)
-        covers = lib.adsr_swin_attn2_covers(C, heads, hdp) if has2 else 0
-        ba, _ = timeit(attn_only)
-        line += f"   | attn-only v{variant}{'*' if covers else ' '} {ba*1e3:7.1f} us {fa/ba/1e9:6.1f} TF"
-    if has2:
-        lib.adsr_debug_set_swin_attn2(1)
+    ba, _ = timeit(attn_only)
+    line += f"   | attn-only {ba*1e3:7.1f} us {fa/ba/1e9:6.1f} TF"
     bp, _ = timeit(proj_only)
     line += f"   proj GEMM {bp*1e3:6.1f} us"
     print(line)

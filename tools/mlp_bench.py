@@ -5,10 +5,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 PKG = "anomaly-detection-super-resolution_b200"
 ops = importlib.import_module(PKG + ".ops"); pack = importlib.import_module(PKG + ".pack")
 dev = "cuda"
-if os.environ.get("ACC1"):      # ACC1=2: never use a third fc1 chunk accumulator (A/B of the folded-adjust kernel)
-    import ctypes
-    _abi = importlib.import_module(PKG + "._abi"); _f = _abi.lib().adsr_debug_set_mlp_acc1; _f.restype = None; _f.argtypes = [ctypes.c_int]
-    _f(int(os.environ["ACC1"]))
 M = int(os.environ.get("M", 262144))
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
 
