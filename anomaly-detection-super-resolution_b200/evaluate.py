@@ -52,6 +52,16 @@ def parse_args(argv=None):
     p.add_argument('--output-dir', type=str, default='')
     p.add_argument('--save-images', action='store_true', default=True)
     p.add_argument('--workers', type=int, default=0 if sys.platform == 'darwin' else 4)
+    # localisation: per-pixel anomaly maps (1 - SSIM of one window size, squared error), their max as image scores, pixel AUROC
+    p.add_argument('--anomaly-maps', action='store_true', default=False,
+                   help='also compute per-pixel 1-SSIM and squared-error maps and report the AUCs of their per-image max')
+    p.add_argument('--map-window-size', type=int, default=11, help='SSIM window size of the 1-SSIM map (odd)')
+    p.add_argument('--map-sigma', type=float, default=4.0, help='Gaussian smoothing of both maps (scipy gaussian_filter sigma; 0 = off)')
+    p.add_argument('--mask-dir', type=str, default=None,
+                   help='ground-truth masks <mask-dir>/<stem>.png or <stem>_mask.png (non-zero = defect): adds pixel AUROC; '
+                        'implies --anomaly-maps')
+    p.add_argument('--save-maps', action='store_true', default=False,
+                   help='write <output-dir>/maps/<split>/<stem>_ssim.npy and <stem>_se.npy (float32 HxW); implies --anomaly-maps')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
 
@@ -169,14 +179,21 @@ class BatchedEvaluator:
 
     `step(lr, hr)` takes what the reference's loader yields (float tensors in [0, rgb_range], on the host or
     already on the device) and returns the fp64 score table [B, n_ws + 2] on the device; nothing else leaves
-    the GPU.  Host tensors are copied with non_blocking=True (pin them for overlap)."""
+    the GPU.  Host tensors are copied with non_blocking=True (pin them for overlap).
 
-    def __init__(self, model, rgb_range: float, window_sizes: Optional[Sequence[int]] = None):
+    maps = (win_size, sigma) also computes the anomaly maps of every step (ops.anomaly_maps on the step's uint8 SR / HR):
+    `last_maps` = (1 - SSIM map, squared-error map, per-image max of both), next to `last_sr_u8` and `last_hr_u8`."""
+
+    def __init__(self, model, rgb_range: float, window_sizes: Optional[Sequence[int]] = None,
+                 maps: Optional[Tuple[int, float]] = None):
         self.model = model
         self.rgb_range = float(rgb_range)
         self.window_sizes = list(window_sizes) if window_sizes is not None else None
+        self.maps = (int(maps[0]), float(maps[1])) if maps is not None else None
         self.device = torch.device('cuda')
         self.last_sr_u8: Optional[torch.Tensor] = None
+        self.last_hr_u8: Optional[torch.Tensor] = None
+        self.last_maps: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None
         self._copy_stream = None
         self._graphs = {}
         self.use_graph = os.environ.get('ADSR_CUDA_GRAPH', '1') != '0'
@@ -195,13 +212,14 @@ class BatchedEvaluator:
     # ---- the whole step (~1000 kernel launches through the C ABI) as ONE CUDA graph per static input buffer pair
     def _score_graphed(self, lr_d: torch.Tensor, hr_d: torch.Tensor) -> torch.Tensor:
         """First call for a buffer pair runs eagerly (workspaces, packed weights), the second one is captured, later ones
-        replay the graph.  The returned table (and last_sr_u8) are the graph's static outputs: valid until the next replay."""
+        replay the graph.  The returned table (and last_sr_u8, last_hr_u8, last_maps) are the graph's static outputs: valid until
+        the next replay."""
         if not self.use_graph or ops.PROFILE is not None:
             return self._score(lr_d, hr_d)
         target = self.model.model if hasattr(self.model, 'model') else self.model
         packed = target._pack() if hasattr(target, '_pack') else None     # repacked weights (new parameters) -> a new graph
         key = (lr_d.data_ptr(), hr_d.data_ptr(), tuple(lr_d.shape), tuple(hr_d.shape), lr_d.dtype, hr_d.dtype,
-               tuple(self.window_sizes) if self.window_sizes is not None else None, id(packed))
+               tuple(self.window_sizes) if self.window_sizes is not None else None, id(packed), self.maps)
         ent = self._graphs.get(key)
         if ent is None:
             while len(self._graphs) >= 8:                     # evict the oldest entry only (no recapture thrash)
@@ -216,6 +234,8 @@ class BatchedEvaluator:
                 with torch.cuda.graph(g):
                     ent["out"] = self._score(lr_d, hr_d)
                     ent["sr_u8"] = self.last_sr_u8
+                    ent["hr_u8"] = self.last_hr_u8
+                    ent["maps"] = self.last_maps
                 ent["launches"] = ops.LAUNCHES - n0
                 ops.LAUNCHES = n0
                 ent["graph"] = g
@@ -229,6 +249,8 @@ class BatchedEvaluator:
         ent["graph"].replay()
         ops.LAUNCHES += ent["launches"]
         self.last_sr_u8 = ent["sr_u8"]
+        self.last_hr_u8 = ent["hr_u8"]
+        self.last_maps = ent["maps"]
         return ent["out"]
 
     def _score(self, lr_d: torch.Tensor, hr_d: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -246,7 +268,10 @@ class BatchedEvaluator:
         if self.window_sizes is None:
             self.window_sizes = metrics.window_sizes_for(min(h, w))
         self.last_sr_u8 = sr_u8
-        return metrics.score_batch(sr_u8, hr_u8, self.window_sizes, out)
+        self.last_hr_u8 = hr_u8
+        scores = metrics.score_batch(sr_u8, hr_u8, self.window_sizes, out)
+        self.last_maps = ops.anomaly_maps(sr_u8, hr_u8, *self.maps) if self.maps is not None else None
+        return scores
 
     # ---- double-buffered input path: the host -> device copies of batch i + 1 run on a copy stream while batch i is computed
     def submit(self, lr: torch.Tensor, hr: torch.Tensor):
@@ -360,6 +385,33 @@ def scores_table(gathered: torch.Tensor, n_total: int) -> np.ndarray:
     return out
 
 
+def find_mask(mask_dir: str, hr_path: str, label: int) -> Optional[str]:
+    """Ground-truth mask of HR image `<stem>.png`: `<mask_dir>/<stem>.png`, else `<mask_dir>/<stem>_mask.png`; None for a good image
+    without one (all clear).  A bad image needs a mask."""
+    stem = os.path.splitext(os.path.basename(hr_path))[0]
+    cands = [os.path.join(mask_dir, f'{stem}.png'), os.path.join(mask_dir, f'{stem}_mask.png')]
+    for c in cands:
+        if os.path.exists(c):
+            return c
+    if label:
+        raise FileNotFoundError(f"mask not found for defective image {hr_path}: tried {', '.join(cands)}")
+    return None
+
+
+def load_mask(path: Optional[str], hr_shape: Tuple[int, int], crop: Tuple[int, int]) -> np.ndarray:
+    """bool [H, W] defect mask (any non-zero channel), cropped like its HR image (`hr[0:crop[0], 0:crop[1]]`); None = all clear."""
+    from PIL import Image
+
+    if path is None:
+        return np.zeros(hr_shape, dtype=bool)
+    m = np.array(Image.open(path))
+    m = (m != 0).any(axis=2) if m.ndim == 3 else m != 0
+    m = m[0:crop[0], 0:crop[1]]
+    if m.shape != tuple(hr_shape):
+        raise ValueError(f"mask {path} is {m.shape[0]}x{m.shape[1]} after cropping, its image is {hr_shape[0]}x{hr_shape[1]}")
+    return m
+
+
 def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str, scale_value: int) -> None:
     from PIL import Image
 
@@ -369,12 +421,22 @@ def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str,
     img.save(str(out_dir / f"{name}.png"))
 
 
-def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: bool, batch_size: Optional[int] = None):
-    """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n)."""
+def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: bool, batch_size: Optional[int] = None,
+                     anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
+                     save_maps: bool = False):
+    """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
+
+    anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
+    a Gaussian of map_sigma; the AUCs of their per-image max are added as auc_map_ssim / auc_map_se (the maxima as `map_max`) and
+    printed on a `Map AUCs - ...` line before the `Test AUCs - ...` line.  mask_dir adds the pixel-level AUROC of both maps
+    (pixel_auroc_ssim / pixel_auroc_se; single process only).  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
     from .model import Model
 
+    anomaly_maps = anomaly_maps or mask_dir is not None or save_maps
     scale = opt.scale[-1] if isinstance(opt.scale, list) else int(opt.scale)
     rank, world = _dist_info()
+    if mask_dir is not None and world > 1:
+        raise RuntimeError("--mask-dir needs the whole maps of every image in one process: run it without sharding (world size 1)")
     entries = []                                             # (label, split, hr path, lr path): good first, then bad
     for label, split in ((0, 'good'), (1, 'bad')):
         d = f'{opt.data_root}/{opt.classe}/test/{split}'
@@ -384,6 +446,7 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     if len(set(y_true)) < 2:
         print('Test set lacks both classes; AUC not available')
         return None
+    mask_paths = [find_mask(mask_dir, e[2], e[0]) for e in entries] if mask_dir is not None else None   # fail before the model runs
 
     # SSIM window sizes come from the smallest HR dimension over the WHOLE test set (src/evaluate.py:233-235), known from the
     # PNG headers before the images are sharded: every rank sweeps the same sizes, also one that holds no image at all
@@ -397,7 +460,8 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
 
     opt.pre_train = checkpoint_model_path
     model = Model(opt, None)
-    ev = BatchedEvaluator(model, opt.rgb_range, metrics.window_sizes_for(min_dim))
+    ev = BatchedEvaluator(model, opt.rgb_range, metrics.window_sizes_for(min_dim),
+                          maps=(map_window_size, map_sigma) if anomaly_maps else None)
     bs = batch_size or getattr(opt, 'eval_batch_size', None) or 64
     mine = list(range(rank, len(entries), world))            # image index i -> rank i mod R
     rows, ids = [], []
@@ -416,8 +480,11 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                 yield (torch.stack([pairs[j][0] for j in g]).pin_memory(), torch.stack([pairs[j][1] for j in g]).pin_memory())
 
     order: List[List[int]] = []
+    pix_maps, pix_masks = ([], []), []                       # host maps and masks of every image (pixel AUROC)
     with torch.no_grad():
         for k, scores in enumerate(ev.run_pipelined(host_batches())):   # PNG decode + H2D of batch k + 1 overlap batch k
+            if ev.last_maps is not None:                      # the two map maxima ride along in the gathered score table
+                scores = torch.cat([scores, ev.last_maps[2]], 1)
             rows.append(scores)
             ids += order[k]
             if save_images:
@@ -425,14 +492,40 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                 for j, i in enumerate(order[k]):
                     name = os.path.splitext(os.path.basename(entries[i][2]))[0]
                     save_sr_image(sr_np[j], output_dir, name, entries[i][1], scale)
+            if mask_dir is not None or save_maps:
+                m_ssim, m_se = ev.last_maps[0].cpu().numpy(), ev.last_maps[1].cpu().numpy()
+                for j, i in enumerate(order[k]):
+                    name = os.path.splitext(os.path.basename(entries[i][2]))[0]
+                    if save_maps:
+                        d = Path(output_dir) / 'maps' / entries[i][1]
+                        d.mkdir(parents=True, exist_ok=True)
+                        np.save(d / f'{name}_ssim.npy', m_ssim[j])
+                        np.save(d / f'{name}_se.npy', m_se[j])
+                    if mask_dir is not None:
+                        with Image.open(entries[i][3]) as im_lr:
+                            crop = (im_lr.size[1] * scale, im_lr.size[0] * scale)
+                        pix_masks.append(load_mask(mask_paths[i], m_ssim.shape[1:], crop))
+                        pix_maps[0].append(m_ssim[j])
+                        pix_maps[1].append(m_se[j])
     n_cols = len(ev.window_sizes) + 2
-    local = torch.cat(rows) if rows else torch.empty(0, n_cols, dtype=torch.float64, device='cuda')
+    local = torch.cat(rows) if rows else torch.empty(0, n_cols + (2 if anomaly_maps else 0), dtype=torch.float64, device='cuda')
     table = gather_scores(local, torch.tensor(ids, dtype=torch.int64, device='cuda'), len(entries))
     if table is None:
         return None
+    table, map_max = table[:, :n_cols], table[:, n_cols:]
     best_ws, auc_ssim, auc_mse, auc_psnr = metrics.aucs_from_scores(y_true, table, ev.window_sizes)
+    res = dict(best_ws=best_ws, auc_ssim=auc_ssim, auc_mse=auc_mse, auc_psnr=auc_psnr, n=len(entries), scores=table)
+    if anomaly_maps:
+        res.update(map_max=map_max, auc_map_ssim=metrics.roc_auc(y_true, map_max[:, 0]), auc_map_se=metrics.roc_auc(y_true, map_max[:, 1]))
+        line = (f"Map AUCs - max 1-SSIM(ws={map_window_size}, sigma={float(map_sigma)}): {res['auc_map_ssim']:.4f}, "
+                f"max SE: {res['auc_map_se']:.4f}")
+        if mask_dir is not None:
+            res.update(pixel_auroc_ssim=metrics.pixel_auroc(pix_maps[0], pix_masks),
+                       pixel_auroc_se=metrics.pixel_auroc(pix_maps[1], pix_masks))
+            line += f", pixel AUROC 1-SSIM: {res['pixel_auroc_ssim']:.4f}, pixel AUROC SE: {res['pixel_auroc_se']:.4f}"
+        print(line)
     print(f"Test AUCs - SSIM(best ws={best_ws}): {auc_ssim:.4f}, MSE: {auc_mse:.4f}, PSNR: {auc_psnr:.4f}")
-    return dict(best_ws=best_ws, auc_ssim=auc_ssim, auc_mse=auc_mse, auc_psnr=auc_psnr, n=len(entries), scores=table)
+    return res
 
 
 def main(argv=None):
@@ -470,7 +563,9 @@ def main(argv=None):
         torch.cuda.set_device(int(os.environ['LOCAL_RANK']))
         dist.init_process_group('nccl')
     out_dir = args.output_dir or (os.path.join(args.run_dir, 'eval_results') if args.run_dir else './workspace/eval_results')
-    return evaluate_on_test(opt, ckpt_path, out_dir, args.save_images, batch_size=args.batch_size)
+    return evaluate_on_test(opt, ckpt_path, out_dir, args.save_images, batch_size=args.batch_size, anomaly_maps=args.anomaly_maps,
+                            map_window_size=args.map_window_size, map_sigma=args.map_sigma, mask_dir=args.mask_dir,
+                            save_maps=args.save_maps)
 
 
 if __name__ == "__main__":

@@ -90,6 +90,27 @@ def score_batch(sr_u8: torch.Tensor, hr_u8: torch.Tensor, window_sizes: Sequence
     return ops.score_images(sr_u8, hr_u8, window_sizes, out)
 
 
+def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int = 11, sigma: float = 0.0):
+    """Where an image is anomalous: uint8 NHWC device tensors -> (1 - SSIM map for one window size, squared-error map averaged over the
+    channels, per-image max of both) as fp32 [B, H, W], fp32 [B, H, W], fp64 [B, 2].  sigma > 0 smooths both maps like
+    scipy.ndimage.gaussian_filter(map, sigma, mode="reflect", truncate=4.0) before the max is taken."""
+    return ops.anomaly_maps(sr_u8, hr_u8, win_size, sigma)
+
+
+def pixel_auroc(maps, masks) -> float:
+    """Pixel-level ROC AUC (the MVTec localisation number): every pixel of every map is one score, a non-zero mask pixel marks a defect.
+    maps / masks: arrays (or sequences of per-image arrays) of matching shapes, on the host."""
+    if isinstance(maps, (list, tuple)):
+        if len(maps) != len(masks) or any(np.shape(a) != np.shape(k) for a, k in zip(maps, masks)):
+            raise ValueError("pixel_auroc: every map needs a mask of its own shape")
+        maps = np.concatenate([np.asarray(m).ravel() for m in maps]) if maps else np.empty(0)
+        masks = np.concatenate([np.asarray(m).ravel() for m in masks]) if masks else np.empty(0)
+    maps, masks = np.asarray(maps), np.asarray(masks)
+    if maps.shape != masks.shape:
+        raise ValueError(f"pixel_auroc: maps {maps.shape} and masks {masks.shape} differ in shape")
+    return roc_auc((masks.ravel() != 0).astype(np.int64), maps.ravel())
+
+
 def roc_auc(y_true, scores) -> float:
     """Image-level ROC AUC on the host (N_img scalars; stays on the CPU like the reference's sklearn call,
     src/evaluate.py:245,263-265).  Uses sklearn when available, else the equivalent rank statistic."""

@@ -304,6 +304,41 @@ def score_images(sr_u8: torch.Tensor, hr_u8: torch.Tensor, window_sizes: Sequenc
     return out
 
 
+def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int, sigma: float = 0.0,
+                 out: Optional[tuple] = None) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """uint8 NHWC pairs -> (ssim_map fp32 [B, H, W] = 1 - SSIM per pixel for one window size, se_map fp32 [B, H, W] = squared error
+    averaged over the channels, map_max fp64 [B, 2] = per-image max of both maps), Gaussian-smoothed when sigma > 0.
+    out: caller-owned (ssim_map, se_map, map_max, scratch) to write into; scratch is the fp32 [B, H, W] buffer of the smoothing and
+    may be None when sigma == 0.  Without `out` everything is allocated here.  Two kernels, six with the smoothing."""
+    _cuda(sr_u8, "sr_u8")
+    _cuda(hr_u8, "hr_u8")
+    if sr_u8.dtype != torch.uint8 or hr_u8.dtype != torch.uint8:
+        raise TypeError(f"anomaly_maps takes uint8 images, got {sr_u8.dtype} / {hr_u8.dtype}")
+    if sr_u8.dim() != 4 or sr_u8.shape != hr_u8.shape or sr_u8.device != hr_u8.device:
+        raise ValueError(f"anomaly_maps needs two [B, H, W, C] images of one shape on one device, got {tuple(sr_u8.shape)} on "
+                         f"{sr_u8.device} and {tuple(hr_u8.shape)} on {hr_u8.device}")
+    sr_u8, hr_u8 = sr_u8.contiguous(), hr_u8.contiguous()
+    b, h, w, c = sr_u8.shape
+    if out is None:
+        f32 = dict(dtype=torch.float32, device=sr_u8.device)
+        out = (torch.empty(b, h, w, **f32), torch.empty(b, h, w, **f32),
+               torch.empty(b, 2, dtype=torch.float64, device=sr_u8.device), torch.empty(b, h, w, **f32) if sigma > 0 else None)
+    ssim_map, se_map, map_max, scratch = out
+    for t, name, dt, shape in ((ssim_map, "ssim_map", torch.float32, (b, h, w)), (se_map, "se_map", torch.float32, (b, h, w)),
+                               (map_max, "map_max", torch.float64, (b, 2)), (scratch, "scratch", torch.float32, (b, h, w))):
+        if t is None and name == "scratch":
+            continue
+        if t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous() or t.device != sr_u8.device:
+            raise ValueError(f"anomaly_maps: {name} must be a contiguous {dt} tensor of shape {shape} on {sr_u8.device}")
+    _t = _begin()
+    check(lib().adsr_anomaly_maps(ptr(sr_u8), ptr(hr_u8), b, h, w, c, int(win_size), float(sigma), ptr(ssim_map), ptr(se_map),
+                                  ptr(scratch), ptr(map_max), stream_ptr()), "adsr_anomaly_maps")
+    global LAUNCHES
+    LAUNCHES += 5 if sigma > 0 else 1                  # raw maps [+ row / column Gaussian passes of both maps]; _count adds the max
+    _count("anomaly_maps", 0.0, _t)
+    return ssim_map, se_map, map_max
+
+
 def score_images_strided(sr: torch.Tensor, hr: torch.Tensor, layout: str, window_sizes: Sequence[int], *, div: float = 1.0,
                          clamp01: bool = False, zero_pad: bool = False, c1: float = 1e-4, c2: float = 9e-4,
                          psnr_peak: float = 1.0) -> torch.Tensor:

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 14
+#define ADSR_ABI_VERSION 15
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -251,6 +251,20 @@ int adsr_score_images_strided(const void* sr, const void* hr, int is_f32, int B,
                               const int64_t* host_strides_sr, const int64_t* host_strides_hr, float div,
                               int clamp01, int zero_pad, double c1, double c2, double psnr_peak,
                               const int32_t* host_ws_list, int n_ws, double* scores, void* stream);
+
+/* Per-pixel anomaly maps of uint8 HWC SR / HR pairs (same pixel conventions as adsr_score_images), for defect localisation.
+ * ssim_map, se_map: fp32 [B, H, W]; scratch: fp32 [B, H, W], needed only when sigma > 0 (NULL otherwise);
+ * map_max: fp64 [B, 2] = per-image max of the (smoothed) ssim_map and se_map.
+ *   ssim_map = 1 - SSIM(hr, sr) per pixel for ONE odd win_size (gray conversion, / 255, reflect padding and C1 / C2 of ssim_numpy;
+ *              fp64 sums, stored as fp32): its mean is 1 - the adsr_score_images SSIM of that window size;
+ *   se_map   = mean over channels of (sr / 255 - hr / 255)^2: its mean is the MSE column.
+ * sigma > 0 smooths both maps with scipy.ndimage.gaussian_filter(map, sigma, mode="reflect", truncate=4.0) semantics: radius
+ * r = int(4 sigma + 0.5) <= 64, normalised taps exp(-x^2 / 2 sigma^2), half-sample reflection at the borders; sigma == 0: no smoothing.
+ * ADSR_ERR_BAD_SHAPE: C not 1 or 3, H < 2, W < 2, W > 1024, even win_size, win_size/2 >= min(H, W), r >= min(H, W), r > 64,
+ * sigma < 0, or sigma > 0 with scratch == NULL.  Deterministic; image i does not depend on the rest of the batch. */
+int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B, int H, int W, int C,
+                      int win_size, float sigma, float* ssim_map, float* se_map, float* scratch,
+                      double* map_max, void* stream);
 
 /* Validation metrics of the reference's training loop, `Trainer.test` (src/trainer.py:242-304), for a batch of fp32 image
  * pairs: the SR value is first quantised with ROUNDING (`quantize`, src/trainer.py:45-47: round(clamp(x * 255 / rgb_range, 0,
