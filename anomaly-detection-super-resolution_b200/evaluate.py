@@ -62,13 +62,21 @@ def parse_args(argv=None):
                         'implies --anomaly-maps')
     p.add_argument('--save-maps', action='store_true', default=False,
                    help='write <output-dir>/maps/<split>/<stem>_ssim.npy and <stem>_se.npy (float32 HxW); implies --anomaly-maps')
+    p.add_argument('--au-pro', type=float, nargs='?', const=0.3, default=None, metavar='FPR_LIMIT',
+                   help='also report the AU-PRO of both maps up to this false-positive rate (bare flag: 0.3); needs --mask-dir')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
 
         with open(pre_args.config, 'r') as f:
             cfg = yaml.safe_load(f) or {}
         p.set_defaults(**{k.replace('-', '_'): v for k, v in cfg.items()})
-    return p.parse_args(argv)
+    args = p.parse_args(argv)
+    if args.au_pro is not None:
+        if args.mask_dir is None:
+            p.error('--au-pro needs --mask-dir (the ground-truth masks define the defect regions)')
+        if not 0.0 < args.au_pro <= 1.0:
+            p.error(f'--au-pro: the false-positive-rate limit must be in (0, 1], got {args.au_pro}')
+    return args
 
 
 def infer_from_run_dir(run_dir: str):
@@ -423,15 +431,22 @@ def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str,
 
 def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: bool, batch_size: Optional[int] = None,
                      anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
-                     save_maps: bool = False):
+                     save_maps: bool = False, au_pro: Optional[float] = None):
     """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
 
     anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
     a Gaussian of map_sigma; the AUCs of their per-image max are added as auc_map_ssim / auc_map_se (the maxima as `map_max`) and
     printed on a `Map AUCs - ...` line before the `Test AUCs - ...` line.  mask_dir adds the pixel-level AUROC of both maps
-    (pixel_auroc_ssim / pixel_auroc_se; single process only).  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
+    (pixel_auroc_ssim / pixel_auroc_se; single process only), ranked on the device by metrics.LocalisationAccumulator.  au_pro (an FPR
+    limit in (0, 1], needs mask_dir) adds the AU-PRO of both maps (au_pro_ssim / au_pro_se, pro_fpr_limit), printed on a `Map PRO - ...`
+    line before the `Map AUCs - ...` line.  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
     from .model import Model
 
+    if au_pro is not None:
+        if mask_dir is None:
+            raise ValueError("au_pro needs mask_dir: the ground-truth masks define the defect regions")
+        if not 0.0 < float(au_pro) <= 1.0:
+            raise ValueError(f"au_pro: the false-positive-rate limit must be in (0, 1], got {au_pro}")
     anomaly_maps = anomaly_maps or mask_dir is not None or save_maps
     scale = opt.scale[-1] if isinstance(opt.scale, list) else int(opt.scale)
     rank, world = _dist_info()
@@ -480,7 +495,7 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                 yield (torch.stack([pairs[j][0] for j in g]).pin_memory(), torch.stack([pairs[j][1] for j in g]).pin_memory())
 
     order: List[List[int]] = []
-    pix_maps, pix_masks = ([], []), []                       # host maps and masks of every image (pixel AUROC)
+    loc = metrics.LocalisationAccumulator(2) if mask_dir is not None else None   # both maps of every image, kept on the device
     with torch.no_grad():
         for k, scores in enumerate(ev.run_pipelined(host_batches())):   # PNG decode + H2D of batch k + 1 overlap batch k
             if ev.last_maps is not None:                      # the two map maxima ride along in the gathered score table
@@ -492,21 +507,21 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                 for j, i in enumerate(order[k]):
                     name = os.path.splitext(os.path.basename(entries[i][2]))[0]
                     save_sr_image(sr_np[j], output_dir, name, entries[i][1], scale)
-            if mask_dir is not None or save_maps:
+            if save_maps:
                 m_ssim, m_se = ev.last_maps[0].cpu().numpy(), ev.last_maps[1].cpu().numpy()
                 for j, i in enumerate(order[k]):
                     name = os.path.splitext(os.path.basename(entries[i][2]))[0]
-                    if save_maps:
-                        d = Path(output_dir) / 'maps' / entries[i][1]
-                        d.mkdir(parents=True, exist_ok=True)
-                        np.save(d / f'{name}_ssim.npy', m_ssim[j])
-                        np.save(d / f'{name}_se.npy', m_se[j])
-                    if mask_dir is not None:
-                        with Image.open(entries[i][3]) as im_lr:
-                            crop = (im_lr.size[1] * scale, im_lr.size[0] * scale)
-                        pix_masks.append(load_mask(mask_paths[i], m_ssim.shape[1:], crop))
-                        pix_maps[0].append(m_ssim[j])
-                        pix_maps[1].append(m_se[j])
+                    d = Path(output_dir) / 'maps' / entries[i][1]
+                    d.mkdir(parents=True, exist_ok=True)
+                    np.save(d / f'{name}_ssim.npy', m_ssim[j])
+                    np.save(d / f'{name}_se.npy', m_se[j])
+            if loc is not None:
+                batch_masks = []
+                for i in order[k]:
+                    with Image.open(entries[i][3]) as im_lr:
+                        crop = (im_lr.size[1] * scale, im_lr.size[0] * scale)
+                    batch_masks.append(load_mask(mask_paths[i], tuple(ev.last_maps[0].shape[1:]), crop))
+                loc.append(ev.last_maps[:2], batch_masks)  # device copies, ordered before the next replay overwrites the maps
     n_cols = len(ev.window_sizes) + 2
     local = torch.cat(rows) if rows else torch.empty(0, n_cols + (2 if anomaly_maps else 0), dtype=torch.float64, device='cuda')
     table = gather_scores(local, torch.tensor(ids, dtype=torch.int64, device='cuda'), len(entries))
@@ -520,9 +535,13 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
         line = (f"Map AUCs - max 1-SSIM(ws={map_window_size}, sigma={float(map_sigma)}): {res['auc_map_ssim']:.4f}, "
                 f"max SE: {res['auc_map_se']:.4f}")
         if mask_dir is not None:
-            res.update(pixel_auroc_ssim=metrics.pixel_auroc(pix_maps[0], pix_masks),
-                       pixel_auroc_se=metrics.pixel_auroc(pix_maps[1], pix_masks))
+            limit = 0.3 if au_pro is None else float(au_pro)
+            (pa_ssim, pro_ssim), (pa_se, pro_se) = loc.finish(limit)
+            res.update(pixel_auroc_ssim=pa_ssim, pixel_auroc_se=pa_se)
             line += f", pixel AUROC 1-SSIM: {res['pixel_auroc_ssim']:.4f}, pixel AUROC SE: {res['pixel_auroc_se']:.4f}"
+            if au_pro is not None:
+                res.update(au_pro_ssim=pro_ssim, au_pro_se=pro_se, pro_fpr_limit=limit)
+                print(f"Map PRO - AU-PRO@{limit:g} 1-SSIM: {pro_ssim:.4f}, AU-PRO@{limit:g} SE: {pro_se:.4f}")
         print(line)
     print(f"Test AUCs - SSIM(best ws={best_ws}): {auc_ssim:.4f}, MSE: {auc_mse:.4f}, PSNR: {auc_psnr:.4f}")
     return res
@@ -565,7 +584,7 @@ def main(argv=None):
     out_dir = args.output_dir or (os.path.join(args.run_dir, 'eval_results') if args.run_dir else './workspace/eval_results')
     return evaluate_on_test(opt, ckpt_path, out_dir, args.save_images, batch_size=args.batch_size, anomaly_maps=args.anomaly_maps,
                             map_window_size=args.map_window_size, map_sigma=args.map_sigma, mask_dir=args.mask_dir,
-                            save_maps=args.save_maps)
+                            save_maps=args.save_maps, au_pro=args.au_pro)
 
 
 if __name__ == "__main__":

@@ -97,9 +97,140 @@ def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int = 11, s
     return ops.anomaly_maps(sr_u8, hr_u8, win_size, sigma)
 
 
+def _map_pieces(maps):
+    """A CUDA map set -> (list of fp32 tensors to append in order, list of per-image (H, W) shapes)."""
+    if isinstance(maps, torch.Tensor):
+        if maps.dim() != 3:
+            raise ValueError(f"maps: expected a [N, H, W] tensor, got shape {tuple(maps.shape)}")
+        pieces, shapes = [maps], [tuple(maps.shape[1:])] * maps.shape[0]
+    else:
+        pieces = list(maps)
+        if any(not isinstance(m, torch.Tensor) or m.dim() != 2 for m in pieces):
+            raise ValueError("maps: expected a [N, H, W] tensor or a sequence of [H, W] tensors")
+        shapes = [tuple(m.shape) for m in pieces]
+    for m in pieces:
+        ops._cuda(m, "maps")
+        if m.dtype != torch.float32:
+            raise TypeError(f"maps must be float32, got {m.dtype}")
+    return pieces, shapes
+
+
+class LocalisationAccumulator:
+    """Pixel AUROC and AU-PRO of `n_maps` anomaly maps over a whole test set, fed one batch at a time.
+
+    append(maps, masks): maps = one entry per map, each a CUDA fp32 [B, H, W] tensor or a sequence of [H, W] tensors (any sizes);
+    masks = the host masks of the same B images (non-zero = defect).  The maps are copied on the device into one growing buffer per map
+    (no device -> host copy); each mask is labelled once on the host (scipy.ndimage.label, 8-connectivity) and its per-pixel region
+    indices are shared by all maps.  finish(fpr_limit) runs adsr_localisation_metrics once per map and returns
+    [(pixel_auroc, au_pro), ...]: the same numbers for the same image sequence however it was split into batches."""
+
+    def __init__(self, n_maps: int = 1):
+        self.n_maps = int(n_maps)
+        self._maps = [None] * self.n_maps             # device fp32 buffers, capacity >= self.n
+        self._regions = None                          # device int32 buffer: -1 = defect-free, else the global region index
+        self.n = 0
+        self.n_ok = 0
+        self._sizes = []                              # host int64 region sizes, one array per image with defects
+
+    @property
+    def n_regions(self) -> int:
+        return sum(len(s) for s in self._sizes)
+
+    def _reserve(self, n_new: int, device) -> None:
+        need = self.n + n_new
+        cap = 0 if self._regions is None else self._regions.numel()
+        if need <= cap:
+            return
+        cap = max(need, 2 * cap)
+        grow = lambda old, dt: (torch.empty(cap, dtype=dt, device=device) if old is None else
+                                torch.cat([old[:self.n], torch.empty(cap - self.n, dtype=dt, device=device)]))
+        self._maps = [grow(m, torch.float32) for m in self._maps]
+        self._regions = grow(self._regions, torch.int32)
+
+    def append(self, maps, masks) -> None:
+        from scipy.ndimage import label
+
+        if len(maps) != self.n_maps:
+            raise ValueError(f"append: {len(maps)} maps given, the accumulator holds {self.n_maps}")
+        parts = [_map_pieces(m) for m in maps]
+        shapes = parts[0][1]
+        masks = [np.asarray(k) for k in masks]
+        if any(p[1] != shapes for p in parts) or len(masks) != len(shapes) or any(k.shape != s for k, s in zip(masks, shapes)):
+            raise ValueError("append: every map needs a mask of its own shape, and all maps the same images")
+        regions, sizes, n_ok, n_reg = [], [], 0, self.n_regions
+        for k in masks:
+            lab, nr = label(k != 0, structure=np.ones((3, 3), dtype=int))
+            lab = lab.ravel()
+            regions.append(np.where(lab > 0, lab + (n_reg - 1), -1).astype(np.int32))
+            if nr:
+                sizes.append(np.bincount(lab, minlength=nr + 1)[1:].astype(np.int64))
+            n_ok += int((lab == 0).sum())
+            n_reg += nr
+        if n_reg > np.iinfo(np.int32).max:
+            raise ValueError("append: more than 2^31 - 1 defect regions")
+        n_new = sum(k.size for k in masks)
+        device = parts[0][0][0].device
+        self._reserve(n_new, device)
+        for buf, (pieces, _) in zip(self._maps, parts):
+            off = self.n
+            for m in pieces:
+                buf[off:off + m.numel()].copy_(m.reshape(-1))
+                off += m.numel()
+        if n_new:
+            self._regions[self.n:self.n + n_new].copy_(torch.from_numpy(np.concatenate(regions)))
+        self._sizes += sizes
+        self.n += n_new
+        self.n_ok += n_ok
+
+    def finish(self, fpr_limit: float = 0.3):
+        """[(pixel AUROC, AU-PRO@fpr_limit)] per map.  ValueError: fpr_limit outside (0, 1], no defect region (R == 0), no defect-free
+        pixel, or a NaN in a map."""
+        fpr_limit = float(fpr_limit)
+        if not 0.0 < fpr_limit <= 1.0:
+            raise ValueError(f"fpr_limit must be in (0, 1], got {fpr_limit}")
+        if self.n_regions == 0:
+            raise ValueError("localisation metrics need at least one defect region (all masks are empty)")
+        if self.n_ok == 0:
+            raise ValueError("localisation metrics need at least one defect-free pixel")
+        device = self._regions.device
+        sizes = torch.from_numpy(np.concatenate(self._sizes)).to(device)
+        ws = torch.empty(ops.localisation_workspace_bytes(self.n), dtype=torch.uint8, device=device)
+        out = torch.empty(self.n_maps, 5, dtype=torch.float64, device=device)
+        for j, buf in enumerate(self._maps):
+            ops.localisation_metrics(buf[:self.n], self._regions[:self.n], sizes, self.n_ok, fpr_limit, ws, out[j])
+        res = out.cpu().numpy()
+        for j in range(self.n_maps):
+            if res[j, 2]:
+                raise ValueError(f"map {j} holds {int(res[j, 2])} NaN scores")
+            if res[j, 3] != self.n_ok or res[j, 4]:
+                raise RuntimeError(f"localisation metrics: inconsistent region indices on the device (map {j}: {res[j, 2:]})")
+        return [(float(r[0]), float(r[1])) for r in res]
+
+
+def _on_device(maps) -> bool:
+    if isinstance(maps, torch.Tensor):
+        return maps.is_cuda
+    return isinstance(maps, (list, tuple)) and len(maps) > 0 and isinstance(maps[0], torch.Tensor) and maps[0].is_cuda
+
+
+def au_pro(maps, masks, fpr_limit: float = 0.3) -> float:
+    """AU-PRO@fpr_limit (the MVTec AD per-region-overlap localisation number): maps = CUDA fp32 [N, H, W] tensor or a sequence of
+    [H, W] tensors of any sizes, masks = host arrays of the same shapes (non-zero = defect).  Defect regions are the 8-connected
+    components of each mask, every region weighs the same; the (FPR, PRO) curve has one point per distinct score and its trapezoid
+    area up to FPR = fpr_limit is divided by fpr_limit.  Computed on the device (adsr_localisation_metrics)."""
+    acc = LocalisationAccumulator(1)
+    acc.append([maps], masks)
+    return acc.finish(fpr_limit)[0][1]
+
+
 def pixel_auroc(maps, masks) -> float:
     """Pixel-level ROC AUC (the MVTec localisation number): every pixel of every map is one score, a non-zero mask pixel marks a defect.
-    maps / masks: arrays (or sequences of per-image arrays) of matching shapes, on the host."""
+    maps / masks: arrays (or sequences of per-image arrays) of matching shapes, on the host.  CUDA maps (an fp32 [N, H, W] tensor or a
+    sequence of [H, W] tensors) with host masks are ranked on the device instead, as au_pro does (the same value)."""
+    if _on_device(maps):
+        acc = LocalisationAccumulator(1)
+        acc.append([maps], masks)
+        return acc.finish()[0][0]
     if isinstance(maps, (list, tuple)):
         if len(maps) != len(masks) or any(np.shape(a) != np.shape(k) for a, k in zip(maps, masks)):
             raise ValueError("pixel_auroc: every map needs a mask of its own shape")

@@ -339,6 +339,37 @@ def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int, sigma:
     return ssim_map, se_map, map_max
 
 
+def localisation_workspace_bytes(n: int) -> int:
+    """Bytes of scratch adsr_localisation_metrics needs for n pixels (two key / region buffer pairs, sort histograms, tile sums)."""
+    b = int(lib().adsr_localisation_workspace_bytes(int(n)))
+    if b < 0:
+        raise ValueError(f"localisation metrics: unsupported pixel count {n}")
+    return b
+
+
+def localisation_metrics(scores: torch.Tensor, regions: torch.Tensor, region_sizes: torch.Tensor, n_ok: int, fpr_limit: float,
+                         workspace: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """Pixel AUROC and AU-PRO@fpr_limit of one map: scores fp32 [n], regions int32 [n] (-1 = defect-free, else an index into
+    region_sizes int64 [R]), n_ok defect-free pixels -> out fp64 [5] = (pixel AUROC, AU-PRO, NaN scores, defect-free pixels seen,
+    out-of-range region indices).  workspace: uint8 [>= localisation_workspace_bytes(n)].  Sixteen kernels, no synchronisation."""
+    for t, name, dt in ((scores, "scores", torch.float32), (regions, "regions", torch.int32), (region_sizes, "region_sizes", torch.int64),
+                        (workspace, "workspace", torch.uint8), (out, "out", torch.float64)):
+        _cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous():
+            raise ValueError(f"localisation_metrics: {name} must be a contiguous {dt} tensor")
+    n = scores.numel()
+    if regions.numel() != n or out.numel() < 5:
+        raise ValueError(f"localisation_metrics: {n} scores, {regions.numel()} region indices, out of {out.numel()} values")
+    _t = _begin()
+    check(lib().adsr_localisation_metrics(ptr(scores), ptr(regions), n, ptr(region_sizes), region_sizes.numel(), int(n_ok),
+                                          float(fpr_limit), ptr(workspace), workspace.numel(), ptr(out), stream_ptr()),
+          "adsr_localisation_metrics")
+    global LAUNCHES
+    LAUNCHES += 15                                     # 4 radix passes x 3 kernels + tile sums + tile scan + curve; _count adds the last
+    _count("localisation_metrics", 0.0, _t)
+    return out
+
+
 def score_images_strided(sr: torch.Tensor, hr: torch.Tensor, layout: str, window_sizes: Sequence[int], *, div: float = 1.0,
                          clamp01: bool = False, zero_pad: bool = False, c1: float = 1e-4, c2: float = 9e-4,
                          psnr_peak: float = 1.0) -> torch.Tensor:

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 15
+#define ADSR_ABI_VERSION 16
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -265,6 +265,22 @@ int adsr_score_images_strided(const void* sr, const void* hr, int is_f32, int B,
 int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B, int H, int W, int C,
                       int win_size, float sigma, float* ssim_map, float* se_map, float* scratch,
                       double* map_max, void* stream);
+
+/* Localisation metrics of ONE anomaly map over a whole test set: pixel AUROC and AU-PRO@fpr_limit, exact (no threshold binning).
+ * scores: fp32 [n] (all pixels of all images, higher = more anomalous); regions: int32 [n], -1 = defect-free pixel, else the index of
+ * the pixel's defect region (8-connected component of a ground-truth mask) in region_sizes: int64 [n_regions] pixel counts.
+ * n_ok = number of defect-free pixels.  All pixels are ranked by score, descending (-0.0 = +0.0); equal scores form one curve point.
+ *   pixel AUROC = sklearn.metrics.roc_auc_score(regions >= 0, scores) (ties count one half);
+ *   AU-PRO      = (1 / fpr_limit) * trapezoid area under (FPR, PRO) from FPR 0 to fpr_limit, the crossing segment cut by linear
+ *                 interpolation; FPR = share of the defect-free pixels at or above the score, PRO = mean over the regions of the share
+ *                 of the region's pixels at or above it.
+ * out: fp64 [5] = {pixel AUROC, AU-PRO, NaN scores, defect-free pixels seen, region indices out of range}: the last three are checks
+ * for the caller (the metrics are only valid when they read 0, n_ok, 0).  workspace: adsr_localisation_workspace_bytes(n) bytes, 16-byte
+ * aligned.  Deterministic (integer sort and counts, fixed-order fp64 area) and a function of the pixel sequence alone.
+ * ADSR_ERR_BAD_SHAPE: n < 1, n_regions < 1, n_ok < 1, n_ok >= n, fpr_limit outside (0, 1], a NULL pointer or a short workspace. */
+int64_t adsr_localisation_workspace_bytes(int64_t n);
+int adsr_localisation_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes, int n_regions,
+                              int64_t n_ok, double fpr_limit, void* workspace, int64_t workspace_bytes, double* out, void* stream);
 
 /* Validation metrics of the reference's training loop, `Trainer.test` (src/trainer.py:242-304), for a batch of fp32 image
  * pairs: the SR value is first quantised with ROUNDING (`quantize`, src/trainer.py:45-47: round(clamp(x * 255 / rgb_range, 0,

@@ -1,0 +1,130 @@
+"""Device time of the localisation metrics (pixel AUROC + AU-PRO of one anomaly map over a whole test set, csrc/localisation.cu) on
+synthetic maps and masks: random rectangles and round blobs as defects, smoothed noise with raised scores on the defects as the map.
+
+Per repetition (CUDA events): the append of one map (device copy of every batch into the accumulator's buffer) and the finish (the
+sixteen kernels of adsr_localisation_metrics).  The default 1024 images of 256 x 256 are 67 M pixels per map: the sort's 16 bytes of
+pairs per pixel are far above the 126 MB of L2.  --host also times the host path of the same inputs (sklearn's roc_auc_score behind
+metrics.pixel_auroc on host arrays, the oracle's AU-PRO) and reports the agreement.  One JSON line, with the card and its power limit.
+
+    python tools/localisation_bench.py [--images 1024] [--side 256] [--reps 20] [--host]
+"""
+from __future__ import annotations
+
+import argparse
+import importlib
+import json
+import os
+import statistics
+import subprocess
+import sys
+import time
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+PKG = "anomaly-detection-super-resolution_b200"
+
+
+def synthetic(n, side, seed):
+    """uint8 masks [n, side, side] (a third of the images defect-free) and fp32 maps, generated on the device from a seed."""
+    g = torch.Generator(device="cuda").manual_seed(seed)
+    rng = np.random.default_rng(seed)
+    masks = np.zeros((n, side, side), np.uint8)
+    yy, xx = np.mgrid[:side, :side]
+    for i in range(n):
+        if i % 3 == 0:
+            continue
+        for _ in range(rng.integers(1, 4)):
+            y, x = rng.integers(0, side, 2)
+            masks[i, y:y + rng.integers(2, side // 6), x:x + rng.integers(2, side // 6)] = 1
+        cy, cx, r = rng.integers(0, side), rng.integers(0, side), rng.integers(3, side // 10)
+        masks[i][(yy - cy) ** 2 + (xx - cx) ** 2 <= r * r] = 1
+    noise = torch.rand(n, 1, side, side, generator=g, device="cuda")
+    k = torch.ones(1, 1, 5, 5, device="cuda") / 25.0
+    smooth = torch.nn.functional.conv2d(noise, k, padding=2)[:, 0]
+    maps = (smooth + 0.15 * torch.from_numpy(masks).cuda().float()).contiguous()
+    return maps, masks
+
+
+def card():
+    name = torch.cuda.get_device_name()
+    try:
+        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits", "-i",
+                            str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30)
+        power = float(q.stdout.strip().splitlines()[0])
+    except Exception:                                       # nvidia-smi missing or unreadable: the number stays unreported
+        power = None
+    return name, power
+
+
+def main(argv=None):
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--images", type=int, default=1024)
+    ap.add_argument("--side", type=int, default=256)
+    ap.add_argument("--batch", type=int, default=64, help="images per append")
+    ap.add_argument("--reps", type=int, default=20)
+    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--fpr-limit", type=float, default=0.3)
+    ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--host", action="store_true", help="also time the host path on the same inputs and report the agreement")
+    a = ap.parse_args(argv)
+    if not torch.cuda.is_available():
+        raise SystemExit("localisation_bench needs a CUDA device")
+    metrics = importlib.import_module(PKG + ".metrics")
+    ops = importlib.import_module(PKG + ".ops")
+
+    maps, masks = synthetic(a.images, a.side, a.seed)
+    acc = metrics.LocalisationAccumulator(1)
+    for s in range(0, a.images, a.batch):                   # host labelling + region upload happen here, once
+        acc.append([maps[s:s + a.batch]], masks[s:s + a.batch])
+    (auroc, aupro), = acc.finish(a.fpr_limit)
+    n = acc.n
+    buf, regions = acc._maps[0], acc._regions[:n]
+    sizes = torch.from_numpy(np.concatenate(acc._sizes)).cuda()
+    ws = torch.empty(ops.localisation_workspace_bytes(n), dtype=torch.uint8, device="cuda")
+    out = torch.empty(5, dtype=torch.float64, device="cuda")
+
+    def one():                                              # the device work of append (per-batch copies) + finish, one map
+        off = 0
+        for s in range(0, a.images, a.batch):
+            m = maps[s:s + a.batch]
+            buf[off:off + m.numel()].copy_(m.reshape(-1))
+            off += m.numel()
+        ops.localisation_metrics(buf[:n], regions, sizes, acc.n_ok, a.fpr_limit, ws, out)
+
+    for _ in range(a.warmup):
+        one()
+    times = []
+    for _ in range(a.reps):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        one()
+        e1.record()
+        e1.synchronize()
+        times.append(e0.elapsed_time(e1))
+    again = out.cpu().numpy()
+    name, power = card()
+    res = dict(tool="localisation_bench", gpu=name, power_limit_w=power, images=a.images, side=a.side, pixels_per_map=n,
+               regions=acc.n_regions, fpr_limit=a.fpr_limit, reps=a.reps, device_ms_per_map_median=statistics.median(times),
+               device_ms_per_map_min=min(times), device_ms_per_map_max=max(times), pixel_auroc=auroc, au_pro=aupro,
+               repeat_bitwise_equal=bool(again[0] == auroc and again[1] == aupro),
+               bytes_per_pixel_floor=80, floor_ms_at_7_7_tbps=n * 80 / 7.7e12 * 1e3)
+    if a.host:
+        from oracle import localisation_oracle as L
+
+        h_maps = maps.cpu().numpy()
+        t0 = time.perf_counter()
+        h_auc = metrics.pixel_auroc(h_maps, masks)
+        res["host_pixel_auroc_s"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        h_pro = L.au_pro(list(h_maps), list(masks), a.fpr_limit)
+        res["host_au_pro_oracle_s"] = time.perf_counter() - t0
+        res["abs_diff_pixel_auroc"] = abs(h_auc - auroc)
+        res["abs_diff_au_pro"] = abs(h_pro - aupro)
+    print(json.dumps(res))
+
+
+if __name__ == "__main__":
+    main()
