@@ -13,7 +13,7 @@ from ctypes import c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_void_
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # ADSR_LIB: developer override for A/B timing of two builds in one session (tools/build_variant.sh); never a fallback
 LIB_PATH = os.environ.get("ADSR_LIB") or os.path.join(_HERE, "libadsr_b200.so")
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 ACT_NONE, ACT_LRELU, ACT_GELU, ACT_RELU = 0, 1, 2, 3
 OUT_ROWS, OUT_PIXEL_SHUFFLE2 = 0, 1

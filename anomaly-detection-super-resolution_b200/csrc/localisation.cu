@@ -1,5 +1,5 @@
-// Localisation metrics of one anomaly map over a whole test set: pixel AUROC and AU-PRO@alpha, exact (no threshold binning) and
-// deterministic.  Both come from ONE descending order of all pixels by score.
+// Localisation metrics of one anomaly map over a whole test set: pixel AUROC, AU-PRO@alpha, pixel AP and F1-max with its threshold,
+// exact (no threshold binning) and deterministic.  All of them come from ONE descending order of all pixels by score.
 //
 // Sort: a stable LSD radix sort of (key, region index) pairs, 4 passes of 8 bits.  The key is the fp32 score made order-preserving and
 // complemented (descending order = ascending keys; -0.0 canonicalised to +0.0), formed on the fly by the first pass, which also counts
@@ -16,6 +16,17 @@
 // seg_tile_kernel (tile aggregates) -> seg_scan_kernel (one CTA: exclusive scan over the tiles) -> seg_curve_kernel (per-tile
 // contributions) -> finish_kernel (one CTA, fixed order).  Everything is integer except the per-run area terms, which are fp64 values
 // of integer prefixes added in a fixed order: bitwise the same on every run, and for the same pixel sequence however it was batched.
+//
+// Precision-recall, from the same run ends.  With d_k / o_k = cumulative defect / defect-free pixels at the end of run k and
+// N_def = n - n_ok:
+//   pixel AP  = sum_k (d_k - d_{k-1}) / N_def * d_k / (d_k + o_k)   (= sklearn.metrics.average_precision_score, ties included);
+//   F1-max    = max_k 2 d_k / (d_k + o_k + N_def), the fractions compared exactly (128-bit cross products), a tie going to the
+//               earlier run (higher score): a unique answer whatever the reduction order;
+//   threshold = the fp32 score of that run (decoded from its key, -0.0 reported as +0.0): `score >= threshold` selects exactly the
+//               pixels that reach F1-max.
+// Only runs holding a defect pixel are evaluated: a run without one adds 0 to AP, and its F1 is at most that of the run before it
+// (same d, larger o), equal only when both are 0, which the tie rule and the final run (d = N_def >= 1) already settle.  The AP
+// terms are fp64 sums in a fixed order like the area; the F1 candidates are reduced by the exact max.
 #include "adsr_kernels.h"
 
 namespace adsr {
@@ -42,6 +53,11 @@ __device__ __forceinline__ uint32_t desc_key(float f) {
 __device__ __forceinline__ u64 warp_sum(u64 v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// inverse of desc_key (the map is its own inverse on non-NaN keys): the fp32 score of a key, +0.0 for a zero
+__device__ __forceinline__ float key_score(uint32_t k) {
+    return __uint_as_float((k & 0x80000000u) ? k : (~k & 0x7fffffffu));
 }
 
 // ---------------------------------------------------------------------------------------------------------- radix sort
@@ -315,23 +331,64 @@ struct CurveParams {
     double inv_n_ok;
     double inv_pro;        // 1 / (n_regions * 2^63)
     double alpha;
+    u64 n_def;             // defect pixels, n - n_ok
 };
+
+// F1 of a run end as an exact fraction: F1 = 2 num / den, num = d_k, den = d_k + o_k + N_def (< 2^64: the products below fit 128 bits)
+struct F1Cand {
+    u64 num, den;
+    uint32_t key;          // the run's key
+};
+
+__device__ __forceinline__ F1Cand f1_identity() {
+    F1Cand c;
+    c.num = 0, c.den = 1, c.key = 0xffffffffu;
+    return c;
+}
+
+// a beats b: a larger fraction, or the same one at a smaller key (an earlier run, a higher score).  A total order on distinct keys,
+// and every key ends one run only, so the max does not depend on the order of the reduction.
+__device__ __forceinline__ bool f1_better(const F1Cand& a, const F1Cand& b) {
+    const u128 l = static_cast<u128>(a.num) * b.den, r = static_cast<u128>(b.num) * a.den;
+    return l > r || (l == r && a.key < b.key);
+}
+
+// lane 0 gets the warp's sum, added in a fixed order
+__device__ __forceinline__ double warp_sum_fixed(double v) {
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    return v;
+}
+
+__device__ __forceinline__ F1Cand warp_f1_max(F1Cand c) {
+    for (int o = 16; o > 0; o >>= 1) {
+        F1Cand x;
+        x.num = __shfl_xor_sync(0xffffffffu, c.num, o);
+        x.den = __shfl_xor_sync(0xffffffffu, c.den, o);
+        x.key = __shfl_xor_sync(0xffffffffu, c.key, o);
+        if (f1_better(x, c)) c = x;
+    }
+    return c;
+}
 
 __global__ void __launch_bounds__(kThreads) seg_curve_kernel(const uint32_t* __restrict__ keys, const int32_t* __restrict__ regs,
                                                              const int64_t* __restrict__ sizes, const Seg* __restrict__ tile_prefix,
-                                                             const CurveParams p, u128* __restrict__ part_num, double* __restrict__ part_area) {
+                                                             const CurveParams p, u128* __restrict__ part_num, double* __restrict__ part_area,
+                                                             double* __restrict__ part_ap, F1Cand* __restrict__ part_f1) {
     __shared__ ScanStage st;
     __shared__ Seg sh[kThreads];
     __shared__ double red_a[kThreads];
     __shared__ u128 red_n[kThreads];
+    __shared__ double warp_ap[kThreads / 32];
+    __shared__ F1Cand warp_f1[kThreads / 32];
     const int tid = threadIdx.x;
     const long long base = static_cast<long long>(blockIdx.x) * kScanTile;
     stage_tile(st, keys, regs, p.n, base);
     Seg total;
     const Seg ex = block_exclusive_scan(thread_aggregate(st, sizes, p.n_regions, p.n, base), sh, &total);
     Seg run = combine(tile_prefix[blockIdx.x], ex);
-    double area = 0.0;
+    double area = 0.0, ap = 0.0;
     u128 num = 0;
+    F1Cand f1 = f1_identity();
     for (int q = 0; q < kScanItems; ++q) {
         const int j = tid * kScanItems + q;
         const long long i = base + j;
@@ -340,6 +397,13 @@ __global__ void __launch_bounds__(kThreads) seg_curve_kernel(const uint32_t* __r
         if (i + 1 < p.n && st.key[1 + j] == st.key[2 + j]) continue;     // not the last pixel of its run
         const u64 ok_run = run.ok - run.sok, def_run = run.def - run.sdef;
         num += static_cast<u128>(def_run) * static_cast<u128>(2ull * (static_cast<u64>(p.n_ok) - run.ok) + ok_run);
+        if (def_run) {                                                  // precision-recall: runs with a defect pixel only
+            const u64 seen = run.def + run.ok;
+            ap += static_cast<double>(def_run) * (static_cast<double>(run.def) / static_cast<double>(seen));
+            F1Cand c;
+            c.num = run.def, c.den = seen + p.n_def, c.key = st.key[1 + j];
+            if (f1_better(c, f1)) f1 = c;
+        }
         const double x0 = static_cast<double>(run.sok) * p.inv_n_ok;
         if (x0 < p.alpha) {
             double x1 = static_cast<double>(run.ok) * p.inv_n_ok;
@@ -351,6 +415,12 @@ __global__ void __launch_bounds__(kThreads) seg_curve_kernel(const uint32_t* __r
             }
             area += (x1 - x0) * (y0 + y1) * 0.5;
         }
+    }
+    ap = warp_sum_fixed(ap);
+    f1 = warp_f1_max(f1);
+    if ((tid & 31) == 0) {
+        warp_ap[tid >> 5] = ap;
+        warp_f1[tid >> 5] = f1;
     }
     red_a[tid] = area;
     red_n[tid] = num;
@@ -365,29 +435,47 @@ __global__ void __launch_bounds__(kThreads) seg_curve_kernel(const uint32_t* __r
     if (tid == 0) {
         part_area[blockIdx.x] = red_a[0];
         part_num[blockIdx.x] = red_n[0];
+        double a = 0.0;
+        F1Cand best = f1_identity();
+        for (int w = 0; w < kThreads / 32; ++w) {
+            a += warp_ap[w];
+            if (f1_better(warp_f1[w], best)) best = warp_f1[w];
+        }
+        part_ap[blockIdx.x] = a;
+        part_f1[blockIdx.x] = best;
     }
 }
 
-// one CTA: out = {pixel AUROC, AU-PRO@alpha, NaN scores, defect-free pixels seen, bad region indices}
-__global__ void __launch_bounds__(kThreads) finish_kernel(const u128* __restrict__ part_num, const double* __restrict__ part_area, int n_tiles,
-                                                          const u64* __restrict__ counters, long long n, long long n_ok, double alpha,
-                                                          double* __restrict__ out) {
+// one CTA: out = {pixel AUROC, AU-PRO@alpha, NaN scores, defect-free pixels seen, bad region indices, pixel AP, F1-max, F1 threshold}
+__global__ void __launch_bounds__(kThreads) finish_kernel(const u128* __restrict__ part_num, const double* __restrict__ part_area,
+                                                          const double* __restrict__ part_ap, const F1Cand* __restrict__ part_f1,
+                                                          int n_tiles, const u64* __restrict__ counters, long long n, long long n_ok,
+                                                          double alpha, double* __restrict__ out) {
     __shared__ double red_a[kThreads];
     __shared__ u128 red_n[kThreads];
+    __shared__ double red_p[kThreads];
+    __shared__ F1Cand red_f[kThreads];
     const int tid = threadIdx.x;
-    double a = 0.0;
+    double a = 0.0, ap = 0.0;
     u128 s = 0;
+    F1Cand f1 = f1_identity();
     for (int t = tid; t < n_tiles; t += kThreads) {
         a += part_area[t];
         s += part_num[t];
+        ap += part_ap[t];
+        if (f1_better(part_f1[t], f1)) f1 = part_f1[t];
     }
     red_a[tid] = a;
     red_n[tid] = s;
+    red_p[tid] = ap;
+    red_f[tid] = f1;
     __syncthreads();
     for (int k = kThreads / 2; k > 0; k >>= 1) {
         if (tid < k) {
             red_a[tid] += red_a[tid + k];
             red_n[tid] += red_n[tid + k];
+            red_p[tid] += red_p[tid + k];
+            if (f1_better(red_f[tid + k], red_f[tid])) red_f[tid] = red_f[tid + k];
         }
         __syncthreads();
     }
@@ -398,12 +486,15 @@ __global__ void __launch_bounds__(kThreads) finish_kernel(const u128* __restrict
         out[2] = static_cast<double>(counters[0]);
         out[3] = static_cast<double>(counters[1]);
         out[4] = static_cast<double>(counters[2]);
+        out[5] = red_p[0] / n_def;
+        out[6] = 2.0 * static_cast<double>(red_f[0].num) / static_cast<double>(red_f[0].den);
+        out[7] = static_cast<double>(key_score(red_f[0].key));
     }
 }
 
 // ---------------------------------------------------------------------------------------------------------- workspace
 struct Layout {
-    size_t keys_a, keys_b, vals_a, vals_b, hist, digit_tot, counters, agg, part_num, part_area, total;
+    size_t keys_a, keys_b, vals_a, vals_b, hist, digit_tot, counters, agg, part_num, part_area, part_ap, part_f1, total;
     int sort_tiles, scan_tiles;
 };
 
@@ -428,6 +519,8 @@ bool make_layout(long long n, Layout& L) {
     L.agg = take(static_cast<size_t>(ct) * sizeof(Seg));
     L.part_num = take(static_cast<size_t>(ct) * sizeof(u128));
     L.part_area = take(static_cast<size_t>(ct) * sizeof(double));
+    L.part_ap = take(static_cast<size_t>(ct) * sizeof(double));
+    L.part_f1 = take(static_cast<size_t>(ct) * sizeof(F1Cand));
     L.total = off;
     return true;
 }
@@ -460,6 +553,8 @@ extern "C" int adsr_localisation_metrics(const float* scores, const int32_t* reg
     Seg* agg = reinterpret_cast<Seg*>(ws + L.agg);
     u128* part_num = reinterpret_cast<u128*>(ws + L.part_num);
     double* part_area = reinterpret_cast<double*>(ws + L.part_area);
+    double* part_ap = reinterpret_cast<double*>(ws + L.part_ap);
+    F1Cand* part_f1 = reinterpret_cast<F1Cand*>(ws + L.part_f1);
 
     if (cudaMemsetAsync(counters, 0, 3 * sizeof(u64), s) != cudaSuccess) return ADSR_ERR_CUDA;
     // pass 0 reads the scores and region indices and writes buffer 1; passes alternate 1 -> 0 -> 1 -> 0: the sorted pairs end in buffer 0
@@ -490,7 +585,8 @@ extern "C" int adsr_localisation_metrics(const float* scores, const int32_t* reg
     p.inv_n_ok = 1.0 / static_cast<double>(n_ok);
     p.inv_pro = 1.0 / (static_cast<double>(n_regions) * static_cast<double>(kProOne));
     p.alpha = fpr_limit;
-    seg_curve_kernel<<<L.scan_tiles, kThreads, 0, s>>>(keys[0], vals[0], region_sizes, agg, p, part_num, part_area);
-    finish_kernel<<<1, kThreads, 0, s>>>(part_num, part_area, L.scan_tiles, counters, n, n_ok, fpr_limit, out);
+    p.n_def = static_cast<u64>(n - n_ok);
+    seg_curve_kernel<<<L.scan_tiles, kThreads, 0, s>>>(keys[0], vals[0], region_sizes, agg, p, part_num, part_area, part_ap, part_f1);
+    finish_kernel<<<1, kThreads, 0, s>>>(part_num, part_area, part_ap, part_f1, L.scan_tiles, counters, n, n_ok, fpr_limit, out);
     return cudaGetLastError() == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
 }

@@ -64,6 +64,11 @@ def parse_args(argv=None):
                    help='write <output-dir>/maps/<split>/<stem>_ssim.npy and <stem>_se.npy (float32 HxW); implies --anomaly-maps')
     p.add_argument('--au-pro', type=float, nargs='?', const=0.3, default=None, metavar='FPR_LIMIT',
                    help='also report the AU-PRO of both maps up to this false-positive rate (bare flag: 0.3); needs --mask-dir')
+    p.add_argument('--pr-metrics', action='store_true', default=False,
+                   help='also report the pixel AP and the F1-max of both maps with the threshold that attains it; needs --mask-dir')
+    p.add_argument('--save-segmentation', action='store_true', default=False,
+                   help='write <output-dir>/segmentation/<split>/<stem>_{ssim,se}.png: each map thresholded at its F1-max threshold '
+                        '(uint8 0 / 255); needs --mask-dir, implies --pr-metrics')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
 
@@ -76,6 +81,8 @@ def parse_args(argv=None):
             p.error('--au-pro needs --mask-dir (the ground-truth masks define the defect regions)')
         if not 0.0 < args.au_pro <= 1.0:
             p.error(f'--au-pro: the false-positive-rate limit must be in (0, 1], got {args.au_pro}')
+    if (args.pr_metrics or args.save_segmentation) and args.mask_dir is None:
+        p.error('--pr-metrics and --save-segmentation need --mask-dir (the ground-truth masks label the defect pixels)')
     return args
 
 
@@ -431,7 +438,8 @@ def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str,
 
 def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: bool, batch_size: Optional[int] = None,
                      anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
-                     save_maps: bool = False, au_pro: Optional[float] = None):
+                     save_maps: bool = False, au_pro: Optional[float] = None, pr_metrics: bool = False,
+                     save_segmentation: bool = False):
     """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
 
     anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
@@ -439,7 +447,11 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     printed on a `Map AUCs - ...` line before the `Test AUCs - ...` line.  mask_dir adds the pixel-level AUROC of both maps
     (pixel_auroc_ssim / pixel_auroc_se; single process only), ranked on the device by metrics.LocalisationAccumulator.  au_pro (an FPR
     limit in (0, 1], needs mask_dir) adds the AU-PRO of both maps (au_pro_ssim / au_pro_se, pro_fpr_limit), printed on a `Map PRO - ...`
-    line before the `Map AUCs - ...` line.  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
+    line before the `Map AUCs - ...` line.  pr_metrics (needs mask_dir) adds the pixel AP and the F1-max of both maps with the score that
+    attains it (pixel_ap_{ssim,se}, f1_max_{ssim,se}, f1_threshold_{ssim,se}), printed on a `Map PR - ...` line before the `Map PRO`
+    line, or before the `Map AUCs` line without one.  The F1 threshold is an oracle threshold: picked with the ground truth it is scored
+    on.  save_segmentation (needs mask_dir, implies pr_metrics) writes each map thresholded at its F1 threshold as a uint8 0 / 255 mask
+    to <output_dir>/segmentation/<split>/<stem>_{ssim,se}.png.  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
     from .model import Model
 
     if au_pro is not None:
@@ -447,6 +459,9 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
             raise ValueError("au_pro needs mask_dir: the ground-truth masks define the defect regions")
         if not 0.0 < float(au_pro) <= 1.0:
             raise ValueError(f"au_pro: the false-positive-rate limit must be in (0, 1], got {au_pro}")
+    if (pr_metrics or save_segmentation) and mask_dir is None:
+        raise ValueError("pr_metrics and save_segmentation need mask_dir: the ground-truth masks label the defect pixels")
+    pr_metrics = pr_metrics or save_segmentation
     anomaly_maps = anomaly_maps or mask_dir is not None or save_maps
     scale = opt.scale[-1] if isinstance(opt.scale, list) else int(opt.scale)
     rank, world = _dist_info()
@@ -536,12 +551,25 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                 f"max SE: {res['auc_map_se']:.4f}")
         if mask_dir is not None:
             limit = 0.3 if au_pro is None else float(au_pro)
-            (pa_ssim, pro_ssim), (pa_se, pro_se) = loc.finish(limit)
-            res.update(pixel_auroc_ssim=pa_ssim, pixel_auroc_se=pa_se)
+            m_ssim, m_se = loc.results(limit)
+            res.update(pixel_auroc_ssim=m_ssim.pixel_auroc, pixel_auroc_se=m_se.pixel_auroc)
             line += f", pixel AUROC 1-SSIM: {res['pixel_auroc_ssim']:.4f}, pixel AUROC SE: {res['pixel_auroc_se']:.4f}"
+            if pr_metrics:
+                res.update(pixel_ap_ssim=m_ssim.pixel_ap, pixel_ap_se=m_se.pixel_ap, f1_max_ssim=m_ssim.f1_max, f1_max_se=m_se.f1_max,
+                           f1_threshold_ssim=m_ssim.f1_threshold, f1_threshold_se=m_se.f1_threshold)
+                print(f"Map PR - pixel AP 1-SSIM: {m_ssim.pixel_ap:.4f}, pixel AP SE: {m_se.pixel_ap:.4f}, "
+                      f"F1-max 1-SSIM: {m_ssim.f1_max:.4f} (thr {m_ssim.f1_threshold:g}), "
+                      f"F1-max SE: {m_se.f1_max:.4f} (thr {m_se.f1_threshold:g})")
+            if save_segmentation:                             # the accumulator holds the images in `ids` order
+                for j, (kind, m) in enumerate((('ssim', m_ssim), ('se', m_se))):
+                    for i, seg in zip(ids, loc.segmentation(j, m.f1_threshold)):
+                        name = os.path.splitext(os.path.basename(entries[i][2]))[0]
+                        d = Path(output_dir) / 'segmentation' / entries[i][1]
+                        d.mkdir(parents=True, exist_ok=True)
+                        Image.fromarray(seg.astype(np.uint8) * 255).save(str(d / f'{name}_{kind}.png'))
             if au_pro is not None:
-                res.update(au_pro_ssim=pro_ssim, au_pro_se=pro_se, pro_fpr_limit=limit)
-                print(f"Map PRO - AU-PRO@{limit:g} 1-SSIM: {pro_ssim:.4f}, AU-PRO@{limit:g} SE: {pro_se:.4f}")
+                res.update(au_pro_ssim=m_ssim.au_pro, au_pro_se=m_se.au_pro, pro_fpr_limit=limit)
+                print(f"Map PRO - AU-PRO@{limit:g} 1-SSIM: {m_ssim.au_pro:.4f}, AU-PRO@{limit:g} SE: {m_se.au_pro:.4f}")
         print(line)
     print(f"Test AUCs - SSIM(best ws={best_ws}): {auc_ssim:.4f}, MSE: {auc_mse:.4f}, PSNR: {auc_psnr:.4f}")
     return res
@@ -584,7 +612,8 @@ def main(argv=None):
     out_dir = args.output_dir or (os.path.join(args.run_dir, 'eval_results') if args.run_dir else './workspace/eval_results')
     return evaluate_on_test(opt, ckpt_path, out_dir, args.save_images, batch_size=args.batch_size, anomaly_maps=args.anomaly_maps,
                             map_window_size=args.map_window_size, map_sigma=args.map_sigma, mask_dir=args.mask_dir,
-                            save_maps=args.save_maps, au_pro=args.au_pro)
+                            save_maps=args.save_maps, au_pro=args.au_pro, pr_metrics=args.pr_metrics,
+                            save_segmentation=args.save_segmentation)
 
 
 if __name__ == "__main__":

@@ -4,7 +4,7 @@ scorer the evaluator uses.  No CPU fallback: a CUDA device and libadsr_b200.so a
 """
 from __future__ import annotations
 
-from typing import Optional, Sequence
+from typing import NamedTuple, Optional, Sequence
 
 import numpy as np
 import torch
@@ -115,14 +115,26 @@ def _map_pieces(maps):
     return pieces, shapes
 
 
+class LocalisationMetrics(NamedTuple):
+    """The localisation numbers of one anomaly map over a whole test set (LocalisationAccumulator.results).  f1_threshold is an oracle
+    threshold: it is chosen with the ground truth of the very pixels it is scored on (anomalib's adaptive threshold is also picked from
+    labelled data, but from a validation set)."""
+    pixel_auroc: float
+    au_pro: float
+    pixel_ap: float         # area under the pixel precision-recall curve (sklearn's average_precision_score)
+    f1_max: float           # the best pixel F1 over all thresholds
+    f1_threshold: float     # the fp32 score that attains it: `map >= f1_threshold` is the F1-max defect mask
+
+
 class LocalisationAccumulator:
-    """Pixel AUROC and AU-PRO of `n_maps` anomaly maps over a whole test set, fed one batch at a time.
+    """Pixel AUROC, AU-PRO, pixel AP and F1-max of `n_maps` anomaly maps over a whole test set, fed one batch at a time.
 
     append(maps, masks): maps = one entry per map, each a CUDA fp32 [B, H, W] tensor or a sequence of [H, W] tensors (any sizes);
     masks = the host masks of the same B images (non-zero = defect).  The maps are copied on the device into one growing buffer per map
     (no device -> host copy); each mask is labelled once on the host (scipy.ndimage.label, 8-connectivity) and its per-pixel region
-    indices are shared by all maps.  finish(fpr_limit) runs adsr_localisation_metrics once per map and returns
-    [(pixel_auroc, au_pro), ...]: the same numbers for the same image sequence however it was split into batches."""
+    indices are shared by all maps.  results(fpr_limit) runs adsr_localisation_metrics once per map and returns one LocalisationMetrics
+    per map, finish(fpr_limit) the [(pixel_auroc, au_pro), ...] part of it: the same numbers for the same image sequence however it was
+    split into batches.  segmentation(map_index, threshold) thresholds the accumulated maps into per-image defect masks."""
 
     def __init__(self, n_maps: int = 1):
         self.n_maps = int(n_maps)
@@ -131,6 +143,7 @@ class LocalisationAccumulator:
         self.n = 0
         self.n_ok = 0
         self._sizes = []                              # host int64 region sizes, one array per image with defects
+        self._shapes = []                             # (H, W) of every appended image, in append order
 
     @property
     def n_regions(self) -> int:
@@ -179,12 +192,13 @@ class LocalisationAccumulator:
         if n_new:
             self._regions[self.n:self.n + n_new].copy_(torch.from_numpy(np.concatenate(regions)))
         self._sizes += sizes
+        self._shapes += shapes
         self.n += n_new
         self.n_ok += n_ok
 
-    def finish(self, fpr_limit: float = 0.3):
-        """[(pixel AUROC, AU-PRO@fpr_limit)] per map.  ValueError: fpr_limit outside (0, 1], no defect region (R == 0), no defect-free
-        pixel, or a NaN in a map."""
+    def results(self, fpr_limit: float = 0.3) -> list[LocalisationMetrics]:
+        """One LocalisationMetrics per map (AU-PRO up to FPR = fpr_limit).  ValueError: fpr_limit outside (0, 1], no defect region
+        (R == 0), no defect-free pixel, or a NaN in a map."""
         fpr_limit = float(fpr_limit)
         if not 0.0 < fpr_limit <= 1.0:
             raise ValueError(f"fpr_limit must be in (0, 1], got {fpr_limit}")
@@ -195,7 +209,7 @@ class LocalisationAccumulator:
         device = self._regions.device
         sizes = torch.from_numpy(np.concatenate(self._sizes)).to(device)
         ws = torch.empty(ops.localisation_workspace_bytes(self.n), dtype=torch.uint8, device=device)
-        out = torch.empty(self.n_maps, 5, dtype=torch.float64, device=device)
+        out = torch.empty(self.n_maps, 8, dtype=torch.float64, device=device)
         for j, buf in enumerate(self._maps):
             ops.localisation_metrics(buf[:self.n], self._regions[:self.n], sizes, self.n_ok, fpr_limit, ws, out[j])
         res = out.cpu().numpy()
@@ -204,7 +218,30 @@ class LocalisationAccumulator:
                 raise ValueError(f"map {j} holds {int(res[j, 2])} NaN scores")
             if res[j, 3] != self.n_ok or res[j, 4]:
                 raise RuntimeError(f"localisation metrics: inconsistent region indices on the device (map {j}: {res[j, 2:]})")
-        return [(float(r[0]), float(r[1])) for r in res]
+        return [LocalisationMetrics(*(float(r[k]) for k in (0, 1, 5, 6, 7))) for r in res]
+
+    def finish(self, fpr_limit: float = 0.3):
+        """[(pixel AUROC, AU-PRO@fpr_limit)] per map, from results() (same checks and errors)."""
+        return [(r.pixel_auroc, r.au_pro) for r in self.results(fpr_limit)]
+
+    def segmentation(self, map_index: int, threshold: float) -> list[np.ndarray]:
+        """Predicted defect masks: bool [H, W] host arrays `map >= threshold` of map `map_index`, one per appended image in append order
+        (one comparison on the device over the accumulated map, one device -> host copy).  With the f1_threshold of results() they are
+        the masks that attain F1-max.  The comparison is that of the fp32 map with the exact double `threshold`."""
+        j = int(map_index)
+        if not 0 <= j < self.n_maps:
+            raise IndexError(f"segmentation: map {map_index} of {self.n_maps}")
+        t = np.float32(threshold)
+        if t < threshold:                             # the smallest fp32 >= threshold: x >= t32 <=> x >= threshold for every fp32 x
+            t = np.nextafter(t, np.float32(np.inf))
+        if self.n == 0:
+            return []
+        flat = (self._maps[j][:self.n] >= float(t)).cpu().numpy()
+        out, off = [], 0
+        for h, w in self._shapes:
+            out.append(flat[off:off + h * w].reshape(h, w))
+            off += h * w
+        return out
 
 
 def _on_device(maps) -> bool:
@@ -221,6 +258,24 @@ def au_pro(maps, masks, fpr_limit: float = 0.3) -> float:
     acc = LocalisationAccumulator(1)
     acc.append([maps], masks)
     return acc.finish(fpr_limit)[0][1]
+
+
+def pixel_ap(maps, masks) -> float:
+    """Pixel-level average precision (area under the precision-recall curve; sklearn.metrics.average_precision_score over every pixel,
+    ties included): maps = CUDA fp32 [N, H, W] tensor or a sequence of [H, W] tensors, masks = host arrays of the same shapes (non-zero
+    = defect).  Computed on the device (adsr_localisation_metrics)."""
+    acc = LocalisationAccumulator(1)
+    acc.append([maps], masks)
+    return acc.results()[0].pixel_ap
+
+
+def f1_max(maps, masks) -> tuple[float, float]:
+    """(best pixel F1 over all thresholds, the fp32 score that attains it; on a tie the higher one) of CUDA maps against host masks,
+    inputs as pixel_ap.  `map >= threshold` reproduces the F1.  An oracle threshold: chosen on the ground truth it is scored on."""
+    acc = LocalisationAccumulator(1)
+    acc.append([maps], masks)
+    r = acc.results()[0]
+    return r.f1_max, r.f1_threshold
 
 
 def pixel_auroc(maps, masks) -> float:

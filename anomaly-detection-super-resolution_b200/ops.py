@@ -349,16 +349,17 @@ def localisation_workspace_bytes(n: int) -> int:
 
 def localisation_metrics(scores: torch.Tensor, regions: torch.Tensor, region_sizes: torch.Tensor, n_ok: int, fpr_limit: float,
                          workspace: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
-    """Pixel AUROC and AU-PRO@fpr_limit of one map: scores fp32 [n], regions int32 [n] (-1 = defect-free, else an index into
-    region_sizes int64 [R]), n_ok defect-free pixels -> out fp64 [5] = (pixel AUROC, AU-PRO, NaN scores, defect-free pixels seen,
-    out-of-range region indices).  workspace: uint8 [>= localisation_workspace_bytes(n)].  Sixteen kernels, no synchronisation."""
+    """Pixel AUROC, AU-PRO@fpr_limit, pixel AP and F1-max of one map: scores fp32 [n], regions int32 [n] (-1 = defect-free, else an
+    index into region_sizes int64 [R]), n_ok defect-free pixels -> out fp64 [8] = (pixel AUROC, AU-PRO, NaN scores, defect-free pixels
+    seen, out-of-range region indices, pixel AP, F1-max, F1 threshold).  workspace: uint8 [>= localisation_workspace_bytes(n)].
+    Sixteen kernels, no synchronisation."""
     for t, name, dt in ((scores, "scores", torch.float32), (regions, "regions", torch.int32), (region_sizes, "region_sizes", torch.int64),
                         (workspace, "workspace", torch.uint8), (out, "out", torch.float64)):
         _cuda(t, name)
         if t.dtype != dt or not t.is_contiguous():
             raise ValueError(f"localisation_metrics: {name} must be a contiguous {dt} tensor")
     n = scores.numel()
-    if regions.numel() != n or out.numel() < 5:
+    if regions.numel() != n or out.numel() < 8:
         raise ValueError(f"localisation_metrics: {n} scores, {regions.numel()} region indices, out of {out.numel()} values")
     _t = _begin()
     check(lib().adsr_localisation_metrics(ptr(scores), ptr(regions), n, ptr(region_sizes), region_sizes.numel(), int(n_ok),

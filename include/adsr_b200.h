@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 16
+#define ADSR_ABI_VERSION 17
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -266,7 +266,8 @@ int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B,
                       int win_size, float sigma, float* ssim_map, float* se_map, float* scratch,
                       double* map_max, void* stream);
 
-/* Localisation metrics of ONE anomaly map over a whole test set: pixel AUROC and AU-PRO@fpr_limit, exact (no threshold binning).
+/* Localisation metrics of ONE anomaly map over a whole test set: pixel AUROC, AU-PRO@fpr_limit, pixel AP and F1-max with its threshold,
+ * exact (no threshold binning).
  * scores: fp32 [n] (all pixels of all images, higher = more anomalous); regions: int32 [n], -1 = defect-free pixel, else the index of
  * the pixel's defect region (8-connected component of a ground-truth mask) in region_sizes: int64 [n_regions] pixel counts.
  * n_ok = number of defect-free pixels.  All pixels are ranked by score, descending (-0.0 = +0.0); equal scores form one curve point.
@@ -274,9 +275,16 @@ int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B,
  *   AU-PRO      = (1 / fpr_limit) * trapezoid area under (FPR, PRO) from FPR 0 to fpr_limit, the crossing segment cut by linear
  *                 interpolation; FPR = share of the defect-free pixels at or above the score, PRO = mean over the regions of the share
  *                 of the region's pixels at or above it.
- * out: fp64 [5] = {pixel AUROC, AU-PRO, NaN scores, defect-free pixels seen, region indices out of range}: the last three are checks
- * for the caller (the metrics are only valid when they read 0, n_ok, 0).  workspace: adsr_localisation_workspace_bytes(n) bytes, 16-byte
- * aligned.  Deterministic (integer sort and counts, fixed-order fp64 area) and a function of the pixel sequence alone.
+ * With runs = maximal sets of equal scores in that order, and d_k / o_k = the defect / defect-free pixels at or above run k's score,
+ * N_def = n - n_ok:
+ *   pixel AP    = sum_k (d_k - d_{k-1}) / N_def * d_k / (d_k + o_k) = sklearn.metrics.average_precision_score(regions >= 0, scores);
+ *   F1-max      = max_k 2 d_k / (d_k + o_k + N_def), exact (the fractions are compared as integers), a tie going to the higher score;
+ *   F1 threshold = the fp32 score of that run (-0.0 reported as +0.0): `scores >= threshold` is the mask that attains F1-max.  It is
+ *                 an oracle threshold: chosen with the ground truth of the very pixels it is scored on.
+ * out: fp64 [8] = {pixel AUROC, AU-PRO, NaN scores, defect-free pixels seen, region indices out of range, pixel AP, F1-max,
+ * F1 threshold}: indices 2-4 are checks for the caller (the metrics are only valid when they read 0, n_ok, 0).  workspace:
+ * adsr_localisation_workspace_bytes(n) bytes, 16-byte aligned.  Deterministic (integer sort and counts, exact F1 max, fixed-order fp64
+ * area and AP sums) and a function of the pixel sequence alone.
  * ADSR_ERR_BAD_SHAPE: n < 1, n_regions < 1, n_ok < 1, n_ok >= n, fpr_limit outside (0, 1], a NULL pointer or a short workspace. */
 int64_t adsr_localisation_workspace_bytes(int64_t n);
 int adsr_localisation_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes, int n_regions,

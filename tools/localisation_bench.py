@@ -1,10 +1,11 @@
-"""Device time of the localisation metrics (pixel AUROC + AU-PRO of one anomaly map over a whole test set, csrc/localisation.cu) on
-synthetic maps and masks: random rectangles and round blobs as defects, smoothed noise with raised scores on the defects as the map.
+"""Device time of the localisation metrics (pixel AUROC, AU-PRO, pixel AP and F1-max of one anomaly map over a whole test set,
+csrc/localisation.cu) on synthetic maps and masks: random rectangles and round blobs as defects, smoothed noise with raised scores on the defects as the map.
 
 Per repetition (CUDA events): the append of one map (device copy of every batch into the accumulator's buffer) and the finish (the
 sixteen kernels of adsr_localisation_metrics).  The default 1024 images of 256 x 256 are 67 M pixels per map: the sort's 16 bytes of
 pairs per pixel are far above the 126 MB of L2.  --host also times the host path of the same inputs (sklearn's roc_auc_score behind
-metrics.pixel_auroc on host arrays, the oracle's AU-PRO) and reports the agreement.  One JSON line, with the card and its power limit.
+metrics.pixel_auroc on host arrays, the oracle's AU-PRO, sklearn's average_precision_score, the oracle's F1-max) and reports the
+agreement.  One JSON line, with the card and its power limit.
 
     python tools/localisation_bench.py [--images 1024] [--side 256] [--reps 20] [--host]
 """
@@ -79,12 +80,13 @@ def main(argv=None):
     acc = metrics.LocalisationAccumulator(1)
     for s in range(0, a.images, a.batch):                   # host labelling + region upload happen here, once
         acc.append([maps[s:s + a.batch]], masks[s:s + a.batch])
-    (auroc, aupro), = acc.finish(a.fpr_limit)
+    r, = acc.results(a.fpr_limit)
+    auroc, aupro = r.pixel_auroc, r.au_pro
     n = acc.n
     buf, regions = acc._maps[0], acc._regions[:n]
     sizes = torch.from_numpy(np.concatenate(acc._sizes)).cuda()
     ws = torch.empty(ops.localisation_workspace_bytes(n), dtype=torch.uint8, device="cuda")
-    out = torch.empty(5, dtype=torch.float64, device="cuda")
+    out = torch.empty(8, dtype=torch.float64, device="cuda")
 
     def one():                                              # the device work of append (per-batch copies) + finish, one map
         off = 0
@@ -109,10 +111,12 @@ def main(argv=None):
     res = dict(tool="localisation_bench", gpu=name, power_limit_w=power, images=a.images, side=a.side, pixels_per_map=n,
                regions=acc.n_regions, fpr_limit=a.fpr_limit, reps=a.reps, device_ms_per_map_median=statistics.median(times),
                device_ms_per_map_min=min(times), device_ms_per_map_max=max(times), pixel_auroc=auroc, au_pro=aupro,
-               repeat_bitwise_equal=bool(again[0] == auroc and again[1] == aupro),
+               pixel_ap=r.pixel_ap, f1_max=r.f1_max, f1_threshold=r.f1_threshold,
+               repeat_bitwise_equal=bool(tuple(float(again[k]) for k in (0, 1, 5, 6, 7)) == tuple(r)),
                bytes_per_pixel_floor=80, floor_ms_at_7_7_tbps=n * 80 / 7.7e12 * 1e3)
     if a.host:
         from oracle import localisation_oracle as L
+        from oracle import pr_oracle as P
 
         h_maps = maps.cpu().numpy()
         t0 = time.perf_counter()
@@ -121,8 +125,17 @@ def main(argv=None):
         t0 = time.perf_counter()
         h_pro = L.au_pro(list(h_maps), list(masks), a.fpr_limit)
         res["host_au_pro_oracle_s"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        h_ap = P.pixel_ap(list(h_maps), list(masks))
+        res["host_pixel_ap_sklearn_s"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        h_f1, h_thr = P.f1_max(list(h_maps), list(masks))
+        res["host_f1_max_oracle_s"] = time.perf_counter() - t0
         res["abs_diff_pixel_auroc"] = abs(h_auc - auroc)
         res["abs_diff_au_pro"] = abs(h_pro - aupro)
+        res["abs_diff_pixel_ap"] = abs(h_ap - r.pixel_ap)
+        res["abs_diff_f1_max"] = abs(h_f1 - r.f1_max)
+        res["f1_threshold_equal"] = h_thr == r.f1_threshold
     print(json.dumps(res))
 
 
