@@ -27,6 +27,15 @@
 // Only runs holding a defect pixel are evaluated: a run without one adds 0 to AP, and its F1 is at most that of the run before it
 // (same d, larger o), equal only when both are 0, which the tie rule and the final run (d = N_def >= 1) already settle.  The AP
 // terms are fp64 sums in a fixed order like the area; the F1 candidates are reduced by the exact max.
+//
+// Two more entry points read the scores without sorting them, for thresholds calibrated on defect-free images:
+//   adsr_score_quantile: the exact k-th smallest score, by an MSD radix select over ascending keys (~desc_key), 4 passes of 8 bits.
+//     A pass = select_hist_kernel (digit histogram of the pixels whose higher digits equal the running prefix: per-warp shared
+//     histograms, integer atomics into one global histogram) + select_pick_kernel (one CTA: the digit that holds rank k, the new
+//     prefix and the rank left inside it, kept in device memory).  No scatter: ~16 B read per pixel over the 4 passes.
+//   adsr_threshold_metrics: one pass, `score >= threshold`, TP / FP / FN counts and the fixed-point PRO weight of the detected
+//     defect pixels (the AU-PRO curve's quantity at one threshold), per-CTA partials added by one CTA in a fixed order.
+// Both are integer-exact, deterministic and free of host synchronisation.
 #include "adsr_kernels.h"
 
 namespace adsr {
@@ -492,6 +501,200 @@ __global__ void __launch_bounds__(kThreads) finish_kernel(const u128* __restrict
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------- radix select
+// The streaming kernels below (select_hist_kernel, threshold_kernel) read the pixels in a grid-stride loop, with 16-byte loads when
+// the arrays are 16-byte aligned (kVec) and the < 4 pixels of the tail read by the first CTA.
+// Running state of the select, in device memory between the kernels: the rank still to find inside the pixels that match the prefix.
+struct SelectState {
+    u64 rank;              // 1-based rank inside the current prefix
+    u64 nan;               // NaN scores (excluded from the ranking)
+    uint32_t prefix;       // ascending key bits fixed so far
+    uint32_t empty;        // 1: fewer non-NaN scores than the rank asked for
+};
+static_assert(sizeof(SelectState) == 3 * sizeof(u64), "the select state lives in the 3 counters of the layout");
+
+// ascending key: order-preserving, so the k-th smallest key is the k-th smallest score
+__device__ __forceinline__ uint32_t asc_key(float f) { return ~desc_key(f); }
+
+template <bool kVec>
+__global__ void __launch_bounds__(kThreads) select_hist_kernel(const float* __restrict__ scores, long long n, int shift,
+                                                               u64* __restrict__ hist, SelectState* __restrict__ st) {
+    __shared__ unsigned int h[kThreads / 32][kBins];
+    const int tid = threadIdx.x, warp = tid >> 5;
+    for (int j = tid; j < (kThreads / 32) * kBins; j += kThreads) (&h[0][0])[j] = 0;
+    __syncthreads();
+    const uint32_t hi_mask = shift == 24 ? 0u : (0xffffffffu << (shift + 8));   // the digits above this pass
+    const uint32_t prefix = st->prefix & hi_mask;
+    u64 nan_c = 0;
+    auto one = [&](float f) {
+        if (f != f) {
+            ++nan_c;
+            return;
+        }
+        const uint32_t a = asc_key(f);
+        if (((a ^ prefix) & hi_mask) == 0) atomicAdd(&h[warp][(a >> shift) & (kBins - 1)], 1u);
+    };
+    const long long stride = static_cast<long long>(gridDim.x) * kThreads;
+    const long long first = static_cast<long long>(blockIdx.x) * kThreads + tid;
+    if (kVec) {
+        const long long n4 = n >> 2;
+        const float4* s4 = reinterpret_cast<const float4*>(scores);
+        for (long long v = first; v < n4; v += stride) {
+            const float4 f = s4[v];
+            one(f.x), one(f.y), one(f.z), one(f.w);
+        }
+        if (blockIdx.x == 0 && tid < (n & 3)) one(scores[(n4 << 2) + tid]);
+    } else {
+        for (long long i = first; i < n; i += stride) one(scores[i]);
+    }
+    __syncthreads();
+    unsigned int c = 0;
+#pragma unroll
+    for (int w = 0; w < kThreads / 32; ++w) c += h[w][tid];
+    if (c) atomicAdd(&hist[tid], static_cast<u64>(c));
+    if (shift == 24) {
+        nan_c = warp_sum(nan_c);
+        if ((tid & 31) == 0 && nan_c) atomicAdd(&st->nan, nan_c);
+    }
+}
+
+// one CTA: the digit holding the rank (first pass: rank k), the new prefix and the rank left inside it; clears the histogram for the
+// next pass.  The last pass writes out = {score, NaN count}.
+__global__ void __launch_bounds__(kThreads) select_pick_kernel(int shift, u64 k, u64* __restrict__ hist, SelectState* __restrict__ st,
+                                                               double* __restrict__ out) {
+    __shared__ u64 s[kBins];
+    const int tid = threadIdx.x;
+    const u64 c = hist[tid];
+    hist[tid] = 0;
+    s[tid] = c;
+    const bool first = shift == 24;
+    const u64 rank = first ? k : st->rank;
+    const uint32_t prefix = first ? 0u : st->prefix;
+    const bool empty = first ? false : st->empty != 0;
+    __syncthreads();
+    for (int d = 1; d < kBins; d <<= 1) {                       // inclusive scan of the digit counts
+        const u64 x = tid >= d ? s[tid - d] : 0;
+        __syncthreads();
+        s[tid] += x;
+        __syncthreads();
+    }
+    const u64 total = s[kBins - 1], before = s[tid] - c;
+    const bool none = empty || rank > total;                    // only NaNs can leave fewer scores than k <= n
+    if (!none && c && before < rank && rank <= s[tid]) {        // exactly one digit
+        const uint32_t p = prefix | (static_cast<uint32_t>(tid) << shift);
+        st->rank = rank - before;
+        st->prefix = p;
+        if (shift == 0) out[0] = static_cast<double>(key_score(~p));
+    }
+    if (tid == 0) {
+        if (first) st->empty = none;
+        if (shift == 0) {
+            if (none) out[0] = __longlong_as_double(0x7ff8000000000000LL);
+            out[1] = static_cast<double>(st->nan);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------- metrics at a threshold
+struct ThrCounts {
+    u128 pro;              // fixed-point PRO weight of the detected defect pixels
+    u64 tp, fp, fn, nan, bad;
+};
+
+__device__ __forceinline__ u128 warp_sum_u128(u128 v) {
+    for (int o = 16; o > 0; o >>= 1) {
+        const u64 lo = __shfl_xor_sync(0xffffffffu, static_cast<u64>(v), o);
+        const u64 hi = __shfl_xor_sync(0xffffffffu, static_cast<u64>(v >> 64), o);
+        v += (static_cast<u128>(hi) << 64) | lo;
+    }
+    return v;
+}
+
+template <bool kVec>
+__global__ void __launch_bounds__(kThreads) threshold_kernel(const float* __restrict__ scores, const int32_t* __restrict__ regions,
+                                                             const int64_t* __restrict__ sizes, int n_regions, long long n,
+                                                             float threshold, ThrCounts* __restrict__ part) {
+    __shared__ ThrCounts wsum[kThreads / 32];
+    const int tid = threadIdx.x;
+    u64 tp = 0, fp = 0, fn = 0, nan_c = 0, bad = 0;
+    u128 pro = 0;
+    auto one = [&](float f, int32_t r) {
+        const bool pred = f >= threshold, def = r >= 0;
+        nan_c += f != f;
+        bad += r < -1 || r >= n_regions || (def && sizes[r] < 1);
+        tp += pred && def;
+        fp += pred && !def;
+        fn += !pred && def;
+        if (pred && def && r < n_regions) {
+            const long long sz = sizes[r];
+            if (sz > 0) pro += kProOne / static_cast<u64>(sz);
+        }
+    };
+    const long long stride = static_cast<long long>(gridDim.x) * kThreads;
+    const long long first = static_cast<long long>(blockIdx.x) * kThreads + tid;
+    if (kVec) {
+        const long long n4 = n >> 2;
+        const float4* s4 = reinterpret_cast<const float4*>(scores);
+        const int4* r4 = reinterpret_cast<const int4*>(regions);
+        for (long long v = first; v < n4; v += stride) {
+            const float4 f = s4[v];
+            const int4 r = r4[v];
+            one(f.x, r.x), one(f.y, r.y), one(f.z, r.z), one(f.w, r.w);
+        }
+        if (blockIdx.x == 0 && tid < (n & 3)) one(scores[(n4 << 2) + tid], regions[(n4 << 2) + tid]);
+    } else {
+        for (long long i = first; i < n; i += stride) one(scores[i], regions[i]);
+    }
+    tp = warp_sum(tp), fp = warp_sum(fp), fn = warp_sum(fn), nan_c = warp_sum(nan_c), bad = warp_sum(bad);
+    pro = warp_sum_u128(pro);
+    if ((tid & 31) == 0) {
+        ThrCounts& w = wsum[tid >> 5];
+        w.pro = pro, w.tp = tp, w.fp = fp, w.fn = fn, w.nan = nan_c, w.bad = bad;
+    }
+    __syncthreads();
+    if (tid == 0) {
+        ThrCounts t = wsum[0];
+        for (int w = 1; w < kThreads / 32; ++w) {
+            t.pro += wsum[w].pro, t.tp += wsum[w].tp, t.fp += wsum[w].fp, t.fn += wsum[w].fn;
+            t.nan += wsum[w].nan, t.bad += wsum[w].bad;
+        }
+        part[blockIdx.x] = t;
+    }
+}
+
+// one CTA: out = {TP, FP, FN, TN, PRO@threshold, NaN scores, bad region indices}
+__global__ void __launch_bounds__(kThreads) threshold_finish_kernel(const ThrCounts* __restrict__ part, int n_parts, long long n,
+                                                                    int n_regions, double* __restrict__ out) {
+    __shared__ ThrCounts red[kThreads];
+    const int tid = threadIdx.x;
+    ThrCounts t = {};
+    for (int b = tid; b < n_parts; b += kThreads) {
+        t.pro += part[b].pro, t.tp += part[b].tp, t.fp += part[b].fp, t.fn += part[b].fn;
+        t.nan += part[b].nan, t.bad += part[b].bad;
+    }
+    red[tid] = t;
+    __syncthreads();
+    for (int s = kThreads / 2; s > 0; s >>= 1) {
+        if (tid < s) {
+            ThrCounts& a = red[tid];
+            const ThrCounts& b = red[tid + s];
+            a.pro += b.pro, a.tp += b.tp, a.fp += b.fp, a.fn += b.fn, a.nan += b.nan, a.bad += b.bad;
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {
+        const ThrCounts& r = red[0];
+        out[0] = static_cast<double>(r.tp);
+        out[1] = static_cast<double>(r.fp);
+        out[2] = static_cast<double>(r.fn);
+        out[3] = static_cast<double>(static_cast<u64>(n) - r.tp - r.fp - r.fn);
+        out[4] = n_regions > 0 ? u128_to_double(r.pro) / (static_cast<double>(n_regions) * static_cast<double>(kProOne))
+                               : __longlong_as_double(0x7ff8000000000000LL);
+        out[5] = static_cast<double>(r.nan);
+        out[6] = static_cast<double>(r.bad);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------- workspace
 struct Layout {
     size_t keys_a, keys_b, vals_a, vals_b, hist, digit_tot, counters, agg, part_num, part_area, part_ap, part_f1, total;
@@ -523,6 +726,15 @@ bool make_layout(long long n, Layout& L) {
     L.part_f1 = take(static_cast<size_t>(ct) * sizeof(F1Cand));
     L.total = off;
     return true;
+}
+
+// CTAs of the streaming kernels: 4 per SM (threshold_kernel's 60 registers allow 4 x 256 threads), never more than the sort tiles
+// (the threshold partials live in the histogram area of the layout, 2 KB per sort tile).
+int stream_grid(const Layout& L) {
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
+        sms = 148;
+    return L.sort_tiles < 4 * sms ? L.sort_tiles : 4 * sms;
 }
 
 }  // namespace
@@ -588,5 +800,54 @@ extern "C" int adsr_localisation_metrics(const float* scores, const int32_t* reg
     p.n_def = static_cast<u64>(n - n_ok);
     seg_curve_kernel<<<L.scan_tiles, kThreads, 0, s>>>(keys[0], vals[0], region_sizes, agg, p, part_num, part_area, part_ap, part_f1);
     finish_kernel<<<1, kThreads, 0, s>>>(part_num, part_area, part_ap, part_f1, L.scan_tiles, counters, n, n_ok, fpr_limit, out);
+    return cudaGetLastError() == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
+}
+
+extern "C" int adsr_score_quantile(const float* scores, int64_t n, int64_t k, void* workspace, int64_t workspace_bytes, double* out,
+                                   void* stream) {
+    using namespace adsr;
+    Layout L;
+    if (!make_layout(n, L) || k < 1 || k > n) return ADSR_ERR_BAD_SHAPE;
+    if (scores == nullptr || workspace == nullptr || out == nullptr || workspace_bytes < static_cast<int64_t>(L.total))
+        return ADSR_ERR_BAD_SHAPE;
+    if (reinterpret_cast<uintptr_t>(workspace) & 15) return ADSR_ERR_BAD_ALIGN;
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    char* ws = static_cast<char*>(workspace);
+    u64* hist = reinterpret_cast<u64*>(ws + L.digit_tot);
+    SelectState* st = reinterpret_cast<SelectState*>(ws + L.counters);
+    if (cudaMemsetAsync(hist, 0, kBins * sizeof(u64), s) != cudaSuccess || cudaMemsetAsync(st, 0, sizeof(SelectState), s) != cudaSuccess)
+        return ADSR_ERR_CUDA;
+    const int grid = stream_grid(L);
+    const bool vec = (reinterpret_cast<uintptr_t>(scores) & 15) == 0;
+    for (int shift = 24; shift >= 0; shift -= 8) {             // most significant digit first
+        if (vec)
+            select_hist_kernel<true><<<grid, kThreads, 0, s>>>(scores, n, shift, hist, st);
+        else
+            select_hist_kernel<false><<<grid, kThreads, 0, s>>>(scores, n, shift, hist, st);
+        select_pick_kernel<<<1, kThreads, 0, s>>>(shift, static_cast<u64>(k), hist, st, out);
+    }
+    return cudaGetLastError() == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
+}
+
+extern "C" int adsr_threshold_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes,
+                                      int n_regions, float threshold, void* workspace, int64_t workspace_bytes, double* out,
+                                      void* stream) {
+    using namespace adsr;
+    Layout L;
+    if (!make_layout(n, L) || n_regions < 0 || threshold != threshold) return ADSR_ERR_BAD_SHAPE;
+    if (scores == nullptr || regions == nullptr || (n_regions > 0 && region_sizes == nullptr) || workspace == nullptr ||
+        out == nullptr || workspace_bytes < static_cast<int64_t>(L.total))
+        return ADSR_ERR_BAD_SHAPE;
+    if (reinterpret_cast<uintptr_t>(workspace) & 15) return ADSR_ERR_BAD_ALIGN;
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    ThrCounts* part = reinterpret_cast<ThrCounts*>(static_cast<char*>(workspace) + L.hist);
+    static_assert(sizeof(ThrCounts) <= kBins * sizeof(long long), "one partial per sort tile fits the tile's histogram slice");
+    const int grid = stream_grid(L);
+    const bool vec = ((reinterpret_cast<uintptr_t>(scores) | reinterpret_cast<uintptr_t>(regions)) & 15) == 0;
+    if (vec)
+        threshold_kernel<true><<<grid, kThreads, 0, s>>>(scores, regions, region_sizes, n_regions, n, threshold, part);
+    else
+        threshold_kernel<false><<<grid, kThreads, 0, s>>>(scores, regions, region_sizes, n_regions, n, threshold, part);
+    threshold_finish_kernel<<<1, kThreads, 0, s>>>(part, grid, n, n_regions, out);
     return cudaGetLastError() == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
 }

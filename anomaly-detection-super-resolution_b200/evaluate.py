@@ -69,6 +69,17 @@ def parse_args(argv=None):
     p.add_argument('--save-segmentation', action='store_true', default=False,
                    help='write <output-dir>/segmentation/<split>/<stem>_{ssim,se}.png: each map thresholded at its F1-max threshold '
                         '(uint8 0 / 255); needs --mask-dir, implies --pr-metrics')
+    # thresholds calibrated on defect-free images: no test label is used to choose them
+    p.add_argument('--calibration-dir', type=str, default=None,
+                   help='defect-free images laid out like a test split (HR/ and an LR folder, e.g. <data-root>/<classe>/train/good): '
+                        'a pixel and an image threshold per map are calibrated on them and the test set is scored at them; implies '
+                        '--anomaly-maps')
+    p.add_argument('--calibration-quantile', type=float, default=0.999, metavar='Q',
+                   help='the thresholds are this quantile (in (0, 1]) of the calibration pixels and of the calibration images\' map maxima; '
+                        'a pixel / image is defective when its score is above it')
+    p.add_argument('--save-calibrated-masks', action='store_true', default=False,
+                   help='write <output-dir>/calibrated/<split>/<stem>_{ssim,se}.png: each map thresholded at its calibrated pixel '
+                        'threshold (uint8 0 / 255); needs --calibration-dir')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
 
@@ -83,6 +94,10 @@ def parse_args(argv=None):
             p.error(f'--au-pro: the false-positive-rate limit must be in (0, 1], got {args.au_pro}')
     if (args.pr_metrics or args.save_segmentation) and args.mask_dir is None:
         p.error('--pr-metrics and --save-segmentation need --mask-dir (the ground-truth masks label the defect pixels)')
+    if not 0.0 < args.calibration_quantile <= 1.0:
+        p.error(f'--calibration-quantile must be in (0, 1], got {args.calibration_quantile}')
+    if args.save_calibrated_masks and args.calibration_dir is None:
+        p.error('--save-calibrated-masks needs --calibration-dir (the defect-free images the threshold is calibrated on)')
     return args
 
 
@@ -427,6 +442,19 @@ def load_mask(path: Optional[str], hr_shape: Tuple[int, int], crop: Tuple[int, i
     return m
 
 
+def hr_size(f_hr: str, f_lr: str, scale: int) -> Tuple[int, int]:
+    """(H, W) of an HR image as load_pair crops it to its LR image, from the PNG headers."""
+    from PIL import Image
+
+    with Image.open(f_hr) as im_hr, Image.open(f_lr) as im_lr:
+        return min(im_hr.size[1], im_lr.size[1] * scale), min(im_hr.size[0], im_lr.size[0] * scale)
+
+
+def above(t: float) -> float:
+    """The fp32 threshold of a strict decision: for every fp32 score x, x >= above(t) <=> x > t (t an fp32 value)."""
+    return float(np.nextafter(np.float32(t), np.float32(np.inf)))
+
+
 def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str, scale_value: int) -> None:
     from PIL import Image
 
@@ -439,7 +467,8 @@ def save_sr_image(sr_u8_hwc: np.ndarray, output_dir: str, name: str, split: str,
 def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: bool, batch_size: Optional[int] = None,
                      anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
                      save_maps: bool = False, au_pro: Optional[float] = None, pr_metrics: bool = False,
-                     save_segmentation: bool = False):
+                     save_segmentation: bool = False, calibration_dir: Optional[str] = None, calibration_quantile: float = 0.999,
+                     save_calibrated_masks: bool = False):
     """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
 
     anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
@@ -451,7 +480,16 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     attains it (pixel_ap_{ssim,se}, f1_max_{ssim,se}, f1_threshold_{ssim,se}), printed on a `Map PR - ...` line before the `Map PRO`
     line, or before the `Map AUCs` line without one.  The F1 threshold is an oracle threshold: picked with the ground truth it is scored
     on.  save_segmentation (needs mask_dir, implies pr_metrics) writes each map thresholded at its F1 threshold as a uint8 0 / 255 mask
-    to <output_dir>/segmentation/<split>/<stem>_{ssim,se}.png.  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy."""
+    to <output_dir>/segmentation/<split>/<stem>_{ssim,se}.png.  save_maps writes <output_dir>/maps/<split>/<stem>_{ssim,se}.npy.
+
+    calibration_dir (implies anomaly_maps; single process only): defect-free images in the layout of a test split, every one of a test
+    image's HR size.  They run first; for each map the pixel threshold t_px is the calibration_quantile (in (0, 1], inverted_cdf: an
+    actual score) of all their pixels and the image threshold t_img the same quantile of their map maxima.  Decisions are strict: a
+    pixel is defective when map > t_px, an image when its map max > t_img, so at most a fraction 1 - q of the calibration pixels and
+    images is flagged.  Adds calib_{pixel,image}_threshold_{ssim,se} and the test set's calib_image_{tpr,fpr}_{ssim,se}, with mask_dir
+    also calib_pixel_{precision,recall,fpr,f1,iou,pro}_{ssim,se} at t_px, printed on a `Map CAL - ...` line before the other `Map`
+    lines.  No test label is used to choose the thresholds.  save_calibrated_masks (needs calibration_dir) writes the `map > t_px` masks
+    as uint8 0 / 255 to <output_dir>/calibrated/<split>/<stem>_{ssim,se}.png."""
     from .model import Model
 
     if au_pro is not None:
@@ -461,12 +499,19 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
             raise ValueError(f"au_pro: the false-positive-rate limit must be in (0, 1], got {au_pro}")
     if (pr_metrics or save_segmentation) and mask_dir is None:
         raise ValueError("pr_metrics and save_segmentation need mask_dir: the ground-truth masks label the defect pixels")
+    if not 0.0 < float(calibration_quantile) <= 1.0:
+        raise ValueError(f"calibration_quantile must be in (0, 1], got {calibration_quantile}")
+    if save_calibrated_masks and calibration_dir is None:
+        raise ValueError("save_calibrated_masks needs calibration_dir: the defect-free images the threshold is calibrated on")
     pr_metrics = pr_metrics or save_segmentation
-    anomaly_maps = anomaly_maps or mask_dir is not None or save_maps
+    anomaly_maps = anomaly_maps or mask_dir is not None or save_maps or calibration_dir is not None
     scale = opt.scale[-1] if isinstance(opt.scale, list) else int(opt.scale)
     rank, world = _dist_info()
     if mask_dir is not None and world > 1:
         raise RuntimeError("--mask-dir needs the whole maps of every image in one process: run it without sharding (world size 1)")
+    if calibration_dir is not None and world > 1:
+        raise RuntimeError("--calibration-dir needs the whole maps of every calibration image in one process: run it without sharding "
+                           "(world size 1)")
     entries = []                                             # (label, split, hr path, lr path): good first, then bad
     for label, split in ((0, 'good'), (1, 'bad')):
         d = f'{opt.data_root}/{opt.classe}/test/{split}'
@@ -482,11 +527,21 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     # PNG headers before the images are sharded: every rank sweeps the same sizes, also one that holds no image at all
     from PIL import Image
 
-    min_dim = None
+    min_dim, test_sizes = None, set()
     for _, _, f_hr, f_lr in entries:
-        with Image.open(f_hr) as im_hr, Image.open(f_lr) as im_lr:
-            dims = (min(im_hr.size[1], im_lr.size[1] * scale), min(im_hr.size[0], im_lr.size[0] * scale))
+        dims = hr_size(f_hr, f_lr, scale)
+        test_sizes.add(dims)
         min_dim = min(dims) if min_dim is None else min(min_dim, *dims)
+    cal_files = []
+    if calibration_dir is not None:                          # checked before the model runs
+        cal_files = list(zip(*scan_split(calibration_dir, scale)))
+        if not cal_files:
+            raise ValueError(f"no calibration images in {calibration_dir}/HR")
+        for f_hr, f_lr in cal_files:
+            dims = hr_size(f_hr, f_lr, scale)
+            if dims not in test_sizes:
+                raise ValueError(f"calibration image {f_hr} is {dims[0]}x{dims[1]}, the test images are "
+                                 f"{', '.join(f'{h}x{w}' for h, w in sorted(test_sizes))}")
 
     opt.pre_train = checkpoint_model_path
     model = Model(opt, None)
@@ -496,23 +551,39 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     mine = list(range(rank, len(entries), world))            # image index i -> rank i mod R
     rows, ids = [], []
 
-    def host_batches():
-        """(lr, hr) pinned host batches in evaluation order; `order` records the image ids of each batch."""
-        for s in range(0, len(mine), bs):
-            idx = mine[s:s + bs]
-            pairs = [load_pair(entries[i][2], entries[i][3], scale, opt.n_colors, opt.rgb_range, raw_u8=True) for i in idx]
+    def host_batches(files, ids_, order):
+        """(lr, hr) pinned host batches of the (hr path, lr path) files[i] for i in ids_; `order` records the ids of each batch."""
+        for s in range(0, len(ids_), bs):
+            idx = ids_[s:s + bs]
+            pairs = [load_pair(files[i][0], files[i][1], scale, opt.n_colors, opt.rgb_range, raw_u8=True) for i in idx]
             if len({p[0].dtype for p in pairs}) > 1:           # mixed decodes (should not happen within a dataset): all float
-                pairs = [load_pair(entries[i][2], entries[i][3], scale, opt.n_colors, opt.rgb_range) for i in idx]
+                pairs = [load_pair(files[i][0], files[i][1], scale, opt.n_colors, opt.rgb_range) for i in idx]
             shapes = {(tuple(p[0].shape), tuple(p[1].shape)) for p in pairs}
             groups = [list(range(len(idx)))] if len(shapes) == 1 else [[j] for j in range(len(idx))]
             for g in groups:                                  # mixed sizes fall back to one image per launch
                 order.append([idx[j] for j in g])
                 yield (torch.stack([pairs[j][0] for j in g]).pin_memory(), torch.stack([pairs[j][1] for j in g]).pin_memory())
 
+    t_px = t_img = px_above = None
+    if cal_files:                                            # calibration pass: maps of the defect-free images, no labels
+        cal = metrics.LocalisationAccumulator(2)
+        cal_max = []
+        with torch.no_grad():
+            for _ in ev.run_pipelined(host_batches(cal_files, list(range(len(cal_files))), [])):
+                cal.append(ev.last_maps[:2])                   # device copies, ordered before the next replay overwrites the maps
+                cal_max.append(ev.last_maps[2].clone())
+        q = float(calibration_quantile)
+        cal_max = torch.cat(cal_max).cpu().numpy()
+        t_px = [cal.quantile(j, q) for j in range(2)]
+        t_img = [float(np.quantile(cal_max[:, j], q, method='inverted_cdf')) for j in range(2)]
+        px_above = [above(t) for t in t_px]
+        del cal                                              # the calibration maps are freed before the test pass
+
     order: List[List[int]] = []
     loc = metrics.LocalisationAccumulator(2) if mask_dir is not None else None   # both maps of every image, kept on the device
+    test_files = [(e[2], e[3]) for e in entries]
     with torch.no_grad():
-        for k, scores in enumerate(ev.run_pipelined(host_batches())):   # PNG decode + H2D of batch k + 1 overlap batch k
+        for k, scores in enumerate(ev.run_pipelined(host_batches(test_files, mine, order))):   # PNG decode + H2D of batch k + 1 overlap batch k
             if ev.last_maps is not None:                      # the two map maxima ride along in the gathered score table
                 scores = torch.cat([scores, ev.last_maps[2]], 1)
             rows.append(scores)
@@ -530,6 +601,14 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                     d.mkdir(parents=True, exist_ok=True)
                     np.save(d / f'{name}_ssim.npy', m_ssim[j])
                     np.save(d / f'{name}_se.npy', m_se[j])
+            if save_calibrated_masks:
+                for j, kind in enumerate(('ssim', 'se')):
+                    pred = (ev.last_maps[j] >= px_above[j]).cpu().numpy()
+                    for b, i in enumerate(order[k]):
+                        name = os.path.splitext(os.path.basename(entries[i][2]))[0]
+                        d = Path(output_dir) / 'calibrated' / entries[i][1]
+                        d.mkdir(parents=True, exist_ok=True)
+                        Image.fromarray(pred[b].astype(np.uint8) * 255).save(str(d / f'{name}_{kind}.png'))
             if loc is not None:
                 batch_masks = []
                 for i in order[k]:
@@ -549,6 +628,22 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
         res.update(map_max=map_max, auc_map_ssim=metrics.roc_auc(y_true, map_max[:, 0]), auc_map_se=metrics.roc_auc(y_true, map_max[:, 1]))
         line = (f"Map AUCs - max 1-SSIM(ws={map_window_size}, sigma={float(map_sigma)}): {res['auc_map_ssim']:.4f}, "
                 f"max SE: {res['auc_map_se']:.4f}")
+        if t_px is not None:
+            y = np.asarray(y_true)
+            parts = []
+            for j, kind, label in ((0, 'ssim', '1-SSIM'), (1, 'se', 'SE')):
+                flagged = map_max[:, j] >= above(t_img[j])
+                tpr, fpr = float(flagged[y == 1].mean()), float(flagged[y == 0].mean())
+                res.update({f'calib_pixel_threshold_{kind}': t_px[j], f'calib_image_threshold_{kind}': t_img[j],
+                            f'calib_image_tpr_{kind}': tpr, f'calib_image_fpr_{kind}': fpr})
+                part = f"{label} t_px {t_px[j]:g}, t_img {t_img[j]:g}, image TPR {tpr:.4f}, FPR {fpr:.4f}"
+                if mask_dir is not None:
+                    m = loc.at_threshold(j, px_above[j])
+                    res.update({f'calib_pixel_{f}_{kind}': getattr(m, f) for f in ('precision', 'recall', 'fpr', 'f1', 'iou', 'pro')})
+                    part += (f", pixel precision {m.precision:.4f}, recall {m.recall:.4f}, FPR {m.fpr:.4f}, F1 {m.f1:.4f}, "
+                             f"IoU {m.iou:.4f}, PRO {m.pro:.4f}")
+                parts.append(part)
+            print(f"Map CAL - q={float(calibration_quantile):g} on {len(cal_files)} defect-free images: " + "; ".join(parts))
         if mask_dir is not None:
             limit = 0.3 if au_pro is None else float(au_pro)
             m_ssim, m_se = loc.results(limit)
@@ -613,7 +708,8 @@ def main(argv=None):
     return evaluate_on_test(opt, ckpt_path, out_dir, args.save_images, batch_size=args.batch_size, anomaly_maps=args.anomaly_maps,
                             map_window_size=args.map_window_size, map_sigma=args.map_sigma, mask_dir=args.mask_dir,
                             save_maps=args.save_maps, au_pro=args.au_pro, pr_metrics=args.pr_metrics,
-                            save_segmentation=args.save_segmentation)
+                            save_segmentation=args.save_segmentation, calibration_dir=args.calibration_dir,
+                            calibration_quantile=args.calibration_quantile, save_calibrated_masks=args.save_calibrated_masks)
 
 
 if __name__ == "__main__":

@@ -126,15 +126,50 @@ class LocalisationMetrics(NamedTuple):
     f1_threshold: float     # the fp32 score that attains it: `map >= f1_threshold` is the F1-max defect mask
 
 
+class ThresholdMetrics(NamedTuple):
+    """The pixel metrics of the prediction `map >= threshold` over a whole test set (LocalisationAccumulator.at_threshold).  Precision
+    is 0 when nothing is predicted; recall, fpr, f1 and iou are NaN when their denominator is 0, pro when there is no defect region."""
+    threshold: float
+    tp: int                 # predicted defect pixels that are defects
+    fp: int                 # predicted defect pixels that are defect-free
+    fn: int                 # defect pixels not predicted
+    tn: int                 # defect-free pixels not predicted
+    precision: float        # tp / (tp + fp)
+    recall: float           # tp / (tp + fn)
+    fpr: float              # fp / (fp + tn)
+    f1: float               # 2 tp / (2 tp + fp + fn)
+    iou: float              # tp / (tp + fp + fn)
+    pro: float              # mean over the defect regions of the share of the region's pixels predicted
+
+
+def inverted_cdf_rank(n: int, q: float) -> int:
+    """The 1-based rank k of np.quantile(x, q, method="inverted_cdf") among n sorted float64 values: max(1, ceil(q n)), with q n
+    formed in float64 exactly as numpy forms it (so q = 0.28, n = 25 gives k = 8: 0.28 * 25 rounds to 7.000000000000001).  (Given an
+    fp32 array numpy forms q n in fp32 instead, which misranks and fails beyond 2^24 values; the scores convert to float64 exactly.)"""
+    index = np.float64(n) * np.float64(q) - 1.0
+    prev = np.floor(index)
+    k0 = int(prev) if index == prev else int(prev) + 1
+    return max(k0, 0) + 1
+
+
+def fp32_at_least(threshold: float) -> np.float32:
+    """The smallest fp32 >= threshold: for every fp32 x, x >= result <=> x >= threshold (the exact double)."""
+    t = np.float32(threshold)
+    if float(t) < threshold:                          # a Python float against np.float32 would be compared in fp32
+        t = np.nextafter(t, np.float32(np.inf))
+    return t
+
+
 class LocalisationAccumulator:
     """Pixel AUROC, AU-PRO, pixel AP and F1-max of `n_maps` anomaly maps over a whole test set, fed one batch at a time.
 
-    append(maps, masks): maps = one entry per map, each a CUDA fp32 [B, H, W] tensor or a sequence of [H, W] tensors (any sizes);
-    masks = the host masks of the same B images (non-zero = defect).  The maps are copied on the device into one growing buffer per map
+    append(maps, masks=None): maps = one entry per map, each a CUDA fp32 [B, H, W] tensor or a sequence of [H, W] tensors (any sizes);
+    masks = the host masks of the same B images (non-zero = defect), or None: every pixel is defect-free (calibration images).  The maps are copied on the device into one growing buffer per map
     (no device -> host copy); each mask is labelled once on the host (scipy.ndimage.label, 8-connectivity) and its per-pixel region
     indices are shared by all maps.  results(fpr_limit) runs adsr_localisation_metrics once per map and returns one LocalisationMetrics
     per map, finish(fpr_limit) the [(pixel_auroc, au_pro), ...] part of it: the same numbers for the same image sequence however it was
-    split into batches.  segmentation(map_index, threshold) thresholds the accumulated maps into per-image defect masks."""
+    split into batches.  segmentation(map_index, threshold) thresholds the accumulated maps into per-image defect masks,
+    at_threshold(map_index, threshold) scores that prediction against the masks, quantile(map_index, q) is an exact score quantile."""
 
     def __init__(self, n_maps: int = 1):
         self.n_maps = int(n_maps)
@@ -160,13 +195,24 @@ class LocalisationAccumulator:
         self._maps = [grow(m, torch.float32) for m in self._maps]
         self._regions = grow(self._regions, torch.int32)
 
-    def append(self, maps, masks) -> None:
+    def append(self, maps, masks=None) -> None:
         from scipy.ndimage import label
 
         if len(maps) != self.n_maps:
             raise ValueError(f"append: {len(maps)} maps given, the accumulator holds {self.n_maps}")
         parts = [_map_pieces(m) for m in maps]
         shapes = parts[0][1]
+        if masks is None:                             # defect-free images: no labelling, every region index is -1
+            if any(p[1] != shapes for p in parts):
+                raise ValueError("append: all maps must hold the same images")
+            n_new = sum(h * w for h, w in shapes)
+            self._reserve(n_new, parts[0][0][0].device)
+            self._copy_maps(parts)
+            self._regions[self.n:self.n + n_new].fill_(-1)
+            self._shapes += shapes
+            self.n += n_new
+            self.n_ok += n_new
+            return
         masks = [np.asarray(k) for k in masks]
         if any(p[1] != shapes for p in parts) or len(masks) != len(shapes) or any(k.shape != s for k, s in zip(masks, shapes)):
             raise ValueError("append: every map needs a mask of its own shape, and all maps the same images")
@@ -184,17 +230,20 @@ class LocalisationAccumulator:
         n_new = sum(k.size for k in masks)
         device = parts[0][0][0].device
         self._reserve(n_new, device)
-        for buf, (pieces, _) in zip(self._maps, parts):
-            off = self.n
-            for m in pieces:
-                buf[off:off + m.numel()].copy_(m.reshape(-1))
-                off += m.numel()
+        self._copy_maps(parts)
         if n_new:
             self._regions[self.n:self.n + n_new].copy_(torch.from_numpy(np.concatenate(regions)))
         self._sizes += sizes
         self._shapes += shapes
         self.n += n_new
         self.n_ok += n_ok
+
+    def _copy_maps(self, parts) -> None:
+        for buf, (pieces, _) in zip(self._maps, parts):
+            off = self.n
+            for m in pieces:
+                buf[off:off + m.numel()].copy_(m.reshape(-1))
+                off += m.numel()
 
     def results(self, fpr_limit: float = 0.3) -> list[LocalisationMetrics]:
         """One LocalisationMetrics per map (AU-PRO up to FPR = fpr_limit).  ValueError: fpr_limit outside (0, 1], no defect region
@@ -228,12 +277,8 @@ class LocalisationAccumulator:
         """Predicted defect masks: bool [H, W] host arrays `map >= threshold` of map `map_index`, one per appended image in append order
         (one comparison on the device over the accumulated map, one device -> host copy).  With the f1_threshold of results() they are
         the masks that attain F1-max.  The comparison is that of the fp32 map with the exact double `threshold`."""
-        j = int(map_index)
-        if not 0 <= j < self.n_maps:
-            raise IndexError(f"segmentation: map {map_index} of {self.n_maps}")
-        t = np.float32(threshold)
-        if t < threshold:                             # the smallest fp32 >= threshold: x >= t32 <=> x >= threshold for every fp32 x
-            t = np.nextafter(t, np.float32(np.inf))
+        j = self._map_index(map_index, "segmentation")
+        t = fp32_at_least(threshold)
         if self.n == 0:
             return []
         flat = (self._maps[j][:self.n] >= float(t)).cpu().numpy()
@@ -242,6 +287,56 @@ class LocalisationAccumulator:
             out.append(flat[off:off + h * w].reshape(h, w))
             off += h * w
         return out
+
+    def _map_index(self, map_index: int, what: str) -> int:
+        j = int(map_index)
+        if not 0 <= j < self.n_maps:
+            raise IndexError(f"{what}: map {map_index} of {self.n_maps}")
+        return j
+
+    def quantile(self, map_index: int, q: float) -> float:
+        """The exact q-quantile of all accumulated scores of map `map_index`: np.quantile(scores.astype(float64), q,
+        method="inverted_cdf"), the fp32 score of rank k = inverted_cdf_rank(n, q) (no interpolation; -0.0 reported as +0.0), found on the device by a radix select.
+        ValueError: q outside [0, 1], nothing appended, or a NaN in the map."""
+        j = self._map_index(map_index, "quantile")
+        q = float(q)
+        if not 0.0 <= q <= 1.0:
+            raise ValueError(f"quantile: q must be in [0, 1], got {q}")
+        if self.n == 0:
+            raise ValueError("quantile: no scores appended")
+        device = self._regions.device
+        ws = torch.empty(ops.localisation_workspace_bytes(self.n), dtype=torch.uint8, device=device)
+        out = torch.empty(2, dtype=torch.float64, device=device)
+        ops.score_quantile(self._maps[j][:self.n], inverted_cdf_rank(self.n, q), ws, out)
+        score, nan = out.tolist()
+        if nan:
+            raise ValueError(f"map {j} holds {int(nan)} NaN scores")
+        return score
+
+    def at_threshold(self, map_index: int, threshold: float) -> ThresholdMetrics:
+        """The pixel metrics of the prediction `map >= threshold` of map `map_index` against the appended masks: the comparison of
+        segmentation() (the fp32 map against the exact double threshold), counted on the device in one pass.  ValueError: a NaN
+        threshold, nothing appended, or a NaN in the map."""
+        j = self._map_index(map_index, "at_threshold")
+        threshold = float(threshold)
+        if threshold != threshold:
+            raise ValueError("at_threshold: the threshold is NaN")
+        if self.n == 0:
+            raise ValueError("at_threshold: no scores appended")
+        device = self._regions.device
+        sizes = torch.from_numpy(np.concatenate(self._sizes)).to(device) if self._sizes else None
+        ws = torch.empty(ops.localisation_workspace_bytes(self.n), dtype=torch.uint8, device=device)
+        out = torch.empty(7, dtype=torch.float64, device=device)
+        ops.threshold_metrics(self._maps[j][:self.n], self._regions[:self.n], sizes, float(fp32_at_least(threshold)), ws, out)
+        r = out.tolist()
+        if r[5]:
+            raise ValueError(f"map {j} holds {int(r[5])} NaN scores")
+        tp, fp, fn, tn = (int(v) for v in r[:4])
+        if r[6] or fp + tn != self.n_ok:
+            raise RuntimeError(f"threshold metrics: inconsistent region indices on the device (map {j}: {r})")
+        ratio = lambda a, b: a / b if b else float("nan")
+        return ThresholdMetrics(threshold, tp, fp, fn, tn, tp / (tp + fp) if tp + fp else 0.0, ratio(tp, tp + fn), ratio(fp, fp + tn),
+                                ratio(2 * tp, 2 * tp + fp + fn), ratio(tp, tp + fp + fn), r[4])
 
 
 def _on_device(maps) -> bool:
@@ -276,6 +371,14 @@ def f1_max(maps, masks) -> tuple[float, float]:
     acc.append([maps], masks)
     r = acc.results()[0]
     return r.f1_max, r.f1_threshold
+
+
+def score_quantile(maps, q: float) -> float:
+    """np.quantile(scores.astype(float64), q, method="inverted_cdf") of every pixel of CUDA fp32 maps (an [N, H, W] tensor or a sequence of [H, W]
+    tensors): an actual score, exact, found on the device (adsr_score_quantile); also beyond the 2^24 elements torch.quantile takes."""
+    acc = LocalisationAccumulator(1)
+    acc.append([maps])
+    return acc.quantile(0, q)
 
 
 def pixel_auroc(maps, masks) -> float:

@@ -371,6 +371,54 @@ def localisation_metrics(scores: torch.Tensor, regions: torch.Tensor, region_siz
     return out
 
 
+def _check_tensors(what: str, *specs) -> None:
+    for t, name, dt in specs:
+        _cuda(t, name)
+        if t.dtype != dt or not t.is_contiguous():
+            raise ValueError(f"{what}: {name} must be a contiguous {dt} tensor")
+
+
+def score_quantile(scores: torch.Tensor, k: int, workspace: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """The exact k-th smallest of the fp32 scores [n], 1 <= k <= n (-0.0 reported as +0.0) -> out fp64 [2] = (score, NaN scores; the
+    score is NaN when fewer than k scores are not NaN).  workspace: uint8 [>= localisation_workspace_bytes(n)].  A radix select: eight
+    kernels, no synchronisation."""
+    _check_tensors("score_quantile", (scores, "scores", torch.float32), (workspace, "workspace", torch.uint8),
+                   (out, "out", torch.float64))
+    n = scores.numel()
+    if not 1 <= int(k) <= n or out.numel() < 2:
+        raise ValueError(f"score_quantile: rank {k} of {n} scores, out of {out.numel()} values")
+    _t = _begin()
+    check(lib().adsr_score_quantile(ptr(scores), n, int(k), ptr(workspace), workspace.numel(), ptr(out), stream_ptr()),
+          "adsr_score_quantile")
+    global LAUNCHES
+    LAUNCHES += 7                                      # 4 passes x (histogram + pick); _count adds the last
+    _count("score_quantile", 0.0, _t)
+    return out
+
+
+def threshold_metrics(scores: torch.Tensor, regions: torch.Tensor, region_sizes: Optional[torch.Tensor], threshold: float,
+                      workspace: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """Pixel counts of the prediction `scores >= threshold` (an fp32 value, not NaN) against the regions of localisation_metrics:
+    out fp64 [7] = (TP, FP, FN, TN, PRO@threshold (NaN without regions), NaN scores, out-of-range region indices).  region_sizes may be
+    None when no pixel belongs to a region.  Two kernels, no synchronisation."""
+    specs = [(scores, "scores", torch.float32), (regions, "regions", torch.int32), (workspace, "workspace", torch.uint8),
+             (out, "out", torch.float64)]
+    if region_sizes is not None:
+        specs.append((region_sizes, "region_sizes", torch.int64))
+    _check_tensors("threshold_metrics", *specs)
+    n = scores.numel()
+    if regions.numel() != n or out.numel() < 7:
+        raise ValueError(f"threshold_metrics: {n} scores, {regions.numel()} region indices, out of {out.numel()} values")
+    _t = _begin()
+    check(lib().adsr_threshold_metrics(ptr(scores), ptr(regions), n, ptr(region_sizes),
+                                       0 if region_sizes is None else region_sizes.numel(), float(threshold), ptr(workspace),
+                                       workspace.numel(), ptr(out), stream_ptr()), "adsr_threshold_metrics")
+    global LAUNCHES
+    LAUNCHES += 1                                      # counting pass; _count adds the reduction
+    _count("threshold_metrics", 0.0, _t)
+    return out
+
+
 def score_images_strided(sr: torch.Tensor, hr: torch.Tensor, layout: str, window_sizes: Sequence[int], *, div: float = 1.0,
                          clamp01: bool = False, zero_pad: bool = False, c1: float = 1e-4, c2: float = 9e-4,
                          psnr_peak: float = 1.0) -> torch.Tensor:

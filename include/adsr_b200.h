@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 17
+#define ADSR_ABI_VERSION 18
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -289,6 +289,23 @@ int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B,
 int64_t adsr_localisation_workspace_bytes(int64_t n);
 int adsr_localisation_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes, int n_regions,
                               int64_t n_ok, double fpr_limit, void* workspace, int64_t workspace_bytes, double* out, void* stream);
+
+/* Thresholds calibrated on defect-free images, and the metrics of one fixed threshold; both read the scores without sorting them,
+ * take the same workspace as adsr_localisation_metrics (adsr_localisation_workspace_bytes(n) bytes, 16-byte aligned), are integer-exact
+ * and deterministic, and do not synchronise with the host.
+ * adsr_score_quantile: the exact k-th smallest of the n fp32 scores, 1 <= k <= n (np.quantile(scores.astype(float64), q,
+ *   method="inverted_cdf") for k = max(1, ceil(q n))): an MSD radix select over the order-preserving 32-bit keys, 4 passes of 8 bits, ~16 B read per pixel.
+ *   -0.0 ranks as +0.0 and is reported as +0.0; NaN scores are counted, not ranked.
+ *   out: fp64 [2] = {score, NaN scores} (score = NaN when fewer than k scores are not NaN).
+ * adsr_threshold_metrics: one pass over the pixels with the rule `score >= threshold` (threshold not NaN); regions / region_sizes /
+ *   n_regions as in adsr_localisation_metrics, except that n_regions may be 0 (region_sizes may then be NULL).
+ *   out: fp64 [7] = {TP, FP, FN, TN, PRO@threshold, NaN scores, region indices out of range}: counts of predicted / actual defect
+ *   pixels (a NaN score is never predicted); PRO@threshold = mean over the regions of the share of the region's pixels predicted,
+ *   from the fixed-point weights the AU-PRO curve sums (NaN when n_regions == 0).  The last two are checks for the caller.
+ * ADSR_ERR_BAD_SHAPE: n < 1, k outside [1, n], n_regions < 0, a NaN threshold, a NULL pointer or a short workspace. */
+int adsr_score_quantile(const float* scores, int64_t n, int64_t k, void* workspace, int64_t workspace_bytes, double* out, void* stream);
+int adsr_threshold_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes, int n_regions,
+                           float threshold, void* workspace, int64_t workspace_bytes, double* out, void* stream);
 
 /* Validation metrics of the reference's training loop, `Trainer.test` (src/trainer.py:242-304), for a batch of fp32 image
  * pairs: the SR value is first quantised with ROUNDING (`quantize`, src/trainer.py:45-47: round(clamp(x * 255 / rgb_range, 0,

@@ -7,7 +7,11 @@ pairs per pixel are far above the 126 MB of L2.  --host also times the host path
 metrics.pixel_auroc on host arrays, the oracle's AU-PRO, sklearn's average_precision_score, the oracle's F1-max) and reports the
 agreement.  One JSON line, with the card and its power limit.
 
-    python tools/localisation_bench.py [--images 1024] [--side 256] [--reps 20] [--host]
+It also times, on the same map, the two passes that need no sort: the exact score quantile (adsr_score_quantile, a radix select
+reading ~16 B per pixel) at --quantile, and the pixel counts + PRO at that score (adsr_threshold_metrics, one pass over the 8 B of
+score and region index per pixel).  --host adds np.quantile(method="inverted_cdf") and the oracle's counts, and their agreement.
+
+    python tools/localisation_bench.py [--images 1024] [--side 256] [--reps 20] [--quantile 0.999] [--host]
 """
 from __future__ import annotations
 
@@ -69,6 +73,7 @@ def main(argv=None):
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--fpr-limit", type=float, default=0.3)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--quantile", type=float, default=0.999, help="q of the timed quantile; its score is the timed threshold")
     ap.add_argument("--host", action="store_true", help="also time the host path on the same inputs and report the agreement")
     a = ap.parse_args(argv)
     if not torch.cuda.is_available():
@@ -107,13 +112,37 @@ def main(argv=None):
         e1.synchronize()
         times.append(e0.elapsed_time(e1))
     again = out.cpu().numpy()
+
+    def timed(fn):                                          # median device ms of fn over the repetitions, after the warm-ups
+        for _ in range(a.warmup):
+            fn()
+        ts = []
+        for _ in range(a.reps):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            e1.synchronize()
+            ts.append(e0.elapsed_time(e1))
+        return statistics.median(ts)
+
+    k = metrics.inverted_cdf_rank(n, a.quantile)
+    q_out, t_out = torch.empty(2, dtype=torch.float64, device="cuda"), torch.empty(7, dtype=torch.float64, device="cuda")
+    q_ms = timed(lambda: ops.score_quantile(buf[:n], k, ws, q_out))
+    t_q = float(q_out[0])
+    thr_ms = timed(lambda: ops.threshold_metrics(buf[:n], regions, sizes, t_q, ws, t_out))
+    th = acc.at_threshold(0, t_q)
     name, power = card()
     res = dict(tool="localisation_bench", gpu=name, power_limit_w=power, images=a.images, side=a.side, pixels_per_map=n,
                regions=acc.n_regions, fpr_limit=a.fpr_limit, reps=a.reps, device_ms_per_map_median=statistics.median(times),
                device_ms_per_map_min=min(times), device_ms_per_map_max=max(times), pixel_auroc=auroc, au_pro=aupro,
                pixel_ap=r.pixel_ap, f1_max=r.f1_max, f1_threshold=r.f1_threshold,
                repeat_bitwise_equal=bool(tuple(float(again[k]) for k in (0, 1, 5, 6, 7)) == tuple(r)),
-               bytes_per_pixel_floor=80, floor_ms_at_7_7_tbps=n * 80 / 7.7e12 * 1e3)
+               bytes_per_pixel_floor=80, floor_ms_at_7_7_tbps=n * 80 / 7.7e12 * 1e3,
+               quantile=a.quantile, quantile_score=t_q, quantile_device_ms_median=q_ms, quantile_floor_ms_at_7_7_tbps=n * 16 / 7.7e12 * 1e3,
+               quantile_equals_accumulator=t_q == acc.quantile(0, a.quantile),
+               threshold_device_ms_median=thr_ms, threshold_floor_ms_at_7_7_tbps=n * 8 / 7.7e12 * 1e3,
+               threshold_counts=[th.tp, th.fp, th.fn, th.tn], threshold_pro=th.pro)
     if a.host:
         from oracle import localisation_oracle as L
         from oracle import pr_oracle as P
@@ -136,6 +165,17 @@ def main(argv=None):
         res["abs_diff_pixel_ap"] = abs(h_ap - r.pixel_ap)
         res["abs_diff_f1_max"] = abs(h_f1 - r.f1_max)
         res["f1_threshold_equal"] = h_thr == r.f1_threshold
+        from oracle import threshold_oracle as T
+
+        t0 = time.perf_counter()
+        h_q = T.quantile(list(h_maps), a.quantile)
+        res["host_quantile_numpy_s"] = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        h_counts = T.counts(list(h_maps), list(masks), t_q)
+        res["host_threshold_oracle_s"] = time.perf_counter() - t0
+        res["quantile_equal"] = h_q == t_q
+        res["threshold_counts_equal"] = list(h_counts[:4]) == [th.tp, th.fp, th.fn, th.tn]
+        res["abs_diff_threshold_pro"] = abs(h_counts[4] - th.pro)
     print(json.dumps(res))
 
 
