@@ -13,7 +13,7 @@ from ctypes import c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_void_
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # ADSR_LIB: developer override for A/B timing of two builds in one session (tools/build_variant.sh); never a fallback
 LIB_PATH = os.environ.get("ADSR_LIB") or os.path.join(_HERE, "libadsr_b200.so")
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 ACT_NONE, ACT_LRELU, ACT_GELU, ACT_RELU = 0, 1, 2, 3
 OUT_ROWS, OUT_PIXEL_SHUFFLE2 = 0, 1
@@ -63,6 +63,8 @@ _SIGNATURES = {
                                   c_void_p]),
     "adsr_anomaly_maps": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
                                   c_void_p, c_void_p]),
+    "adsr_gms_workspace_bytes": (c_int64, [c_int, c_int, c_int]),
+    "adsr_gms_map": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
     "adsr_localisation_workspace_bytes": (c_int64, [c_int64]),
     "adsr_localisation_metrics": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int, c_int64, c_double, c_void_p, c_int64, c_void_p,
                                           c_void_p]),

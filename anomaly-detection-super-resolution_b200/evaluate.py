@@ -57,17 +57,21 @@ def parse_args(argv=None):
                    help='also compute per-pixel 1-SSIM and squared-error maps and report the AUCs of their per-image max')
     p.add_argument('--map-window-size', type=int, default=11, help='SSIM window size of the 1-SSIM map (odd)')
     p.add_argument('--map-sigma', type=float, default=4.0, help='Gaussian smoothing of both maps (scipy gaussian_filter sigma; 0 = off)')
+    p.add_argument('--gms-map', action='store_true', default=False,
+                   help='also compute the multi-scale gradient-magnitude-similarity (MSGMS) map, smoothed with --map-sigma, and report '
+                        'every map metric for it too; implies --anomaly-maps')
     p.add_argument('--mask-dir', type=str, default=None,
                    help='ground-truth masks <mask-dir>/<stem>.png or <stem>_mask.png (non-zero = defect): adds pixel AUROC; '
                         'implies --anomaly-maps')
     p.add_argument('--save-maps', action='store_true', default=False,
-                   help='write <output-dir>/maps/<split>/<stem>_ssim.npy and <stem>_se.npy (float32 HxW); implies --anomaly-maps')
+                   help='write <output-dir>/maps/<split>/<stem>_ssim.npy and <stem>_se.npy (float32 HxW; also <stem>_gms.npy with '
+                        '--gms-map); implies --anomaly-maps')
     p.add_argument('--au-pro', type=float, nargs='?', const=0.3, default=None, metavar='FPR_LIMIT',
                    help='also report the AU-PRO of both maps up to this false-positive rate (bare flag: 0.3); needs --mask-dir')
     p.add_argument('--pr-metrics', action='store_true', default=False,
                    help='also report the pixel AP and the F1-max of both maps with the threshold that attains it; needs --mask-dir')
     p.add_argument('--save-segmentation', action='store_true', default=False,
-                   help='write <output-dir>/segmentation/<split>/<stem>_{ssim,se}.png: each map thresholded at its F1-max threshold '
+                   help='write <output-dir>/segmentation/<split>/<stem>_{ssim,se[,gms]}.png: each map thresholded at its F1-max threshold '
                         '(uint8 0 / 255); needs --mask-dir, implies --pr-metrics')
     # thresholds calibrated on defect-free images: no test label is used to choose them
     p.add_argument('--calibration-dir', type=str, default=None,
@@ -78,7 +82,7 @@ def parse_args(argv=None):
                    help='the thresholds are this quantile (in (0, 1]) of the calibration pixels and of the calibration images\' map maxima; '
                         'a pixel / image is defective when its score is above it')
     p.add_argument('--save-calibrated-masks', action='store_true', default=False,
-                   help='write <output-dir>/calibrated/<split>/<stem>_{ssim,se}.png: each map thresholded at its calibrated pixel '
+                   help='write <output-dir>/calibrated/<split>/<stem>_{ssim,se[,gms]}.png: each map thresholded at its calibrated pixel '
                         'threshold (uint8 0 / 255); needs --calibration-dir')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
@@ -212,18 +216,23 @@ class BatchedEvaluator:
     the GPU.  Host tensors are copied with non_blocking=True (pin them for overlap).
 
     maps = (win_size, sigma) also computes the anomaly maps of every step (ops.anomaly_maps on the step's uint8 SR / HR):
-    `last_maps` = (1 - SSIM map, squared-error map, per-image max of both), next to `last_sr_u8` and `last_hr_u8`."""
+    `last_maps` = (1 - SSIM map, squared-error map, per-image max of both), next to `last_sr_u8` and `last_hr_u8`.  gms=True (needs maps)
+    adds the MSGMS map of the same sigma (ops.gms_map): `last_maps` = (1 - SSIM map, squared-error map, MSGMS map, per-image max of the
+    three [B, 3]).  Either way the maps are all entries but the last, the maxima the last one."""
 
     def __init__(self, model, rgb_range: float, window_sizes: Optional[Sequence[int]] = None,
-                 maps: Optional[Tuple[int, float]] = None):
+                 maps: Optional[Tuple[int, float]] = None, gms: bool = False):
+        if gms and maps is None:
+            raise ValueError("gms=True needs maps=(win_size, sigma): the MSGMS map comes with the other maps and uses their sigma")
         self.model = model
         self.rgb_range = float(rgb_range)
         self.window_sizes = list(window_sizes) if window_sizes is not None else None
         self.maps = (int(maps[0]), float(maps[1])) if maps is not None else None
+        self.gms = bool(gms)
         self.device = torch.device('cuda')
         self.last_sr_u8: Optional[torch.Tensor] = None
         self.last_hr_u8: Optional[torch.Tensor] = None
-        self.last_maps: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None
+        self.last_maps: Optional[Tuple[torch.Tensor, ...]] = None
         self._copy_stream = None
         self._graphs = {}
         self.use_graph = os.environ.get('ADSR_CUDA_GRAPH', '1') != '0'
@@ -249,7 +258,7 @@ class BatchedEvaluator:
         target = self.model.model if hasattr(self.model, 'model') else self.model
         packed = target._pack() if hasattr(target, '_pack') else None     # repacked weights (new parameters) -> a new graph
         key = (lr_d.data_ptr(), hr_d.data_ptr(), tuple(lr_d.shape), tuple(hr_d.shape), lr_d.dtype, hr_d.dtype,
-               tuple(self.window_sizes) if self.window_sizes is not None else None, id(packed), self.maps)
+               tuple(self.window_sizes) if self.window_sizes is not None else None, id(packed), self.maps, self.gms)
         ent = self._graphs.get(key)
         if ent is None:
             while len(self._graphs) >= 8:                     # evict the oldest entry only (no recapture thrash)
@@ -301,6 +310,9 @@ class BatchedEvaluator:
         self.last_hr_u8 = hr_u8
         scores = metrics.score_batch(sr_u8, hr_u8, self.window_sizes, out)
         self.last_maps = ops.anomaly_maps(sr_u8, hr_u8, *self.maps) if self.maps is not None else None
+        if self.gms:
+            gms, gms_max = ops.gms_map(sr_u8, hr_u8, self.maps[1])
+            self.last_maps = self.last_maps[:2] + (gms, torch.cat([self.last_maps[2], gms_max[:, None]], 1))
         return scores
 
     # ---- double-buffered input path: the host -> device copies of batch i + 1 run on a copy stream while batch i is computed
@@ -468,7 +480,7 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                      anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
                      save_maps: bool = False, au_pro: Optional[float] = None, pr_metrics: bool = False,
                      save_segmentation: bool = False, calibration_dir: Optional[str] = None, calibration_quantile: float = 0.999,
-                     save_calibrated_masks: bool = False):
+                     save_calibrated_masks: bool = False, gms_map: bool = False):
     """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
 
     anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
@@ -489,7 +501,11 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     images is flagged.  Adds calib_{pixel,image}_threshold_{ssim,se} and the test set's calib_image_{tpr,fpr}_{ssim,se}, with mask_dir
     also calib_pixel_{precision,recall,fpr,f1,iou,pro}_{ssim,se} at t_px, printed on a `Map CAL - ...` line before the other `Map`
     lines.  No test label is used to choose the thresholds.  save_calibrated_masks (needs calibration_dir) writes the `map > t_px` masks
-    as uint8 0 / 255 to <output_dir>/calibrated/<split>/<stem>_{ssim,se}.png."""
+    as uint8 0 / 255 to <output_dir>/calibrated/<split>/<stem>_{ssim,se}.png.
+
+    gms_map (implies anomaly_maps) adds a third map kind, the multi-scale gradient-magnitude-similarity map smoothed with map_sigma:
+    everything above is also computed for it, with the suffix _gms in the result keys and file names and `MSGMS` on the printed lines
+    (after the SE entry of each kind)."""
     from .model import Model
 
     if au_pro is not None:
@@ -504,7 +520,9 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     if save_calibrated_masks and calibration_dir is None:
         raise ValueError("save_calibrated_masks needs calibration_dir: the defect-free images the threshold is calibrated on")
     pr_metrics = pr_metrics or save_segmentation
-    anomaly_maps = anomaly_maps or mask_dir is not None or save_maps or calibration_dir is not None
+    anomaly_maps = anomaly_maps or gms_map or mask_dir is not None or save_maps or calibration_dir is not None
+    kinds = [('ssim', '1-SSIM'), ('se', 'SE')] + ([('gms', 'MSGMS')] if gms_map else [])   # (key / file suffix, printed label)
+    n_maps = len(kinds)
     scale = opt.scale[-1] if isinstance(opt.scale, list) else int(opt.scale)
     rank, world = _dist_info()
     if mask_dir is not None and world > 1:
@@ -546,7 +564,7 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     opt.pre_train = checkpoint_model_path
     model = Model(opt, None)
     ev = BatchedEvaluator(model, opt.rgb_range, metrics.window_sizes_for(min_dim),
-                          maps=(map_window_size, map_sigma) if anomaly_maps else None)
+                          maps=(map_window_size, map_sigma) if anomaly_maps else None, gms=gms_map)
     bs = batch_size or getattr(opt, 'eval_batch_size', None) or 64
     mine = list(range(rank, len(entries), world))            # image index i -> rank i mod R
     rows, ids = [], []
@@ -566,26 +584,26 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
 
     t_px = t_img = px_above = None
     if cal_files:                                            # calibration pass: maps of the defect-free images, no labels
-        cal = metrics.LocalisationAccumulator(2)
+        cal = metrics.LocalisationAccumulator(n_maps)
         cal_max = []
         with torch.no_grad():
             for _ in ev.run_pipelined(host_batches(cal_files, list(range(len(cal_files))), [])):
-                cal.append(ev.last_maps[:2])                   # device copies, ordered before the next replay overwrites the maps
-                cal_max.append(ev.last_maps[2].clone())
+                cal.append(ev.last_maps[:-1])                  # device copies, ordered before the next replay overwrites the maps
+                cal_max.append(ev.last_maps[-1].clone())
         q = float(calibration_quantile)
         cal_max = torch.cat(cal_max).cpu().numpy()
-        t_px = [cal.quantile(j, q) for j in range(2)]
-        t_img = [float(np.quantile(cal_max[:, j], q, method='inverted_cdf')) for j in range(2)]
+        t_px = [cal.quantile(j, q) for j in range(n_maps)]
+        t_img = [float(np.quantile(cal_max[:, j], q, method='inverted_cdf')) for j in range(n_maps)]
         px_above = [above(t) for t in t_px]
         del cal                                              # the calibration maps are freed before the test pass
 
     order: List[List[int]] = []
-    loc = metrics.LocalisationAccumulator(2) if mask_dir is not None else None   # both maps of every image, kept on the device
+    loc = metrics.LocalisationAccumulator(n_maps) if mask_dir is not None else None   # every map of every image, kept on the device
     test_files = [(e[2], e[3]) for e in entries]
     with torch.no_grad():
         for k, scores in enumerate(ev.run_pipelined(host_batches(test_files, mine, order))):   # PNG decode + H2D of batch k + 1 overlap batch k
-            if ev.last_maps is not None:                      # the two map maxima ride along in the gathered score table
-                scores = torch.cat([scores, ev.last_maps[2]], 1)
+            if ev.last_maps is not None:                      # the map maxima ride along in the gathered score table
+                scores = torch.cat([scores, ev.last_maps[-1]], 1)
             rows.append(scores)
             ids += order[k]
             if save_images:
@@ -594,15 +612,15 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                     name = os.path.splitext(os.path.basename(entries[i][2]))[0]
                     save_sr_image(sr_np[j], output_dir, name, entries[i][1], scale)
             if save_maps:
-                m_ssim, m_se = ev.last_maps[0].cpu().numpy(), ev.last_maps[1].cpu().numpy()
+                host_maps = [m.cpu().numpy() for m in ev.last_maps[:-1]]
                 for j, i in enumerate(order[k]):
                     name = os.path.splitext(os.path.basename(entries[i][2]))[0]
                     d = Path(output_dir) / 'maps' / entries[i][1]
                     d.mkdir(parents=True, exist_ok=True)
-                    np.save(d / f'{name}_ssim.npy', m_ssim[j])
-                    np.save(d / f'{name}_se.npy', m_se[j])
+                    for (kind, _), m in zip(kinds, host_maps):
+                        np.save(d / f'{name}_{kind}.npy', m[j])
             if save_calibrated_masks:
-                for j, kind in enumerate(('ssim', 'se')):
+                for j, (kind, _) in enumerate(kinds):
                     pred = (ev.last_maps[j] >= px_above[j]).cpu().numpy()
                     for b, i in enumerate(order[k]):
                         name = os.path.splitext(os.path.basename(entries[i][2]))[0]
@@ -615,9 +633,9 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                     with Image.open(entries[i][3]) as im_lr:
                         crop = (im_lr.size[1] * scale, im_lr.size[0] * scale)
                     batch_masks.append(load_mask(mask_paths[i], tuple(ev.last_maps[0].shape[1:]), crop))
-                loc.append(ev.last_maps[:2], batch_masks)  # device copies, ordered before the next replay overwrites the maps
+                loc.append(ev.last_maps[:-1], batch_masks)  # device copies, ordered before the next replay overwrites the maps
     n_cols = len(ev.window_sizes) + 2
-    local = torch.cat(rows) if rows else torch.empty(0, n_cols + (2 if anomaly_maps else 0), dtype=torch.float64, device='cuda')
+    local = torch.cat(rows) if rows else torch.empty(0, n_cols + (n_maps if anomaly_maps else 0), dtype=torch.float64, device='cuda')
     table = gather_scores(local, torch.tensor(ids, dtype=torch.int64, device='cuda'), len(entries))
     if table is None:
         return None
@@ -625,13 +643,15 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
     best_ws, auc_ssim, auc_mse, auc_psnr = metrics.aucs_from_scores(y_true, table, ev.window_sizes)
     res = dict(best_ws=best_ws, auc_ssim=auc_ssim, auc_mse=auc_mse, auc_psnr=auc_psnr, n=len(entries), scores=table)
     if anomaly_maps:
-        res.update(map_max=map_max, auc_map_ssim=metrics.roc_auc(y_true, map_max[:, 0]), auc_map_se=metrics.roc_auc(y_true, map_max[:, 1]))
-        line = (f"Map AUCs - max 1-SSIM(ws={map_window_size}, sigma={float(map_sigma)}): {res['auc_map_ssim']:.4f}, "
-                f"max SE: {res['auc_map_se']:.4f}")
+        res['map_max'] = map_max
+        for j, (kind, _) in enumerate(kinds):
+            res[f'auc_map_{kind}'] = metrics.roc_auc(y_true, map_max[:, j])
+        params = {'ssim': f'(ws={map_window_size}, sigma={float(map_sigma)})'}
+        line = "Map AUCs - " + ", ".join(f"max {label}{params.get(kind, '')}: {res['auc_map_' + kind]:.4f}" for kind, label in kinds)
         if t_px is not None:
             y = np.asarray(y_true)
             parts = []
-            for j, kind, label in ((0, 'ssim', '1-SSIM'), (1, 'se', 'SE')):
+            for j, (kind, label) in enumerate(kinds):
                 flagged = map_max[:, j] >= above(t_img[j])
                 tpr, fpr = float(flagged[y == 1].mean()), float(flagged[y == 0].mean())
                 res.update({f'calib_pixel_threshold_{kind}': t_px[j], f'calib_image_threshold_{kind}': t_img[j],
@@ -646,25 +666,27 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
             print(f"Map CAL - q={float(calibration_quantile):g} on {len(cal_files)} defect-free images: " + "; ".join(parts))
         if mask_dir is not None:
             limit = 0.3 if au_pro is None else float(au_pro)
-            m_ssim, m_se = loc.results(limit)
-            res.update(pixel_auroc_ssim=m_ssim.pixel_auroc, pixel_auroc_se=m_se.pixel_auroc)
-            line += f", pixel AUROC 1-SSIM: {res['pixel_auroc_ssim']:.4f}, pixel AUROC SE: {res['pixel_auroc_se']:.4f}"
+            loc_res = loc.results(limit)                      # one LocalisationMetrics per map kind
+            for (kind, _), m in zip(kinds, loc_res):
+                res[f'pixel_auroc_{kind}'] = m.pixel_auroc
+            line += "".join(f", pixel AUROC {label}: {m.pixel_auroc:.4f}" for (_, label), m in zip(kinds, loc_res))
             if pr_metrics:
-                res.update(pixel_ap_ssim=m_ssim.pixel_ap, pixel_ap_se=m_se.pixel_ap, f1_max_ssim=m_ssim.f1_max, f1_max_se=m_se.f1_max,
-                           f1_threshold_ssim=m_ssim.f1_threshold, f1_threshold_se=m_se.f1_threshold)
-                print(f"Map PR - pixel AP 1-SSIM: {m_ssim.pixel_ap:.4f}, pixel AP SE: {m_se.pixel_ap:.4f}, "
-                      f"F1-max 1-SSIM: {m_ssim.f1_max:.4f} (thr {m_ssim.f1_threshold:g}), "
-                      f"F1-max SE: {m_se.f1_max:.4f} (thr {m_se.f1_threshold:g})")
+                for (kind, _), m in zip(kinds, loc_res):
+                    res.update({f'pixel_ap_{kind}': m.pixel_ap, f'f1_max_{kind}': m.f1_max, f'f1_threshold_{kind}': m.f1_threshold})
+                print("Map PR - " + ", ".join(f"pixel AP {label}: {m.pixel_ap:.4f}" for (_, label), m in zip(kinds, loc_res)) + ", " +
+                      ", ".join(f"F1-max {label}: {m.f1_max:.4f} (thr {m.f1_threshold:g})" for (_, label), m in zip(kinds, loc_res)))
             if save_segmentation:                             # the accumulator holds the images in `ids` order
-                for j, (kind, m) in enumerate((('ssim', m_ssim), ('se', m_se))):
+                for j, ((kind, _), m) in enumerate(zip(kinds, loc_res)):
                     for i, seg in zip(ids, loc.segmentation(j, m.f1_threshold)):
                         name = os.path.splitext(os.path.basename(entries[i][2]))[0]
                         d = Path(output_dir) / 'segmentation' / entries[i][1]
                         d.mkdir(parents=True, exist_ok=True)
                         Image.fromarray(seg.astype(np.uint8) * 255).save(str(d / f'{name}_{kind}.png'))
             if au_pro is not None:
-                res.update(au_pro_ssim=m_ssim.au_pro, au_pro_se=m_se.au_pro, pro_fpr_limit=limit)
-                print(f"Map PRO - AU-PRO@{limit:g} 1-SSIM: {m_ssim.au_pro:.4f}, AU-PRO@{limit:g} SE: {m_se.au_pro:.4f}")
+                for (kind, _), m in zip(kinds, loc_res):
+                    res[f'au_pro_{kind}'] = m.au_pro
+                res['pro_fpr_limit'] = limit
+                print("Map PRO - " + ", ".join(f"AU-PRO@{limit:g} {label}: {m.au_pro:.4f}" for (_, label), m in zip(kinds, loc_res)))
         print(line)
     print(f"Test AUCs - SSIM(best ws={best_ws}): {auc_ssim:.4f}, MSE: {auc_mse:.4f}, PSNR: {auc_psnr:.4f}")
     return res
@@ -709,7 +731,8 @@ def main(argv=None):
                             map_window_size=args.map_window_size, map_sigma=args.map_sigma, mask_dir=args.mask_dir,
                             save_maps=args.save_maps, au_pro=args.au_pro, pr_metrics=args.pr_metrics,
                             save_segmentation=args.save_segmentation, calibration_dir=args.calibration_dir,
-                            calibration_quantile=args.calibration_quantile, save_calibrated_masks=args.save_calibrated_masks)
+                            calibration_quantile=args.calibration_quantile, save_calibrated_masks=args.save_calibrated_masks,
+                            gms_map=args.gms_map)
 
 
 if __name__ == "__main__":

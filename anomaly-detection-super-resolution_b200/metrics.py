@@ -97,6 +97,14 @@ def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int = 11, s
     return ops.anomaly_maps(sr_u8, hr_u8, win_size, sigma)
 
 
+def gms_map(sr_u8: torch.Tensor, hr_u8: torch.Tensor, sigma: float = 0.0):
+    """Where edge structure was not reconstructed: uint8 NHWC device tensors -> (multi-scale gradient-magnitude-similarity map, per-image
+    max) as fp32 [B, H, W], fp64 [B].  RIAD's MSGMS on the gray plane of anomaly_maps: 4 pyramid levels of 2 x 2 means, Prewitt gradient
+    magnitudes, 1 - GMS with c = 0.0026 per level, bilinear upsampling, mean over the levels.  sigma > 0 smooths it like anomaly_maps
+    before the max is taken."""
+    return ops.gms_map(sr_u8, hr_u8, sigma)
+
+
 def _map_pieces(maps):
     """A CUDA map set -> (list of fp32 tensors to append in order, list of per-image (H, W) shapes)."""
     if isinstance(maps, torch.Tensor):

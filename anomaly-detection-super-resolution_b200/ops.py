@@ -339,6 +339,49 @@ def anomaly_maps(sr_u8: torch.Tensor, hr_u8: torch.Tensor, win_size: int, sigma:
     return ssim_map, se_map, map_max
 
 
+def gms_workspace_bytes(b: int, h: int, w: int) -> int:
+    """Bytes of scratch adsr_gms_map needs for B images of H x W (both gray pyramids, the per-level similarity planes, the Gaussian
+    scratch)."""
+    n = int(lib().adsr_gms_workspace_bytes(int(b), int(h), int(w)))
+    if n < 0:
+        raise ValueError(f"gms_map: unsupported batch shape {b} x {h} x {w}")
+    return n
+
+
+def gms_map(sr_u8: torch.Tensor, hr_u8: torch.Tensor, sigma: float = 0.0,
+            out: Optional[tuple] = None) -> tuple[torch.Tensor, torch.Tensor]:
+    """uint8 NHWC pairs -> (gms_map fp32 [B, H, W] = the multi-scale gradient-magnitude-similarity map (1/4) sum over 4 pyramid levels
+    of the upsampled 1 - GMS of the gray planes, map_max fp64 [B] = per-image max of the map), Gaussian-smoothed like anomaly_maps when
+    sigma > 0.  out: caller-owned (gms_map, map_max, workspace) to write into; workspace is uint8 [>= gms_workspace_bytes(B, H, W)].
+    Without `out` everything is allocated here.  Four kernels, six with the smoothing."""
+    _cuda(sr_u8, "sr_u8")
+    _cuda(hr_u8, "hr_u8")
+    if sr_u8.dtype != torch.uint8 or hr_u8.dtype != torch.uint8:
+        raise TypeError(f"gms_map takes uint8 images, got {sr_u8.dtype} / {hr_u8.dtype}")
+    if sr_u8.dim() != 4 or sr_u8.shape != hr_u8.shape or sr_u8.device != hr_u8.device:
+        raise ValueError(f"gms_map needs two [B, H, W, C] images of one shape on one device, got {tuple(sr_u8.shape)} on "
+                         f"{sr_u8.device} and {tuple(hr_u8.shape)} on {hr_u8.device}")
+    sr_u8, hr_u8 = sr_u8.contiguous(), hr_u8.contiguous()
+    b, h, w, c = sr_u8.shape
+    ws_bytes = gms_workspace_bytes(b, h, w)
+    if out is None:
+        out = (torch.empty(b, h, w, dtype=torch.float32, device=sr_u8.device), torch.empty(b, dtype=torch.float64, device=sr_u8.device),
+               torch.empty(ws_bytes, dtype=torch.uint8, device=sr_u8.device))
+    gms, map_max, workspace = out
+    for t, name, dt, shape in ((gms, "gms_map", torch.float32, (b, h, w)), (map_max, "map_max", torch.float64, (b,))):
+        if t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous() or t.device != sr_u8.device:
+            raise ValueError(f"gms_map: {name} must be a contiguous {dt} tensor of shape {shape} on {sr_u8.device}")
+    if workspace.dtype != torch.uint8 or not workspace.is_contiguous() or workspace.device != sr_u8.device or workspace.numel() < ws_bytes:
+        raise ValueError(f"gms_map: workspace must be a contiguous uint8 tensor of at least {ws_bytes} bytes on {sr_u8.device}")
+    _t = _begin()
+    check(lib().adsr_gms_map(ptr(sr_u8), ptr(hr_u8), b, h, w, c, float(sigma), ptr(gms), ptr(map_max), ptr(workspace), stream_ptr()),
+          "adsr_gms_map")
+    global LAUNCHES
+    LAUNCHES += 5 if sigma > 0 else 3                  # pyramid, levels, combine [+ row / column Gaussian passes]; _count adds the max
+    _count("gms_map", 0.0, _t)
+    return gms, map_max
+
+
 def localisation_workspace_bytes(n: int) -> int:
     """Bytes of scratch adsr_localisation_metrics needs for n pixels (two key / region buffer pairs, sort histograms, tile sums)."""
     b = int(lib().adsr_localisation_workspace_bytes(int(n)))

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 18
+#define ADSR_ABI_VERSION 19
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -265,6 +265,23 @@ int adsr_score_images_strided(const void* sr, const void* hr, int is_f32, int B,
 int adsr_anomaly_maps(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B, int H, int W, int C,
                       int win_size, float sigma, float* ssim_map, float* se_map, float* scratch,
                       double* map_max, void* stream);
+
+/* Multi-scale gradient-magnitude-similarity (MSGMS) map of uint8 HWC SR / HR pairs (RIAD, Zavrtanik et al. 2021, after GMSD, Xue et
+ * al. 2014), for defect localisation next to adsr_anomaly_maps.  On the gray plane of the 1 - SSIM map (x = HR, y = SR, in [0, 1]):
+ * 4 pyramid levels (level k + 1 = avg_pool2d(level k, 2, 2), odd sizes floored); at each level Prewitt gradient magnitudes
+ * g = sqrt(gx^2 + gy^2 + 1e-12) (kernels [[1/3, 0, -1/3]] x 3 and its transpose, zero padding) and
+ * gms = (2 g_x g_y + c) / (g_x^2 + g_y^2 + c), c = 0.0026; the map is (1/4) sum_k up_k(1 - gms_k), up_k = bilinear resize to H x W
+ * (align_corners = False), summed in level order.  sigma > 0 smooths it with the Gaussian of adsr_anomaly_maps (same radius rule and
+ * limit).  fp32 arithmetic; the GMS products are rounded one by one, so an identical pair gives exact zeros.
+ * gms_map: fp32 [B, H, W]; map_max: fp64 [B] = per-image max of the final map; workspace: adsr_gms_workspace_bytes(B, H, W) bytes,
+ * 4-byte aligned (pyramids of both images, per-level similarity planes, Gaussian scratch).  No allocation, no synchronisation; the
+ * launch count is fixed by (B, H, W, sigma): 4 kernels, 6 with smoothing.
+ * ADSR_ERR_BAD_SHAPE: C not 1 or 3, H < 8, W < 8, B H W >= 2^31, sigma NaN or < 0, r > 64, r >= min(H, W), or a NULL workspace or
+ * output with B > 0.  Deterministic; image i does not depend on the rest of the batch.
+ * adsr_gms_workspace_bytes: -1 for negative sizes. */
+int64_t adsr_gms_workspace_bytes(int B, int H, int W);
+int adsr_gms_map(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B, int H, int W, int C, float sigma, float* gms_map,
+                 double* map_max, void* workspace, void* stream);
 
 /* Localisation metrics of ONE anomaly map over a whole test set: pixel AUROC, AU-PRO@fpr_limit, pixel AP and F1-max with its threshold,
  * exact (no threshold binning).
