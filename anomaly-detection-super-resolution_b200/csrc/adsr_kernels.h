@@ -44,6 +44,19 @@ inline cudaError_t launch_pdl(Kernel kernel, dim3 grid, dim3 block, size_t smem,
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// SSIM of one pixel from its five window sums (x, y, x^2, y^2, xy) and 1 / (ws * ws), shared by the three scorer kernels
+// (scoring.cu) and the 1 - SSIM map (anomaly_maps.cu).  Every operation is rounded on its own (no FMA contraction), so the kernels
+// give the same bits for the same window sums, and for an identical pair (sums 0 == 1, 2 == 3 == 4) the numerator and the
+// denominator are the same double: exactly 1.
+__device__ __forceinline__ double ssim_term(const double (&sum)[5], double inv_n, double C1, double C2) {
+    const double mu1 = __dmul_rn(sum[0], inv_n), mu2 = __dmul_rn(sum[1], inv_n);
+    const double m11 = __dmul_rn(mu1, mu1), m22 = __dmul_rn(mu2, mu2), m12 = __dmul_rn(mu1, mu2);
+    const double s1 = __dsub_rn(__dmul_rn(sum[2], inv_n), m11), s2 = __dsub_rn(__dmul_rn(sum[3], inv_n), m22),
+                 s12 = __dsub_rn(__dmul_rn(sum[4], inv_n), m12);
+    return __ddiv_rn(__dmul_rn(__dadd_rn(__dmul_rn(2.0, m12), C1), __dadd_rn(__dmul_rn(2.0, s12), C2)),
+                     __dmul_rn(__dadd_rn(__dadd_rn(m11, m22), C1), __dadd_rn(__dadd_rn(s1, s2), C2)));
+}
 #endif
 
 struct TcGemmParams {

@@ -128,14 +128,10 @@ __global__ void __launch_bounds__(1024) anomaly_maps_raw_kernel(const RawParams 
                 double t = Pq[a1 + 1] - Pq[a0];
                 if (lo < 0) t += Pq[-lo + 1] - Pq[1];                       // reflected columns 1 .. -lo
                 if (hi > W - 1) t += Pq[W - 1] - Pq[2 * (W - 1) - hi];      // reflected columns 2(W-1)-hi .. W-2
-                box[q] = t * inv_n;
+                box[q] = t;
             }
-            // products rounded on their own (no FMA contraction): for an identical pair m11 = m22 = m12 and s1 = s2 = s12, so the
-            // numerator and the denominator are the same double and the map is exactly 0
-            const double mu1 = box[0], mu2 = box[1];
-            const double m11 = __dmul_rn(mu1, mu1), m22 = __dmul_rn(mu2, mu2), m12 = __dmul_rn(mu1, mu2);
-            const double s1 = box[2] - m11, s2 = box[3] - m22, s12 = box[4] - m12;
-            const double ssim = __dmul_rn(__dmul_rn(2.0, m12) + C1, __dmul_rn(2.0, s12) + C2) / __dmul_rn(m11 + m22 + C1, s1 + s2 + C2);
+            // the scorer's per-pixel term (no FMA contraction): an identical pair gives exactly 0
+            const double ssim = ssim_term(box, inv_n, C1, C2);
             const long long o = img + static_cast<long long>(i) * W + col;
             p.ssim_map[o] = static_cast<float>(1.0 - ssim);
         }

@@ -11,15 +11,18 @@
 // into prefix sums across the row (warp shuffles + one shared-memory hop), so each horizontal window
 // sum is a difference of two prefix values (three differences when the window reflects at a border).
 // Work per pixel is O(1) in the window size; the images are read straight from L2 as uint8 and no
-// workspace is needed.  Sums are fp64, so the result equals the vectorised oracle to ~1e-12 and the
-// reference's fp32 loop to ~1e-6.
+// workspace is needed.  Sums are fp64 and the per-pixel term is ssim_term (adsr_kernels.h), so the result is
+// within 1e-10 of the kernel-faithful oracle (oracle/scoring_oracle.py: the kernels' fmaf gray chain, exact
+// window sums; MSE to 1e-14 relative) and within ~1e-6 of the reference's fp32 loop; an identical pair gives
+// exactly 1.  The two kernels for images of up to 128 columns sum in the same order, so an image's row does
+// not depend on the batch size that picks between them (tests/test_gpu_scoring_dispatch.py).
 #include "adsr_kernels.h"
 #include "ptx.cuh"
 
 namespace adsr {
 namespace {
 
-constexpr int kMaxWs = 64;
+constexpr int kMaxWs = 128;      // metrics.window_sizes_for(1024) gives 102 window sizes; W <= 1024 is the kernels' own limit
 struct WsList { int32_t ws[kMaxWs]; };
 
 __device__ __forceinline__ int reflect_idx(int i, int n) {        // np.pad(mode="reflect"), |overhang| < n
@@ -184,11 +187,9 @@ __global__ void __launch_bounds__(1024) score_images_kernel(const ScoreParams p)
                     if (lo < 0) t += Pq[-lo + 1] - Pq[1];                       // reflected columns 1 .. -lo
                     if (hi > W - 1) t += Pq[W - 1] - Pq[2 * (W - 1) - hi];      // reflected columns 2(W-1)-hi .. W-2
                 }
-                box[q] = t * inv_n;
+                box[q] = t;
             }
-            const double mu1 = box[0], mu2 = box[1];
-            const double s1 = box[2] - mu1 * mu1, s2 = box[3] - mu2 * mu2, s12 = box[4] - mu1 * mu2;
-            acc += ((2.0 * mu1 * mu2 + C1) * (2.0 * s12 + C2)) / ((mu1 * mu1 + mu2 * mu2 + C1) * (s1 + s2 + C2));
+            acc += ssim_term(box, inv_n, C1, C2);
         }
     }
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
@@ -342,11 +343,9 @@ __global__ void __launch_bounds__(kFastThreads, 1) score_images_fast_kernel(cons
                             if (lo < 0) t += Pq[pidx(-lo + 1)] - Pq[pidx(1)];                       // reflected columns 1 .. -lo
                             if (hi > W - 1) t += Pq[pidx(W - 1)] - Pq[pidx(2 * (W - 1) - hi)];      // reflected columns 2(W-1)-hi .. W-2
                         }
-                        box[q] = t * inv_n;
+                        box[q] = t;
                     }
-                    const double mu1 = box[0], mu2 = box[1];
-                    const double s1 = box[2] - mu1 * mu1, s2 = box[3] - mu2 * mu2, s12 = box[4] - mu1 * mu2;
-                    acc += ((2.0 * mu1 * mu2 + C1) * (2.0 * s12 + C2)) / ((mu1 * mu1 + mu2 * mu2 + C1) * (s1 + s2 + C2));
+                    acc += ssim_term(box, inv_n, C1, C2);
                 }
             }
             __syncwarp();                                              // the next row overwrites the prefix rows
@@ -357,10 +356,13 @@ __global__ void __launch_bounds__(kFastThreads, 1) score_images_fast_kernel(cons
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Small-batch variant of the fast path (round 1's layout): 8 workers of 128 threads per CTA, one column per thread, worker k
-// runs window sizes k, k + 8, ... with a cross-warp prefix (two named barriers per row).  It issues ~2x the instructions of the
-// warp-per-window kernel above but finishes ONE window size in a quarter of the time, which is what counts when the batch leaves
-// SMs idle (DRN-L's batch of 64: two CTAs per image, 0.47 ms instead of 0.57 ms).
+// Small-batch variant of the fast path: 8 workers of 128 threads per CTA, one column per thread, worker k runs window sizes
+// k, k + 8, ... with a cross-warp prefix (two named barriers per row).  It issues more instructions than the warp-per-window kernel
+// above but finishes ONE window size in about a quarter of the time, which is what counts when the batch leaves SMs idle.
+// It produces the warp-per-window kernel's bits, so an image's score row does not depend on which of the two the batch size picks:
+// the MSE is reduced by the first 16 warps in that kernel's order; a column's sums form a sequential prefix within its group of 4
+// columns (the fast kernel's lane), the 32 group totals go through the same Hillis-Steele scan and P = (scan - total) + prefix;
+// the group leader adds its 4 columns' SSIM terms in column order and the 32 group sums end in one xor butterfly.
 constexpr int kFastWorkers = 8;
 
 __global__ void __launch_bounds__(1024, 1) score_images_fast4_kernel(const ScoreParams p) {
@@ -371,40 +373,47 @@ __global__ void __launch_bounds__(1024, 1) score_images_fast4_kernel(const Score
     const int part = blockIdx.y, nparts = gridDim.y;                    // small batches: the window sizes of an image split over CTAs
     const long long srb = static_cast<long long>(b) * p.sr.sb, hrb = static_cast<long long>(b) * p.hr.sb;
     double* red = sm;                                                   // [32]
-    double* wbase = sm + 32;                                            // per worker: wtot [2][5][4], pref [2][5][W+1]
-    const int wstride = 2 * 5 * 4 + 2 * 5 * (W + 1);
+    double* wbase = sm + 32;                                            // per worker: gtot [5][32], pref [5][W + 1]
+    const int wstride = 5 * 32 + 5 * (W + 1);
     float* gx = reinterpret_cast<float*>(wbase + kFastWorkers * wstride);   // HR gray plane
     float* gy = gx + H * W;                                             // SR gray plane
 
-    // ---- gray planes + MSE
-    double acc_mse = 0.0;
+    // ---- gray planes, then the MSE in score_images_fast_kernel's order (thread t < 512 takes pixels t, t + 512, ...)
     for (int idx = tid; idx < H * W; idx += 1024) {
         const int r = idx / W, c = idx - r * W;
-        const long long oh = hrb + r * p.hr.sr + c * p.hr.sc, os = srb + r * p.sr.sr + c * p.sr.sc;
-        gx[idx] = gray_at(p.hr, oh, C);
-        gy[idx] = gray_at(p.sr, os, C);
-        for (int ch = 0; ch < C; ++ch) {
-            const float d = fetch_mse(p.sr, os + ch * p.sr.sch, p.mse_noclamp) - fetch_mse(p.hr, oh + ch * p.hr.sch, p.mse_noclamp);
-            acc_mse += static_cast<double>(d * d);
-        }
+        gx[idx] = gray_at(p.hr, hrb + r * p.hr.sr + c * p.hr.sc, C);
+        gy[idx] = gray_at(p.sr, srb + r * p.sr.sr + c * p.sr.sc, C);
     }
-    for (int o = 16; o > 0; o >>= 1) acc_mse += __shfl_xor_sync(0xffffffffu, acc_mse, o);
-    if (lane == 0) red[warp] = acc_mse;
+    if (part == 0 && warp < kFastWarps) {
+        double acc_mse = 0.0;
+        for (int idx = tid; idx < H * W; idx += kFastThreads) {
+            const int r = idx / W, c = idx - r * W;
+            const long long oh = hrb + r * p.hr.sr + c * p.hr.sc, os = srb + r * p.sr.sr + c * p.sr.sc;
+            for (int ch = 0; ch < C; ++ch) {
+                const float d = fetch_mse(p.sr, os + ch * p.sr.sch, p.mse_noclamp) - fetch_mse(p.hr, oh + ch * p.hr.sch, p.mse_noclamp);
+                acc_mse += static_cast<double>(d * d);
+            }
+        }
+        for (int o = 16; o > 0; o >>= 1) acc_mse += __shfl_xor_sync(0xffffffffu, acc_mse, o);
+        if (lane == 0) red[warp] = acc_mse;
+    }
     __syncthreads();
     if (tid == 0 && part == 0) {
         double t = 0;
-        for (int w = 0; w < 32; ++w) t += red[w];
+        for (int w = 0; w < kFastWarps; ++w) t += red[w];
         const double mse = t / (static_cast<double>(H) * W * C);
         p.scores[static_cast<long long>(b) * (n_ws + 2) + n_ws] = mse;
         p.scores[static_cast<long long>(b) * (n_ws + 2) + n_ws + 1] =
             mse == 0.0 ? __longlong_as_double(0x7ff0000000000000LL) : 10.0 * log10(p.psnr_peak2 / mse);
     }
 
-    // ---- SSIM sweep: worker = 4 warps, thread = column
-    const int worker = tid >> 7, col = tid & 127, wwarp = warp & 3;
+    // ---- SSIM sweep: worker = 4 warps, thread = column, group g = the 4 columns a fast-kernel lane owns
+    const int worker = tid >> 7, col = tid & 127, wwarp = warp & 3, k = col & 3, g = col >> 2;
     const bool active = col < W;
-    double* wtot = wbase + worker * wstride;                            // [2][5][4]
-    double* pref = wtot + 2 * 5 * 4;                                    // [2][5][W + 1]
+    // Single-buffered scratch: gtot is read only between a row's two barriers and written before the next row's first one; pref
+    // is written after a row's first barrier and read after its second, before the next row's first one.
+    double* gtot = wbase + worker * wstride;                            // [5][32] group totals, then the 32 group SSIM sums
+    double* P = gtot + 5 * 32;                                          // [5][W + 1]
     const bool zp = p.zero_pad != 0;
     const double C1 = p.C1, C2 = p.C2;
     for (int j = worker + kFastWorkers * part; j < n_ws; j += kFastWorkers * nparts) {
@@ -424,9 +433,8 @@ __global__ void __launch_bounds__(1024, 1) score_images_fast4_kernel(const Score
                 if (zp) { if (r >= 0 && r < H) add_row(r, 1.0); }
                 else add_row(reflect_idx(r, H), 1.0);
             }
-        double acc = 0.0;
+        double acc = 0.0;                                               // group leader: SSIM sum of its 4 columns
         for (int i = 0; i < H; ++i) {
-            const int bufi = i & 1;
             if (i > 0 && active) {
                 if (zp) {
                     if (i + pad < H) add_row(i + pad, 1.0);
@@ -436,28 +444,33 @@ __global__ void __launch_bounds__(1024, 1) score_images_fast4_kernel(const Score
                     add_row(reflect_idx(i - pad - 1, H), -1.0);
                 }
             }
-            double s5[5];
+            double l[5];                                                // prefix of my column within its group, left to right
 #pragma unroll
             for (int q = 0; q < 5; ++q) {
-                double t = active ? v[q] : 0.0;
+                double t = v[q];
+#pragma unroll
+                for (int s = 1; s < 4; ++s) {
+                    const double u = shfl_up_d(t, 1);
+                    if (k == s) t = u + t;
+                }
+                l[q] = t;
+                if (k == 3) gtot[q * 32 + g] = t;
+            }
+            named_bar_sync(1 + worker, 128);
+#pragma unroll
+            for (int q = 0; q < 5; ++q) {
+                double t = gtot[q * 32 + lane];                         // every warp scans all 32 group totals
 #pragma unroll
                 for (int d = 1; d < 32; d <<= 1) {
                     const double u = shfl_up_d(t, d);
                     if (lane >= d) t += u;
                 }
-                s5[q] = t;
-                if (lane == 31) wtot[(bufi * 5 + q) * 4 + wwarp] = t;
-            }
-            named_bar_sync(1 + worker, 128);
-            double* P = pref + bufi * 5 * (W + 1);
-#pragma unroll
-            for (int q = 0; q < 5; ++q) {
-                double base = 0.0;
-                for (int w = 0; w < wwarp; ++w) base += wtot[(bufi * 5 + q) * 4 + w];
-                if (active) P[q * (W + 1) + col + 1] = s5[q] + base;
+                const double base = __shfl_sync(0xffffffffu, t, g) - gtot[q * 32 + g];   // sum of the groups to my left
+                if (active) P[q * (W + 1) + col + 1] = base + l[q];
                 if (col == 0) P[q * (W + 1)] = 0.0;
             }
             named_bar_sync(1 + worker, 128);
+            double term = 0.0;
             if (active) {
                 const int lo = col - pad, hi = col + pad;
                 const int a0 = lo < 0 ? 0 : lo, a1 = hi > W - 1 ? W - 1 : hi;
@@ -470,20 +483,27 @@ __global__ void __launch_bounds__(1024, 1) score_images_fast4_kernel(const Score
                         if (lo < 0) t += Pq[-lo + 1] - Pq[1];
                         if (hi > W - 1) t += Pq[W - 1] - Pq[2 * (W - 1) - hi];
                     }
-                    box[q] = t * inv_n;
+                    box[q] = t;
                 }
-                const double mu1 = box[0], mu2 = box[1];
-                const double s1 = box[2] - mu1 * mu1, s2 = box[3] - mu2 * mu2, s12 = box[4] - mu1 * mu2;
-                acc += ((2.0 * mu1 * mu2 + C1) * (2.0 * s12 + C2)) / ((mu1 * mu1 + mu2 * mu2 + C1) * (s1 + s2 + C2));
+                term = ssim_term(box, inv_n, C1, C2);
+            }
+            const double t1 = __shfl_down_sync(0xffffffffu, term, 1), t2 = __shfl_down_sync(0xffffffffu, term, 2),
+                         t3 = __shfl_down_sync(0xffffffffu, term, 3);
+            if (k == 0) {
+                if (col < W) acc += term;
+                if (col + 1 < W) acc += t1;
+                if (col + 2 < W) acc += t2;
+                if (col + 3 < W) acc += t3;
             }
         }
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-        named_bar_sync(1 + worker, 128);                                // everyone is done with wtot of the last row
-        if (lane == 0) wtot[wwarp] = acc;
+        if (k == 0) gtot[g] = acc;                                      // the last row's scan reads of gtot are behind its 2nd barrier
         named_bar_sync(1 + worker, 128);
-        if (col == 0)
-            p.scores[static_cast<long long>(b) * (n_ws + 2) + j] = (wtot[0] + wtot[1] + wtot[2] + wtot[3]) / (static_cast<double>(H) * W);
-        named_bar_sync(1 + worker, 128);
+        if (wwarp == 0) {
+            double t = gtot[lane];
+            for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+            if (lane == 0) p.scores[static_cast<long long>(b) * (n_ws + 2) + j] = t / (static_cast<double>(H) * W);
+        }
+        named_bar_sync(1 + worker, 128);                                // gtot is rewritten by the next window size
     }
 }
 
@@ -521,7 +541,7 @@ int launch_score(adsr::ScoreParams& p, int B, const int32_t* host_ws_list, int n
             const int per_worker = (n_ws + kFastWarps * parts - 1) / (kFastWarps * parts);
             return waves * (0.3 + per_worker);
         };
-        const size_t fast4_smem = (32 + kFastWorkers * (2 * 5 * 4 + 2 * 5 * static_cast<size_t>(p.W + 1))) * sizeof(double) +
+        const size_t fast4_smem = (32 + kFastWorkers * (5 * 32 + 5 * static_cast<size_t>(p.W + 1))) * sizeof(double) +
                                   2 * static_cast<size_t>(p.H) * p.W * sizeof(float);
         if (2 * B <= sms && n_ws > kFastWorkers && fast4_smem <= 227 * 1024) {
             // the batch leaves more than half of the SMs idle: latency per window size counts, not instructions per SM

@@ -237,8 +237,10 @@ int adsr_rcab_ca_scale(const void* res, int64_t ldr, const void* x, int64_t ldx,
 /* ---- per-image anomaly scores ---------------------------------------------------------------------------------
  * replaces ssim_numpy (src/metrics.py:26-67) for every window size of the sweep (src/evaluate.py:233-248),
  * MSE (src/evaluate.py:259-260) and psnr_numpy (src/metrics.py:15-23) on uint8 HWC pairs.
- * host_ws_list: int32 [n_ws <= 64] in HOST memory (odd window sizes, ws/2 < min(H,W));
- * scores: fp64 [B, n_ws + 2] = ssim(ws_0..), mse, psnr (+inf when mse == 0). */
+ * host_ws_list: int32 [n_ws <= 128] in HOST memory (odd window sizes, ws/2 < min(H,W)): the evaluator's full sweep of images up to
+ * the kernels' limit of W <= 1024 columns (102 window sizes at 1024 px);
+ * scores: fp64 [B, n_ws + 2] = ssim(ws_0..), mse, psnr (+inf when mse == 0).  An image's row is bit-identical whatever batch it is
+ * scored in; an identical pair gives exactly 1 / 0 / +inf. */
 int adsr_score_images(const uint8_t* sr_u8_hwc, const uint8_t* hr_u8_hwc, int B, int H, int W, int C,
                       const int32_t* host_ws_list, int n_ws, double* scores, void* stream);
 

@@ -93,6 +93,78 @@ def ssim_box(ref01: np.ndarray, out01: np.ndarray, ws: int) -> float:
     return float(np.mean(m))
 
 
+# ---------------------------------------------------------------------------------------------------------------------
+# kernel-faithful restatement: what csrc/scoring.cu and csrc/anomaly_maps.cu compute, to the last bits, for tests that hold the
+# kernels to ~1e-10 instead of the reference's fp32 tolerance
+# ---------------------------------------------------------------------------------------------------------------------
+def gray01_like_kernel(img: np.ndarray) -> np.ndarray:
+    """[H, W, C] (C = 1 or 3) -> fp32 [H, W] gray plane as the kernels build it.  uint8 input is divided by 255 in fp32 first; float
+    input is taken as is.  One channel: as is.  Three channels: the kernels' fmaf chain fmaf(b, c2, fmaf(g, c1, r * c0)) -- r * c0
+    rounded to fp32, then each fmaf formed exactly and rounded once to fp32 (np.longdouble holds the exact sum of an fp32 product and
+    an fp32 value of these magnitudes).  This is NOT the reference's formula: `to_gray01` uses np.tensordot, which can differ from the
+    kernels in the last bit of a pixel."""
+    f = img.astype(np.float32) / np.float32(255.0) if img.dtype == np.uint8 else img.astype(np.float32)
+    if f.ndim == 2:
+        return f
+    if f.shape[2] == 1:
+        return f[:, :, 0]
+    c0, c1, c2 = (np.longdouble(c) for c in GRAY_COEFFS)
+    r, g, b = (f[:, :, k].astype(np.longdouble) for k in range(3))
+    p0 = (r * c0).astype(np.float32)
+    t1 = (g * c1 + p0.astype(np.longdouble)).astype(np.float32)
+    return (b * c2 + t1.astype(np.longdouble)).astype(np.float32)
+
+
+def _prefix2d(x: np.ndarray, pad: int, mode: str) -> np.ndarray:
+    xp = np.pad(x, pad, mode=mode)
+    c = np.zeros((xp.shape[0] + 1, xp.shape[1] + 1), dtype=np.float64)
+    c[1:, 1:] = xp.cumsum(0).cumsum(1)
+    return c
+
+
+def ssim_maps_like_kernel(ref: np.ndarray, out: np.ndarray, window_sizes: Sequence[int], c1: float = 0.01 * 0.01,
+                          c2: float = 0.03 * 0.03, zero_pad: bool = False):
+    """Per-pixel SSIM maps (fp64 [H, W], one per odd window size, yielded in order) of two fp32 gray planes [H, W] as the kernels form
+    them: window sums of the values and of their fp32 products (x * x, y * y, x * y) with np.pad(mode="reflect") borders (zero_pad:
+    zeros, as ssim_torch), then the fp64 term of ssim_term in csrc/adsr_kernels.h (every operation rounded on its own, means =
+    sums * (1 / ws^2)).  The window sums come from a 2-D prefix of each plane split as hi + lo, hi a multiple of 2^-20: the hi sums
+    are exact and the lo sums tiny, so each window sum is the exact one to ~1e-16 relative, well inside the kernels' own rounding.
+    (A plain fp64 prefix reaches H * W in magnitude and loses ~1e-13 on one window, which 1 / C2 turns into ~1e-10 of SSIM.)"""
+    planes = [ref.astype(np.float32), out.astype(np.float32)]
+    planes += [planes[0] * planes[0], planes[1] * planes[1], planes[0] * planes[1]]
+    H, W = ref.shape
+    P = max(window_sizes) // 2
+    mode = "constant" if zero_pad else "reflect"
+    prefixes = []
+    for x in planes:
+        x = x.astype(np.float64)
+        hi = np.round(x * 2.0 ** 20) / 2.0 ** 20
+        prefixes.append((_prefix2d(hi, P, mode), _prefix2d(x - hi, P, mode)))
+    for ws in window_sizes:
+        a, e = P - ws // 2, P + ws // 2 + 1           # prefix rows / columns bounding the window of pixel 0
+
+        def box(c):
+            return c[e:e + H, e:e + W] - c[a:a + H, e:e + W] - c[e:e + H, a:a + W] + c[a:a + H, a:a + W]
+
+        inv_n = 1.0 / (float(ws) * ws)
+        mu1, mu2, e11, e22, e12 = ((box(ch) + box(cl)) * inv_n for ch, cl in prefixes)
+        m11, m22, m12 = mu1 * mu1, mu2 * mu2, mu1 * mu2
+        s1, s2, s12 = e11 - m11, e22 - m22, e12 - m12
+        yield ((2.0 * m12 + c1) * (2.0 * s12 + c2)) / ((m11 + m22 + c1) * (s1 + s2 + c2))
+
+
+def ssim_sweep_like_kernel(ref: np.ndarray, out: np.ndarray, window_sizes: Sequence[int], c1: float = 0.01 * 0.01,
+                           c2: float = 0.03 * 0.03, zero_pad: bool = False) -> np.ndarray:
+    """The scorer's SSIM for each window size: the mean of each of ssim_maps_like_kernel's maps."""
+    return np.array([np.mean(m) for m in ssim_maps_like_kernel(ref, out, window_sizes, c1, c2, zero_pad)], dtype=np.float64)
+
+
+def mse_like_kernel(sr01: np.ndarray, hr01: np.ndarray) -> float:
+    """Mean over every element of (sr - hr)^2 with the difference and its square in fp32, summed in fp64 (the kernels' MSE term)."""
+    d = sr01.astype(np.float32) - hr01.astype(np.float32)
+    return float(np.sum((d * d).astype(np.float64)) / d.size)
+
+
 def mse01(sr_u8: np.ndarray, hr_u8: np.ndarray) -> float:
     """src/evaluate.py:255-260."""
     d = sr_u8.astype(np.float32) / np.float32(255.0) - hr_u8.astype(np.float32) / np.float32(255.0)

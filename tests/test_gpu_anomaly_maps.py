@@ -51,23 +51,35 @@ def _pairs(h, w, c, seed):
     return sr, hr
 
 
+# a partial last band of 16 rows (100, 130, 17), partially active warps (84, 33), the dynamic shared memory of W >= 582 (1024) and a
+# Gaussian radius of H - 1 (sigma 4 on 17 rows: r = 16); "max" is the largest window, ws / 2 = min(H, W) - 1
+MAP_SHAPES = [(128, 128, 3), (128, 128, 1), (64, 96, 3), (256, 256, 3), (100, 84, 3), (130, 33, 3), (17, 1024, 1)]
+
+
 @pytest.mark.parametrize("sigma", [0.0, 4.0])
-@pytest.mark.parametrize("ws", [3, 11, 33])
-@pytest.mark.parametrize("h,w,c", [(128, 128, 3), (128, 128, 1), (64, 96, 3), (256, 256, 3)])
+@pytest.mark.parametrize("ws", [3, 11, 33, "max"])
+@pytest.mark.parametrize("h,w,c", MAP_SHAPES)
 def test_maps_match_oracle(h, w, c, ws, sigma):
+    ws = 2 * min(h, w) - 1 if ws == "max" else ws
     sr, hr = _pairs(h, w, c, seed=h + w + c + ws)
     m_ssim, m_se, m_max = (t.cpu().numpy() for t in ops.anomaly_maps(torch.from_numpy(sr).cuda(), torch.from_numpy(hr).cuda(), ws, sigma))
     assert m_ssim.shape == (4, h, w) and m_se.shape == (4, h, w) and m_max.shape == (4, 2)
     for i in range(4):
         raw_ssim, raw_se = oracle_maps(sr[i], hr[i], ws, 0.0)
         want_ssim, want_se = (raw_ssim, raw_se) if sigma == 0 else oracle_maps(sr[i], hr[i], ws, sigma)
+        if sigma == 0:
+            # the kernels' own gray and per-pixel term: 1 - SSIM in fp64, rounded once to fp32
+            exact = 1.0 - next(S.ssim_maps_like_kernel(S.gray01_like_kernel(hr[i]), S.gray01_like_kernel(sr[i]), [ws]))
+            ulp = np.spacing(np.abs(exact).astype(np.float32)).astype(np.float64)
+            worst = float((np.abs(m_ssim[i] - exact) / ulp).max())
+            assert worst <= 1.0, f"image {i}: 1-SSIM map off by {worst:.2f} fp32 ulp of the kernel-faithful oracle"
         assert np.abs(m_ssim[i] - want_ssim).max() <= 1e-5, f"image {i}: 1-SSIM map"
         assert np.abs(m_se[i] - want_se).max() <= (1e-7 if sigma == 0 else 1e-5), f"image {i}: SE map"
     assert not m_ssim[1].any() and not m_se[1].any(), "an identical pair must give all-zero maps"
     assert np.array_equal(m_max, np.stack([m_ssim.reshape(4, -1).max(1), m_se.reshape(4, -1).max(1)], 1).astype(np.float64))
 
 
-@pytest.mark.parametrize("h,w,c", [(128, 128, 3), (128, 128, 1), (64, 96, 3), (256, 256, 3)])
+@pytest.mark.parametrize("h,w,c", MAP_SHAPES)
 def test_map_means_equal_scorer_columns(h, w, c):
     """The unsmoothed 1 - SSIM map averages to 1 - the scorer's SSIM of that window size, the SE map to its MSE column."""
     sr, hr = _pairs(h, w, c, seed=3)

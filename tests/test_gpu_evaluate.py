@@ -11,7 +11,7 @@ from PIL import Image
 
 from oracle import drct_oracle as O
 from oracle import scoring_oracle as S
-from gpu_common import PKG
+from gpu_common import PKG, TableModel
 
 pytestmark = pytest.mark.gpu
 
@@ -141,19 +141,6 @@ def test_evaluate_cli_drn_l_matches_oracle(tmp_path, capsys):
     assert abs(res["auc_mse"] - a_mse) <= 1.5e-2 and abs(res["auc_psnr"] - a_psnr) <= 1.5e-2 and abs(res["auc_ssim"] - a_ssim) <= 1.5e-2
 
 
-class _TableModel:
-    """Stands in for the SR network: `run` returns precomputed uint8 SR images for the LR batch it is handed (the LR tensor's
-    first element carries the index of the batch's first image), so the evaluator's batching, scoring, gather and AUC logic can
-    be driven over a large image set without a forward pass."""
-
-    def __init__(self, sr_u8: torch.Tensor):
-        self.sr_u8 = sr_u8
-
-    def run(self, lr_d, want_float=False, want_u8=True):
-        i0 = int(lr_d[0, 0, 0, 0].item())
-        return None, self.sr_u8[i0:i0 + lr_d.shape[0]]
-
-
 @pytest.mark.timeout(900)
 def test_auc_over_1024_images_matches_oracle():
     """SURVEY.md 8d: >= 1024 images for the AUC check.  Synthetic good / bad uint8 pairs (SR = HR + reconstruction noise; bad
@@ -170,7 +157,7 @@ def test_auc_over_1024_images_matches_oracle():
         sr[i, y0:y0 + 24, x0:x0 + 24] += rng.integers(4, 40)
     sr = np.clip(sr, 0, 255).astype(np.uint8)
     wss = S.window_sizes_for(128)
-    ev = evaluate.BatchedEvaluator(_TableModel(torch.from_numpy(sr).cuda()), 255.0, wss)
+    ev = evaluate.BatchedEvaluator(TableModel(torch.from_numpy(sr).cuda()), 255.0, wss)
     ev.use_graph = False
     rows, ids = [], []
     for i0 in range(0, n, bs):
