@@ -84,6 +84,12 @@ def parse_args(argv=None):
     p.add_argument('--save-calibrated-masks', action='store_true', default=False,
                    help='write <output-dir>/calibrated/<split>/<stem>_{ssim,se[,gms]}.png: each map thresholded at its calibrated pixel '
                         'threshold (uint8 0 / 255); needs --calibration-dir')
+    p.add_argument('--defect-regions', action='store_true', default=False,
+                   help='report every 8-connected blob of each map above its calibrated pixel threshold as one defect in '
+                        '<output-dir>/defects.csv (box, area, centroid, peak score), with the region counts and the region image TPR / FPR '
+                        '(with --mask-dir also region recall, precision and false regions per image); needs --calibration-dir')
+    p.add_argument('--min-region-area', type=int, default=None, metavar='A',
+                   help='drop defect regions of fewer than A pixels (A >= 1, default 1); needs --defect-regions')
     if pre_args.config and os.path.isfile(pre_args.config):
         import yaml
 
@@ -102,6 +108,13 @@ def parse_args(argv=None):
         p.error(f'--calibration-quantile must be in (0, 1], got {args.calibration_quantile}')
     if args.save_calibrated_masks and args.calibration_dir is None:
         p.error('--save-calibrated-masks needs --calibration-dir (the defect-free images the threshold is calibrated on)')
+    if args.defect_regions and args.calibration_dir is None:
+        p.error('--defect-regions needs --calibration-dir (the defect-free images the pixel threshold is calibrated on)')
+    if args.min_region_area is not None:
+        if not args.defect_regions:
+            p.error('--min-region-area needs --defect-regions (it filters the defect regions)')
+        if args.min_region_area < 1:
+            p.error(f'--min-region-area must be >= 1, got {args.min_region_area}')
     return args
 
 
@@ -480,7 +493,8 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                      anomaly_maps: bool = False, map_window_size: int = 11, map_sigma: float = 4.0, mask_dir: Optional[str] = None,
                      save_maps: bool = False, au_pro: Optional[float] = None, pr_metrics: bool = False,
                      save_segmentation: bool = False, calibration_dir: Optional[str] = None, calibration_quantile: float = 0.999,
-                     save_calibrated_masks: bool = False, gms_map: bool = False):
+                     save_calibrated_masks: bool = False, gms_map: bool = False, defect_regions: bool = False,
+                     min_region_area: int = 1):
     """src/evaluate.py:138-267 with the loops batched.  Returns dict(best_ws, auc_ssim, auc_mse, auc_psnr, n, scores).
 
     anomaly_maps (implied by mask_dir / save_maps): per-pixel 1 - SSIM (window map_window_size) and squared-error maps, smoothed with
@@ -505,7 +519,16 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
 
     gms_map (implies anomaly_maps) adds a third map kind, the multi-scale gradient-magnitude-similarity map smoothed with map_sigma:
     everything above is also computed for it, with the suffix _gms in the result keys and file names and `MSGMS` on the printed lines
-    (after the SE entry of each kind)."""
+    (after the SE entry of each kind).
+
+    defect_regions (needs calibration_dir) reports every 8-connected blob of `map > t_px` with at least min_region_area pixels as one
+    defect (metrics.defect_regions, on the device, batch by batch): one row per region and map in <output_dir>/defects.csv (split, stem,
+    map, region, area, half-open box y0 x0 y1 x1, centroid_y, centroid_x, peak score and its first pixel peak_y peak_x; with mask_dir also
+    gt_pixels, the region's ground-truth pixels), and a `Map REG - ...` line after the `Map CAL` line with, per map, the regions on good
+    and on bad images and the TPR / FPR of the decision "an image is defective when it has a region" (region_count_{good,bad}_{kind},
+    region_image_{tpr,fpr}_{kind}).  With mask_dir it adds region recall (ground-truth regions, the 8-connected components of the masks,
+    that hold a pixel of a region, over all of them), region precision (regions holding a ground-truth pixel over all regions) and false
+    regions per test image (region_{recall,precision,false_per_image}_{kind})."""
     from .model import Model
 
     if au_pro is not None:
@@ -519,6 +542,10 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
         raise ValueError(f"calibration_quantile must be in (0, 1], got {calibration_quantile}")
     if save_calibrated_masks and calibration_dir is None:
         raise ValueError("save_calibrated_masks needs calibration_dir: the defect-free images the threshold is calibrated on")
+    if defect_regions and calibration_dir is None:
+        raise ValueError("defect_regions needs calibration_dir: the defect-free images the pixel threshold is calibrated on")
+    if int(min_region_area) < 1:
+        raise ValueError(f"min_region_area must be >= 1, got {min_region_area}")
     pr_metrics = pr_metrics or save_segmentation
     anomaly_maps = anomaly_maps or gms_map or mask_dir is not None or save_maps or calibration_dir is not None
     kinds = [('ssim', '1-SSIM'), ('se', 'SE')] + ([('gms', 'MSGMS')] if gms_map else [])   # (key / file suffix, printed label)
@@ -597,6 +624,9 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
         px_above = [above(t) for t in t_px]
         del cal                                              # the calibration maps are freed before the test pass
 
+    if defect_regions:                                       # per map and test image: regions, false regions, ground-truth regions, detected
+        reg_counts = np.zeros((n_maps, 4, len(entries)), dtype=np.int64)
+        reg_rows = []
     order: List[List[int]] = []
     loc = metrics.LocalisationAccumulator(n_maps) if mask_dir is not None else None   # every map of every image, kept on the device
     test_files = [(e[2], e[3]) for e in entries]
@@ -634,6 +664,33 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                         crop = (im_lr.size[1] * scale, im_lr.size[0] * scale)
                     batch_masks.append(load_mask(mask_paths[i], tuple(ev.last_maps[0].shape[1:]), crop))
                 loc.append(ev.last_maps[:-1], batch_masks)  # device copies, ordered before the next replay overwrites the maps
+            if defect_regions:
+                found = [metrics.defect_regions(ev.last_maps[j], px_above[j], min_region_area,
+                                                np.stack(batch_masks) if mask_dir is not None else None) for j in range(n_maps)]
+                for j, d in enumerate(found):
+                    idx = np.asarray(order[k])
+                    reg_counts[j, 0, idx] = d.n_regions
+                    if mask_dir is not None:
+                        false = d.regions['image'][d.regions['gt_pixels'] == 0]
+                        reg_counts[j, 1, idx] = np.bincount(false, minlength=len(idx))
+                        reg_counts[j, 2, idx], reg_counts[j, 3, idx] = d.gt_regions, d.gt_detected
+                for b, i in enumerate(order[k]):
+                    name = os.path.splitext(os.path.basename(entries[i][2]))[0]
+                    for (kind, _), d in zip(kinds, found):
+                        for r in d.regions[d.regions['image'] == b]:
+                            row = [entries[i][1], name, kind, int(r['label']), int(r['area']), int(r['y0']), int(r['x0']), int(r['y1']),
+                                   int(r['x1']), repr(int(r['sum_y']) / int(r['area'])), repr(int(r['sum_x']) / int(r['area'])),
+                                   repr(float(r['peak'])), int(r['peak_y']), int(r['peak_x'])]
+                            reg_rows.append(row + ([int(r['gt_pixels'])] if mask_dir is not None else []))
+    if defect_regions:
+        import csv
+
+        Path(output_dir).mkdir(parents=True, exist_ok=True)
+        with open(Path(output_dir) / 'defects.csv', 'w', newline='') as f:
+            out = csv.writer(f)
+            out.writerow(['split', 'stem', 'map', 'region', 'area', 'y0', 'x0', 'y1', 'x1', 'centroid_y', 'centroid_x', 'peak', 'peak_y',
+                          'peak_x'] + (['gt_pixels'] if mask_dir is not None else []))
+            out.writerows(reg_rows)
     n_cols = len(ev.window_sizes) + 2
     local = torch.cat(rows) if rows else torch.empty(0, n_cols + (n_maps if anomaly_maps else 0), dtype=torch.float64, device='cuda')
     table = gather_scores(local, torch.tensor(ids, dtype=torch.int64, device='cuda'), len(entries))
@@ -664,6 +721,26 @@ def evaluate_on_test(opt, checkpoint_model_path, output_dir: str, save_images: b
                              f"IoU {m.iou:.4f}, PRO {m.pro:.4f}")
                 parts.append(part)
             print(f"Map CAL - q={float(calibration_quantile):g} on {len(cal_files)} defect-free images: " + "; ".join(parts))
+            if defect_regions:
+                parts = []
+                for j, (kind, label) in enumerate(kinds):
+                    n_reg, n_false, n_gt, n_det = (reg_counts[j, c] for c in range(4))
+                    flagged = n_reg > 0                       # with min_region_area 1: map_max > t_px
+                    tpr, fpr = float(flagged[y == 1].mean()), float(flagged[y == 0].mean())
+                    good, bad = int(n_reg[y == 0].sum()), int(n_reg[y == 1].sum())
+                    res.update({f'region_count_good_{kind}': good, f'region_count_bad_{kind}': bad, f'region_image_tpr_{kind}': tpr,
+                                f'region_image_fpr_{kind}': fpr})
+                    part = f"{label} regions good {good}, bad {bad}, image TPR {tpr:.4f}, FPR {fpr:.4f}"
+                    if mask_dir is not None:
+                        n_pred, n_f, n_g = good + bad, int(n_false.sum()), int(n_gt.sum())
+                        recall = int(n_det.sum()) / n_g if n_g else float('nan')
+                        precision = (n_pred - n_f) / n_pred if n_pred else float('nan')
+                        per_image = n_f / len(entries)
+                        res.update({f'region_recall_{kind}': recall, f'region_precision_{kind}': precision,
+                                    f'region_false_per_image_{kind}': per_image})
+                        part += f", region recall {recall:.4f}, precision {precision:.4f}, false regions per image {per_image:.4f}"
+                    parts.append(part)
+                print(f"Map REG - min area {int(min_region_area)}: " + "; ".join(parts))
         if mask_dir is not None:
             limit = 0.3 if au_pro is None else float(au_pro)
             loc_res = loc.results(limit)                      # one LocalisationMetrics per map kind
@@ -732,7 +809,8 @@ def main(argv=None):
                             save_maps=args.save_maps, au_pro=args.au_pro, pr_metrics=args.pr_metrics,
                             save_segmentation=args.save_segmentation, calibration_dir=args.calibration_dir,
                             calibration_quantile=args.calibration_quantile, save_calibrated_masks=args.save_calibrated_masks,
-                            gms_map=args.gms_map)
+                            gms_map=args.gms_map, defect_regions=args.defect_regions,
+                            min_region_area=1 if args.min_region_area is None else args.min_region_area)
 
 
 if __name__ == "__main__":

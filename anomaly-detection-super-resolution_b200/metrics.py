@@ -347,6 +347,94 @@ class LocalisationAccumulator:
                                 ratio(2 * tp, 2 * tp + fp + fn), ratio(tp, tp + fp + fn), r[4])
 
 
+REGION_COLUMNS = ("image", "label", "area", "y0", "x0", "y1", "x1", "sum_y", "sum_x", "peak", "peak_y", "peak_x")
+
+
+def region_dtype(with_gt: bool) -> np.dtype:
+    """Row type of DefectRegions.regions: int64 columns, peak float32, gt_pixels only with ground truth."""
+    cols = REGION_COLUMNS + (("gt_pixels",) if with_gt else ())
+    return np.dtype([(c, np.float32 if c == "peak" else np.int64) for c in cols])
+
+
+class DefectRegions(NamedTuple):
+    """The defects of a batch of anomaly maps (defect_regions).  regions has one row per region, sorted by (image, label): area,
+    the half-open box y0 <= y < y1, x0 <= x < x1 (scipy.ndimage.find_objects), the integer sums of y and x (centroid = sum / area),
+    the largest fp32 score and the first raster pixel that attains it, and with masks the region's ground-truth pixels."""
+    labels: torch.Tensor                  # CUDA int32 [B, H, W]: 0 = background, 1..n_regions[b] = the regions of image b
+    regions: np.ndarray                   # host table, dtype region_dtype(masks given)
+    n_regions: np.ndarray                 # int64 [B] regions per image
+    gt_regions: Optional[np.ndarray]      # int64 [B] ground-truth regions (8-connected components of the mask) per image, with masks
+    gt_detected: Optional[np.ndarray]     # int64 [B] of those, the ones holding a pixel of a region, with masks
+
+
+def _region_counts(counts: torch.Tensor, workspace: torch.Tensor, what: str) -> np.ndarray:
+    host = torch.cat([counts, workspace[:4].view(torch.int32)]).cpu().numpy().astype(np.int64)
+    if host[-1]:
+        raise RuntimeError(f"{what}: {int(host[-1])} union-find loops or labels out of range on the device")
+    return host[:-1]
+
+
+def defect_regions(maps: torch.Tensor, threshold: float, min_area: int = 1, masks=None) -> DefectRegions:
+    """Every 8-connected blob of `maps >= threshold` as one defect: maps = CUDA fp32 [B, H, W], compared with the exact double
+    threshold like LocalisationAccumulator.segmentation (a NaN score is never foreground; pass evaluate.above(t) for the strict
+    `map > t`).  Blobs of fewer than min_area pixels are dropped, the rest numbered 1..n per image in raster order of their first pixel
+    (scipy.ndimage.label of the kept foreground with structure ones((3, 3))).  masks (bool / uint8 [B, H, W], host or device, non-zero
+    = defect) add gt_pixels per region and the ground-truth regions and detections per image.  Labels and statistics are computed on
+    the device with integer atomics (csrc/regions.cu): the same bits on every run and for an image whatever batch it is in."""
+    ops._cuda(maps, "maps")
+    if maps.dtype != torch.float32 or maps.dim() != 3:
+        raise ValueError(f"defect_regions: maps must be a float32 [B, H, W] tensor, got {maps.dtype} {tuple(maps.shape)}")
+    threshold = float(threshold)
+    if threshold != threshold:
+        raise ValueError("defect_regions: the threshold is NaN")
+    if int(min_area) != min_area or int(min_area) < 1:
+        raise ValueError(f"defect_regions: min_area must be an integer >= 1, got {min_area}")
+    maps = maps.contiguous()
+    b, h, w = maps.shape
+    dev = maps.device
+    ws = torch.empty(ops.regions_workspace_bytes(b, h, w), dtype=torch.uint8, device=dev)
+    labels = torch.empty(b, h, w, dtype=torch.int32, device=dev)
+    counts = torch.empty(b, dtype=torch.int32, device=dev)
+    ops.label_regions(maps, float(fp32_at_least(threshold)), None, int(min_area), ws, labels, counts)
+    n_regions = _region_counts(counts, ws, "label_regions")
+    gt_labels = gt_off = gt_hit = gt_regions = None
+    if masks is not None:
+        m = masks if isinstance(masks, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(np.asarray(masks)))
+        if tuple(m.shape) != (b, h, w):
+            raise ValueError(f"defect_regions: masks {tuple(m.shape)} for maps {(b, h, w)}")
+        m = (m.to(dev) != 0).to(torch.uint8).contiguous()
+        gt_ws = torch.empty_like(ws)
+        gt_labels = torch.empty_like(labels)
+        gt_counts = torch.empty_like(counts)
+        ops.label_regions(None, 0.0, m, 1, gt_ws, gt_labels, gt_counts)
+        gt_regions = _region_counts(gt_counts, gt_ws, "label_regions (masks)")
+        gt_off = torch.from_numpy(np.concatenate([[0], np.cumsum(gt_regions)]).astype(np.int64)).to(dev)
+        gt_hit = torch.empty(int(gt_regions.sum()), dtype=torch.int32, device=dev)
+    offsets = np.concatenate([[0], np.cumsum(n_regions)]).astype(np.int64)
+    n_rows = int(offsets[-1])
+    table = torch.empty(n_rows, 9, dtype=torch.int64, device=dev)
+    ops.region_stats(labels, maps, gt_labels, torch.from_numpy(offsets).to(dev), gt_off, ws, table, gt_hit)
+    tab = table.cpu().numpy()
+    _region_counts(counts[:0], ws, "region_stats")            # no counts: only the error counter (labels out of range)
+    out = np.zeros(n_rows, dtype=region_dtype(masks is not None))
+    out["image"] = np.repeat(np.arange(b), n_regions)
+    out["label"] = np.arange(n_rows) - np.repeat(offsets[:-1], n_regions) + 1
+    for name, col in (("area", 0), ("y0", 1), ("x0", 2), ("sum_y", 5), ("sum_x", 6)):
+        out[name] = tab[:, col]
+    out["y1"], out["x1"] = tab[:, 3] + 1, tab[:, 4] + 1
+    key = tab[:, 7].view(np.uint64)
+    k = (key >> np.uint64(32)).astype(np.uint32)             # order-preserving key: sign bit set for scores >= 0, all bits flipped below
+    out["peak"] = np.where(k & np.uint32(0x80000000), k & np.uint32(0x7fffffff), ~k).astype(np.uint32).view(np.float32)
+    idx = (~(key & np.uint64(0xffffffff))).astype(np.uint32).astype(np.int64)   # the low word holds ~(y W + x)
+    out["peak_y"], out["peak_x"] = idx // w, idx % w
+    gt_detected = None
+    if masks is not None:
+        out["gt_pixels"] = tab[:, 8]
+        hit = gt_hit.cpu().numpy().astype(np.int64)
+        gt_detected = np.bincount(np.repeat(np.arange(b), gt_regions), weights=hit, minlength=b).astype(np.int64)
+    return DefectRegions(labels, out, n_regions, gt_regions, gt_detected)
+
+
 def _on_device(maps) -> bool:
     if isinstance(maps, torch.Tensor):
         return maps.is_cuda

@@ -462,6 +462,83 @@ def threshold_metrics(scores: torch.Tensor, regions: torch.Tensor, region_sizes:
     return out
 
 
+def regions_workspace_bytes(b: int, h: int, w: int) -> int:
+    """Bytes of scratch adsr_label_regions / adsr_region_stats need for B images of H x W (error counter, parent and area per pixel,
+    per-chunk counts)."""
+    n = int(lib().adsr_regions_workspace_bytes(int(b), int(h), int(w)))
+    if n < 0:
+        raise ValueError(f"label_regions: unsupported batch shape {b} x {h} x {w}")
+    return n
+
+
+def _bhw(t: torch.Tensor, name: str, dt) -> tuple:
+    _check_tensors("label_regions", (t, name, dt))
+    if t.dim() != 3:
+        raise ValueError(f"label_regions: {name} must be [B, H, W], got shape {tuple(t.shape)}")
+    return tuple(t.shape)
+
+
+def label_regions(scores: Optional[torch.Tensor], threshold: float, mask: Optional[torch.Tensor], min_area: int,
+                  workspace: torch.Tensor, labels: torch.Tensor, counts: torch.Tensor) -> torch.Tensor:
+    """8-connected components of `scores >= threshold` (fp32 [B, H, W], threshold an fp32 value, not NaN) or of `mask != 0` (uint8
+    [B, H, W]) -- exactly one of the two -- image by image, components of fewer than min_area pixels dropped, the rest numbered 1..n in
+    raster order of their first pixel: labels int32 [B, H, W], counts int32 [B].  workspace: uint8 [>= regions_workspace_bytes(B, H, W)];
+    workspace[:4] as int32 is the error counter (non-zero: the labels are invalid).  Seven kernels, no synchronisation."""
+    if (scores is None) == (mask is None):
+        raise ValueError("label_regions takes exactly one of scores and mask")
+    shape = _bhw(scores, "scores", torch.float32) if scores is not None else _bhw(mask, "mask", torch.uint8)
+    b, h, w = shape
+    if tuple(labels.shape) != shape or counts.numel() != b:
+        raise ValueError(f"label_regions: labels {tuple(labels.shape)} / counts {tuple(counts.shape)} for a {shape} batch")
+    _check_tensors("label_regions", (labels, "labels", torch.int32), (counts, "counts", torch.int32), (workspace, "workspace", torch.uint8))
+    if int(min_area) < 1:
+        raise ValueError(f"label_regions: min_area must be >= 1, got {min_area}")
+    _t = _begin()
+    check(lib().adsr_label_regions(ptr(scores), float(threshold), ptr(mask), b, h, w, int(min_area), ptr(labels), ptr(counts),
+                                   ptr(workspace), workspace.numel(), stream_ptr()), "adsr_label_regions")
+    global LAUNCHES
+    LAUNCHES += 6                                      # tile labels, borders, compress, count, scan, assign; _count adds the relabel
+    _count("label_regions", 0.0, _t)
+    return labels
+
+
+REGION_FIELDS = ("area", "ymin", "xmin", "ymax", "xmax", "sum_y", "sum_x", "peak_key", "gt_pixels")
+
+
+def region_stats(labels: torch.Tensor, scores: Optional[torch.Tensor], gt_labels: Optional[torch.Tensor], row_offsets: torch.Tensor,
+                 gt_offsets: Optional[torch.Tensor], workspace: torch.Tensor, table: torch.Tensor,
+                 gt_hit: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Per-region statistics of label_regions output: table int64 [R, 9] with the columns REGION_FIELDS, region l of image b in row
+    row_offsets[b] + l - 1 (row_offsets: int64 [B + 1] on the device, R = row_offsets[B]).  scores (fp32 [B, H, W], nullable) give the
+    peak key; gt_labels (int32 [B, H, W], the label_regions of the ground-truth mask, nullable) with gt_offsets give the ground-truth
+    pixels per region and gt_hit int32 [n_gt] = 1 for each ground-truth region a region touches.  workspace[:4] as int32 counts labels
+    out of range.  Two kernels, no synchronisation."""
+    b, h, w = _bhw(labels, "labels", torch.int32)
+    specs = [(row_offsets, "row_offsets", torch.int64), (workspace, "workspace", torch.uint8), (table, "table", torch.int64)]
+    if scores is not None:
+        specs.append((scores, "scores", torch.float32))
+    if gt_labels is not None:
+        if gt_offsets is None or gt_hit is None:
+            raise ValueError("region_stats: gt_labels need gt_offsets and gt_hit")
+        specs += [(gt_labels, "gt_labels", torch.int32), (gt_offsets, "gt_offsets", torch.int64), (gt_hit, "gt_hit", torch.int32)]
+    _check_tensors("region_stats", *specs)
+    for t, name in ((scores, "scores"), (gt_labels, "gt_labels")):
+        if t is not None and tuple(t.shape) != (b, h, w):
+            raise ValueError(f"region_stats: {name} {tuple(t.shape)} for labels {(b, h, w)}")
+    if row_offsets.numel() != b + 1 or (gt_offsets is not None and gt_offsets.numel() != b + 1) or table.dim() != 2 or table.shape[1] != 9:
+        raise ValueError("region_stats: offsets must hold B + 1 values and the table 9 columns")
+    n_gt = 0 if gt_labels is None else gt_hit.numel()
+    _t = _begin()
+    check(lib().adsr_region_stats(ptr(labels), ptr(scores), ptr(gt_labels), b, h, w, ptr(row_offsets), table.shape[0],
+                                  ptr(gt_offsets) if gt_labels is not None else 0, n_gt, ptr(table),
+                                  ptr(gt_hit) if gt_labels is not None else 0, ptr(workspace), workspace.numel(), stream_ptr()),
+          "adsr_region_stats")
+    global LAUNCHES
+    LAUNCHES += 1                                      # table initialisation; _count adds the statistics pass
+    _count("region_stats", 0.0, _t)
+    return table
+
+
 def score_images_strided(sr: torch.Tensor, hr: torch.Tensor, layout: str, window_sizes: Sequence[int], *, div: float = 1.0,
                          clamp01: bool = False, zero_pad: bool = False, c1: float = 1e-4, c2: float = 9e-4,
                          psnr_peak: float = 1.0) -> torch.Tensor:

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 19
+#define ADSR_ABI_VERSION 20
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -325,6 +325,33 @@ int adsr_localisation_metrics(const float* scores, const int32_t* regions, int64
 int adsr_score_quantile(const float* scores, int64_t n, int64_t k, void* workspace, int64_t workspace_bytes, double* out, void* stream);
 int adsr_threshold_metrics(const float* scores, const int32_t* regions, int64_t n, const int64_t* region_sizes, int n_regions,
                            float threshold, void* workspace, int64_t workspace_bytes, double* out, void* stream);
+
+/* Defect regions of a [B, H, W] batch, image by image: the 8-connected components of the foreground (scipy.ndimage.label with
+ * structure = ones((3, 3))), components of fewer than min_area >= 1 pixels dropped, the kept ones numbered 1..n in raster order of their
+ * first pixel (0 = background).  Exact and deterministic: the same labels whatever the scheduling, and image i does not depend on the
+ * rest of the batch.
+ * adsr_label_regions: foreground = scores >= threshold (fp32 scores, threshold not NaN; a NaN score is never foreground) or mask != 0
+ *   (uint8): exactly one of scores / mask is given.  labels: int32 [B, H, W]; counts: int32 [B] regions kept per image.
+ *   workspace: adsr_regions_workspace_bytes(B, H, W) bytes, 16-byte aligned; its first 4 bytes (uint32) count union / find loops that
+ *   hit their iteration cap (the pixel count of a tile or an image; each pass strictly lowers a root index, so 0 unless memory was
+ *   corrupted): the labels are only valid when it reads 0.  Nine launches (two memsets, seven kernels).
+ * adsr_region_stats: one pass over labels (as adsr_label_regions left them) with integer atomics.  row_offsets: int64 [B + 1] device,
+ *   region l of image b is table row row_offsets[b] + l - 1 (row_offsets[B] = n_rows); table: int64 [n_rows, 9] =
+ *   {area, y min, x min, y max, x max, sum of y, sum of x, peak key, ground-truth pixels}, the peak key = (k << 32) | ~(y W + x) as an
+ *   unsigned 64-bit value with k the order-preserving key of the fp32 score (-0.0 as +0.0; sign bit set for scores >= 0, all bits
+ *   flipped for negative ones): the highest score wins, a tie goes to the first raster pixel.  scores NULL: peak keys stay 0.
+ *   gt_labels (nullable): int32 [B, H, W] ground-truth regions (adsr_label_regions of the mask, min_area 1) with gt_offsets int64 [B + 1]
+ *   as row_offsets; field 8 counts the region's pixels with gt_labels > 0 and gt_hit: int32 [n_gt] is 1 for every ground-truth region
+ *   that holds a pixel of a region, else 0.  The workspace (that of adsr_label_regions) receives the number of labels out of range in
+ *   its first 4 bytes.  Two kernels.
+ * ADSR_ERR_BAD_SHAPE: B, H or W < 1, H W >= 2^31, min_area < 1, a NaN threshold, neither or both of scores / mask, n_rows or n_gt < 0, a
+ *   NULL output or a short workspace.  adsr_regions_workspace_bytes: -1 for unsupported sizes. */
+int64_t adsr_regions_workspace_bytes(int B, int H, int W);
+int adsr_label_regions(const float* scores, float threshold, const uint8_t* mask, int B, int H, int W, int min_area, int32_t* labels,
+                       int32_t* counts, void* workspace, int64_t workspace_bytes, void* stream);
+int adsr_region_stats(const int32_t* labels, const float* scores, const int32_t* gt_labels, int B, int H, int W,
+                      const int64_t* row_offsets, int64_t n_rows, const int64_t* gt_offsets, int64_t n_gt, int64_t* table,
+                      int32_t* gt_hit, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* Validation metrics of the reference's training loop, `Trainer.test` (src/trainer.py:242-304), for a batch of fp32 image
  * pairs: the SR value is first quantised with ROUNDING (`quantize`, src/trainer.py:45-47: round(clamp(x * 255 / rgb_range, 0,
