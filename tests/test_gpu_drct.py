@@ -12,6 +12,16 @@ from gpu_common import DrctOpt, mod
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 TOL = 2e-2          # max |dSR| / rgb_range, bf16 storage + fp32 accumulate (north star; SURVEY.md section 8d)
+# Per case: about twice the max |dSR| / rgb_range measured on a B200 at a 1000 W power limit (DESIGN.md section 2), so that a kernel change that
+# doubles the end-to-end error fails here even while it stays inside the north-star TOL.
+BOUND = {"small_golden": 1e-3, "l_rgb_golden": 1.5e-3, "l_batch1": 1.2e-3, "l_batch5": 1.2e-3, "rect_gray": 1.2e-3, "l_64px": 1.5e-3,
+         "rgb_range_1": 3e-3, "odd_windows": 1e-3, "odd_windows_pair": 1e-3}
+U8_MAX_DIFF, U8_EQUAL_SHARE = 1, 0.97          # measured: 1 and 0.985
+
+
+def _within(case, err):
+    print(f"[drct] {case}: max|dSR|/rgb_range = {err:.3e} (bound {BOUND[case]:.1e})")
+    assert err < BOUND[case], f"{case}: max|dSR|/rgb_range = {err}"
 
 
 def _model(cfg: O.DrctCfg, sd):
@@ -33,8 +43,7 @@ def test_drct_small_golden(golden_dir):
     m = _model(cfg, sd)
     x = torch.from_numpy(g["x"]).to(DEV)
     sr = m(x).cpu().numpy()
-    err = np.abs(sr - g["sr"]).max() / 255.0
-    assert err < TOL, f"max|dSR|/rgb_range = {err}"
+    _within("small_golden", float(np.abs(sr - g["sr"]).max() / 255.0))
 
 
 def test_drct_l_rgb_golden(golden_dir):
@@ -43,10 +52,14 @@ def test_drct_l_rgb_golden(golden_dir):
     sd = O.make_state_dict(cfg, seed=1)
     m = _model(cfg, sd)
     sr, u8 = m.run(torch.from_numpy(g["x"]).to(DEV), want_float=True, want_u8=True)
-    err = np.abs(sr.cpu().numpy() - g["sr"]).max() / 255.0
-    assert err < TOL, f"max|dSR|/rgb_range = {err}"
+    _within("l_rgb_golden", float(np.abs(sr.cpu().numpy() - g["sr"]).max() / 255.0))
     from oracle import scoring_oracle as S
-    assert np.array_equal(u8.cpu().numpy(), S.quantize_u8(sr.cpu().numpy(), 255.0))
+    u8 = u8.cpu().numpy()
+    assert np.array_equal(u8, S.quantize_u8(sr.cpu().numpy(), 255.0))
+    # the scored image against the reference's own truncation: off by at most one grey level, and equal almost everywhere
+    d = np.abs(u8.astype(np.int32) - S.quantize_u8(g["sr"], 255.0).astype(np.int32))
+    print(f"[drct] l_rgb_golden u8: max diff {d.max()}, equal {float((d == 0).mean()):.5f}")
+    assert d.max() <= U8_MAX_DIFF and float((d == 0).mean()) >= U8_EQUAL_SHARE
 
 
 @pytest.mark.parametrize("B", [1, 5])
@@ -59,8 +72,7 @@ def test_drct_l_vs_oracle_batch(B):
     with torch.no_grad():
         want = O.drct_forward(sd, x, cfg)
     got = m(x.to(DEV)).cpu()
-    err = float((got - want).abs().max()) / 255.0
-    assert err < TOL, f"max|dSR|/rgb_range = {err}"
+    _within(f"l_batch{B}", float((got - want).abs().max()) / 255.0)
     # batch independence: image i of a batch equals the same image run alone (units are independent)
     if B > 1:
         solo = m(x[2:3].to(DEV)).cpu()
@@ -75,7 +87,7 @@ def test_drct_rectangular_input_and_gray():
     with torch.no_grad():
         want = O.drct_forward(sd, x, cfg)
     got = m(x.to(DEV)).cpu()
-    assert float((got - want).abs().max()) / 255.0 < TOL
+    _within("rect_gray", float((got - want).abs().max()) / 255.0)
 
 
 @pytest.mark.timeout(600)
@@ -89,8 +101,7 @@ def test_drct_l_64px_lr_vs_oracle():
         want = O.drct_forward(sd, x, cfg)
     got = m(x.to(DEV)).cpu()
     assert got.shape == (2, 3, 256, 256)
-    err = float((got - want).abs().max()) / 255.0
-    assert err < TOL, f"max|dSR|/rgb_range = {err}"
+    _within("l_64px", float((got - want).abs().max()) / 255.0)
 
 
 def test_drct_rgb_range_1_full_model():
@@ -108,8 +119,7 @@ def test_drct_rgb_range_1_full_model():
     with torch.no_grad():
         want = O.drct_forward(sd, x, cfg)
     sr, u8 = m.run(x.to(DEV), want_float=True, want_u8=True)
-    err = float((sr.cpu() - want).abs().max()) / 1.0
-    assert err < TOL, f"max|dSR|/rgb_range = {err}"
+    _within("rgb_range_1", float((sr.cpu() - want).abs().max()) / 1.0)
     assert np.array_equal(u8.cpu().numpy(), S.quantize_u8(sr.cpu().numpy(), 1.0))
 
 
@@ -130,7 +140,7 @@ def test_drct_odd_window_count_falls_back_inside_forward():
     finally:
         ops.PROFILE = None
     assert "swin_attn" not in kinds and kinds.count("window_attention") == 5
-    assert float((got - want).abs().max()) / 255.0 < TOL
+    _within("odd_windows", float((got - want).abs().max()) / 255.0)
     x2 = torch.cat([x, x.flip(-1)])                        # two images: 18 windows, the fused kernel runs again
     ops.PROFILE = []
     try:
@@ -139,4 +149,4 @@ def test_drct_odd_window_count_falls_back_inside_forward():
     finally:
         ops.PROFILE = None
     assert kinds2.count("swin_attn") == 5
-    assert float((got2[0] - want[0]).abs().max()) / 255.0 < TOL
+    _within("odd_windows_pair", float((got2[0] - want[0]).abs().max()) / 255.0)
