@@ -13,7 +13,7 @@ from ctypes import c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_void_
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # ADSR_LIB: developer override for A/B timing of two builds in one session (tools/build_variant.sh); never a fallback
 LIB_PATH = os.environ.get("ADSR_LIB") or os.path.join(_HERE, "libadsr_b200.so")
-ABI_VERSION = 20
+ABI_VERSION = 21
 
 ACT_NONE, ACT_LRELU, ACT_GELU, ACT_RELU = 0, 1, 2, 3
 OUT_ROWS, OUT_PIXEL_SHUFFLE2 = 0, 1
@@ -92,9 +92,9 @@ _SIGNATURES = {
     "adsr_bicubic_affine": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "adsr_conv3x3_small": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_int64,
                                    c_void_p, c_int64, c_int, c_void_p]),
-    "adsr_channel_mean": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_void_p, c_void_p]),
-    "adsr_rcab_ca_scale": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
-                                   c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "adsr_channel_mean": (c_int, [c_void_p, c_int64, c_int, c_int, c_int, c_int, c_void_p, c_int64, c_void_p]),
+    "adsr_rcab_ca_scale": (c_int, [c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int, c_int, c_int,
+                                   c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -107,45 +107,11 @@ __global__ void __launch_bounds__(128) conv3x3_small_kernel(const float* __restr
     for (int c0 = C; c0 < npad1; c0 += 4) *reinterpret_cast<uint2*>(out1 + pix * ld1 + c0) = make_uint2(0, 0);
 }
 
-// mean over the HW pixels of each image, per channel: x [B, HW, ld] bf16 -> mean [B, C] fp32 (AdaptiveAvgPool2d(1)).
-// grid = (slices, B): each CTA reduces a slice of pixels and atomically adds its partial mean.
-__global__ void __launch_bounds__(256) channel_mean_kernel(const __nv_bfloat16* __restrict__ x, long long ld, int HW, int C,
-                                                            float* __restrict__ mean) {
-    __shared__ float red[8][128];
-    const int b = blockIdx.y;
-    const int cpairs = C / 2;
-    const int lanes_per_pix = cpairs;                      // one thread per channel pair
-    const int pix_per_iter = blockDim.x / lanes_per_pix;
-    const int cp = threadIdx.x % lanes_per_pix, pslot = threadIdx.x / lanes_per_pix;
-    const int per_slice = (HW + gridDim.x - 1) / gridDim.x;
-    const int p0 = blockIdx.x * per_slice, p1 = min(HW, p0 + per_slice);
-    float s0 = 0.f, s1 = 0.f;
-    if (pslot < pix_per_iter)
-        for (int p = p0 + pslot; p < p1; p += pix_per_iter) {
-            const uint32_t v = __ldg(reinterpret_cast<const uint32_t*>(x + (static_cast<long long>(b) * HW + p) * ld + 2 * cp));
-            s0 += bf16_lo(v);
-            s1 += bf16_hi(v);
-        }
-    // reduce over pixel slots through shared memory (C <= 128 channels, <= 8 slots kept)
-    const int nslots = min(pix_per_iter, 8);
-    if (pslot < 8) { red[pslot][2 * cp] = 0.f; red[pslot][2 * cp + 1] = 0.f; }
-    __syncthreads();
-    if (pslot < pix_per_iter) {
-        atomicAdd(&red[pslot % nslots][2 * cp], s0);
-        atomicAdd(&red[pslot % nslots][2 * cp + 1], s1);
-    }
-    __syncthreads();
-    if (threadIdx.x < C) {
-        float t = 0.f;
-        for (int s = 0; s < nslots; ++s) t += red[s][threadIdx.x];
-        atomicAdd(mean + static_cast<long long>(b) * C + threadIdx.x, t / static_cast<float>(HW));
-    }
-}
-
-// Same reduction with 16-byte loads (C % 8 == 0, 16-byte aligned rows): thread = (pixel slot, 8-channel group), four pixels in
-// flight per thread; the slots meet in shared memory.
-__global__ void __launch_bounds__(256) channel_mean8_kernel(const __nv_bfloat16* __restrict__ x, long long ld, int HW, int C,
-                                                             float* __restrict__ mean) {
+// Column sums of slice s of image b's HW pixels: x [B, HW, ld] bf16 -> part[(b * slices + s) * ld_part + c] fp32, the partial-row
+// layout channel_mean_parts_kernel reduces in a fixed order (CALayer's AdaptiveAvgPool2d(1) where the halo conv does not run).
+// grid = (slices, B), 16-byte loads (C % 8 == 0): thread = (pixel slot, 8-channel group), the slots meet in shared memory in order.
+__global__ void __launch_bounds__(256) channel_sum8_kernel(const __nv_bfloat16* __restrict__ x, long long ld, int HW, int C,
+                                                            float* __restrict__ part, int ld_part) {
     __shared__ float red[256 * 8];
     const int b = blockIdx.y;
     const int groups = C >> 3;
@@ -169,7 +135,7 @@ __global__ void __launch_bounds__(256) channel_mean8_kernel(const __nv_bfloat16*
     if (threadIdx.x < C) {
         float t = 0.f;
         for (int sl = 0; sl < ppi; ++sl) t += red[sl * C + threadIdx.x];
-        atomicAdd(mean + static_cast<long long>(b) * C + threadIdx.x, t / static_cast<float>(HW));
+        part[(static_cast<long long>(b) * gridDim.x + blockIdx.x) * ld_part + threadIdx.x] = t;
     }
 }
 
@@ -242,31 +208,16 @@ __global__ void __launch_bounds__(1024) channel_mean_parts_kernel(const float* _
     }
 }
 
-// out = res * sigmoid(W2 relu(W1 mean_b + b1) + b2) + x       (CALayer + RCAB residual, src/drn.py:123-158)
+// out = res * scale[b] + x       (CALayer + RCAB residual, src/drn.py:123-158; the scales from channel_mean_parts with the MLP)
 __global__ void __launch_bounds__(256) rcab_ca_scale_kernel(const __nv_bfloat16* __restrict__ res, long long ldr,
                                                              const __nv_bfloat16* __restrict__ x, long long ldx,
                                                              __nv_bfloat16* __restrict__ out, long long ldo,
-                                                             const float* __restrict__ mean, const float* __restrict__ w1,
-                                                             const float* __restrict__ b1, const float* __restrict__ w2,
-                                                             const float* __restrict__ b2, int HW, int C, int Cr) {
-    __shared__ float hid[16];
+                                                             const float* __restrict__ scale, int HW, int C) {
     __shared__ float sc[128];
     const int b = blockIdx.y;
     pdl_launch_dependents();
-    pdl_wait();                                             // mean / res / x come from the previous kernels
-    if (Cr == 0) {                                          // `mean` already holds the scales (channel_mean_parts with the MLP)
-        if (threadIdx.x < C) sc[threadIdx.x] = mean[static_cast<long long>(b) * C + threadIdx.x];
-    } else if (threadIdx.x < Cr) {
-        float a = b1[threadIdx.x];
-        for (int c = 0; c < C; ++c) a = fmaf(w1[threadIdx.x * C + c], mean[static_cast<long long>(b) * C + c], a);
-        hid[threadIdx.x] = fmaxf(a, 0.f);
-    }
-    __syncthreads();
-    if (Cr > 0 && threadIdx.x < C) {
-        float a = b2[threadIdx.x];
-        for (int j = 0; j < Cr; ++j) a = fmaf(w2[threadIdx.x * Cr + j], hid[j], a);
-        sc[threadIdx.x] = 1.f / (1.f + __expf(-a));
-    }
+    pdl_wait();                                             // scale / res / x come from the previous kernels
+    if (threadIdx.x < C) sc[threadIdx.x] = scale[static_cast<long long>(b) * C + threadIdx.x];
     __syncthreads();
     const uint32_t vec = static_cast<uint32_t>(C) / 8u;               // 16-byte vectors per pixel
     const uint32_t n = static_cast<uint32_t>(HW) * vec;                 // per image: < 2^31 (checked by the wrapper)
@@ -333,17 +284,13 @@ extern "C" int adsr_conv3x3_small(const float* x_nchw, int B, int nc, int H, int
     return check_launch();
 }
 
-extern "C" int adsr_channel_mean(const void* x, int64_t ld, int B, int HW, int C, float* mean, void* stream) {
+extern "C" int adsr_channel_mean(const void* x, int64_t ld, int B, int HW, int C, int slices, float* part, int64_t ld_part,
+                                 void* stream) {
     if (B <= 0) return ADSR_OK;
-    if (C < 2 || C > 128 || (C % 2) || (ld % 2)) return ADSR_ERR_BAD_SHAPE;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (cudaMemsetAsync(mean, 0, static_cast<size_t>(B) * C * sizeof(float), st) != cudaSuccess) return ADSR_ERR_CUDA;
-    const int slices = std::max(1, std::min(32, HW / 256));
-    if ((C % 8) == 0 && (ld % 8) == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0) {
-        channel_mean8_kernel<<<dim3(slices, B), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), ld, HW, C, mean);
-        return check_launch();
-    }
-    channel_mean_kernel<<<dim3(slices, B), 256, 0, st>>>(static_cast<const __nv_bfloat16*>(x), ld, HW, C, mean);
+    if (C < 8 || C > 128 || (C % 8) || (ld % 8) || (reinterpret_cast<uintptr_t>(x) & 15) || slices < 1 || slices > HW || ld_part < C)
+        return ADSR_ERR_BAD_SHAPE;
+    channel_sum8_kernel<<<dim3(slices, B), 256, 0, static_cast<cudaStream_t>(stream)>>>(static_cast<const __nv_bfloat16*>(x), ld, HW,
+                                                                                         C, part, static_cast<int>(ld_part));
     return check_launch();
 }
 
@@ -357,14 +304,13 @@ extern "C" int adsr_channel_mean_parts(const float* chan_part, int B, int parts,
 }
 
 extern "C" int adsr_rcab_ca_scale(const void* res, int64_t ldr, const void* x, int64_t ldx, void* out, int64_t ldo,
-                                  const float* mean, const float* w1, const float* b1, const float* w2, const float* b2,
-                                  int B, int HW, int C, int Cr, void* stream) {
+                                  const float* scale, int B, int HW, int C, void* stream) {
     if (B <= 0) return ADSR_OK;
-    if (C < 8 || C > 128 || (C % 8) || Cr < 0 || Cr > 16 || (ldr % 8) || (ldx % 8) || (ldo % 8)) return ADSR_ERR_BAD_SHAPE;
+    if (C < 8 || C > 128 || (C % 8) || (ldr % 8) || (ldx % 8) || (ldo % 8)) return ADSR_ERR_BAD_SHAPE;
     if (static_cast<long long>(HW) * (C / 8) >= (1ll << 31)) return ADSR_ERR_BAD_SHAPE;
     const int slices = std::max(1, std::min(64, HW * (C / 8) / 1024));
     return launch_pdl(rcab_ca_scale_kernel, dim3(slices, B), dim3(256), 0, static_cast<cudaStream_t>(stream),
                       static_cast<const __nv_bfloat16*>(res), static_cast<long long>(ldr), static_cast<const __nv_bfloat16*>(x),
-                      static_cast<long long>(ldx), static_cast<__nv_bfloat16*>(out), static_cast<long long>(ldo), mean, w1, b1, w2, b2, HW, C,
-                      Cr) == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
+                      static_cast<long long>(ldx), static_cast<__nv_bfloat16*>(out), static_cast<long long>(ldo), scale, HW,
+                      C) == cudaSuccess ? ADSR_OK : ADSR_ERR_LAUNCH;
 }

@@ -211,17 +211,18 @@ class DRN(nn.Module):
             t1 = torch.empty(rows[p], round_up(c, 16), **bf)
             t2 = torch.empty(rows[p], round_up(c, 16), **bf)
             gap = torch.empty(B, c, dtype=torch.float32, device=dev)
-            n_parts = ops.halo_parts(res[p][0], res[p][1])
+            n_parts = ops.halo_parts(res[p][0], res[p][1])                   # >= channel_mean_slices(hw)
             parts = torch.empty(B * n_parts, round_up(c, 16), dtype=torch.float32, device=dev)
             for r in lvl["rcabs"]:
                 ops.conv3x3(xbuf, B, res[p][0], res[p][1], c, r["c1"], t1, act=ops.ACT_RELU)
-                # CALayer's pooled mean leaves the second conv's epilogue as per-tile partial sums when the halo kernel covers it
-                if ops.conv3x3(t1, B, res[p][0], res[p][1], c, r["c2"], t2, chan_part=parts):
-                    ops.channel_mean_parts(parts, B, n_parts, c, hw, gap, r["w1"], r["b1"], r["w2"], r["b2"], r["cr"])
-                    ops.rcab_ca_scale(t2, xbuf, xbuf, gap, r["w1"], r["b1"], r["w2"], r["b2"], B, hw, c, 0)     # gap = the scales
-                    continue
-                ops.channel_mean(t2, B, hw, c, gap)
-                ops.rcab_ca_scale(t2, xbuf, xbuf, gap, r["w1"], r["b1"], r["w2"], r["b2"], B, hw, c, r["cr"])
+                # CALayer's pooled mean leaves the second conv's epilogue as per-tile partial sums when the halo kernel covers it,
+                # else channel_mean writes per-slice sums in the same layout: both reduced in a fixed order
+                n = n_parts
+                if not ops.conv3x3(t1, B, res[p][0], res[p][1], c, r["c2"], t2, chan_part=parts):
+                    n = ops.channel_mean_slices(hw)
+                    ops.channel_sums(t2, B, hw, c, parts)
+                ops.channel_mean_parts(parts, B, n, c, hw, gap, r["w1"], r["b1"], r["w2"], r["b2"], r["cr"])
+                ops.rcab_ca_scale(t2, xbuf, xbuf, gap, r["w1"], r["b1"], r["w2"], r["b2"], B, hw, c, 0)     # gap = the scales
             shuf = torch.empty(rows[p - 1], round_up(c, 16), **bf)
             ops.conv3x3(xbuf, B, res[p][0], res[p][1], c, lvl["up"], shuf, out_mode=ops.OUT_PIXEL_SHUFFLE2)
             ops.tc_gemm(shuf, c, lvl["c1x1"], cat[p - 1], n_store=lvl["cout"])

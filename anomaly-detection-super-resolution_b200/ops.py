@@ -187,7 +187,7 @@ def halo_parts(h: int, wd: int) -> int:
 def channel_mean_parts(part: torch.Tensor, b: int, parts: int, c: int, hw: int, mean: torch.Tensor, w1=None, b1=None, w2=None, b2=None,
                        cr: int = 0) -> None:
     """mean [b, c] <- pooled means from the halo conv's partial sums; with the CALayer weights given: the sigmoid scales instead
-    (pass them to rcab_ca_scale with cr=0)."""
+    (pass them to rcab_ca_scale)."""
     _t = _begin()
     check(lib().adsr_channel_mean_parts(ptr(part), b, parts, part.stride(0), c, hw, ptr(mean), ptr(w1), ptr(b1), ptr(w2), ptr(b2), cr,
                                         stream_ptr()), "adsr_channel_mean_parts")
@@ -598,17 +598,39 @@ def conv3x3_small(x: torch.Tensor, weight, bias, c: int, out1: torch.Tensor, out
     _count("conv3x3_small", 2.0 * b * h * w * 9 * nc * c, _t)
 
 
-def channel_mean(x: torch.Tensor, b: int, hw: int, c: int, mean: torch.Tensor) -> None:
+def channel_mean_slices(hw: int) -> int:
+    """Partial-sum rows per image written by channel_sums: pixel slices of at least 256 pixels, at most 32."""
+    return max(1, min(32, hw // 256))
+
+
+def channel_sums(x: torch.Tensor, b: int, hw: int, c: int, part: torch.Tensor) -> None:
+    """part [b * channel_mean_slices(hw), >= c] fp32 <- per-slice column sums of x, the partial-row layout channel_mean_parts
+    reduces in a fixed order (CALayer's pooled mean where the halo conv does not run)."""
     _cuda(x, "x")
     _t = _begin()
-    check(lib().adsr_channel_mean(ptr(x), x.stride(0), b, hw, c, ptr(mean), stream_ptr()), "adsr_channel_mean")
+    check(lib().adsr_channel_mean(ptr(x), x.stride(0), b, hw, c, channel_mean_slices(hw), ptr(part), part.stride(0), stream_ptr()),
+          "adsr_channel_mean")
     _count("channel_mean", 0.0, _t)
+
+
+def channel_mean(x: torch.Tensor, b: int, hw: int, c: int, mean: torch.Tensor) -> None:
+    """mean [b, c] <- AdaptiveAvgPool2d(1) of x [b*hw, >= c] bf16 rows: channel_sums + channel_mean_parts, a fixed order."""
+    n = channel_mean_slices(hw)
+    part = torch.empty(b * n, c, dtype=torch.float32, device=x.device)
+    channel_sums(x, b, hw, c, part)
+    channel_mean_parts(part, b, n, c, hw, mean)
 
 
 def rcab_ca_scale(res: torch.Tensor, x: torch.Tensor, out: torch.Tensor, mean, w1, b1, w2, b2, b: int, hw: int, c: int,
                   cr: int) -> None:
+    """out = x + res * s[b].  cr = 0: `mean` already holds the scales (channel_mean_parts with the CALayer weights); cr > 0: the
+    means, and s = sigmoid(W2 relu(W1 mean + b1) + b2) comes from channel_mean_parts over one partial row per image."""
     _cuda(res, "res")
+    scale = mean
+    if cr > 0:
+        scale = torch.empty(b, c, dtype=torch.float32, device=res.device)
+        channel_mean_parts(mean, b, 1, c, 1, scale, w1, b1, w2, b2, cr)
     _t = _begin()
-    check(lib().adsr_rcab_ca_scale(ptr(res), res.stride(0), ptr(x), x.stride(0), ptr(out), out.stride(0), ptr(mean), ptr(w1),
-                                   ptr(b1), ptr(w2), ptr(b2), b, hw, c, cr, stream_ptr()), "adsr_rcab_ca_scale")
+    check(lib().adsr_rcab_ca_scale(ptr(res), res.stride(0), ptr(x), x.stride(0), ptr(out), out.stride(0), ptr(scale), b, hw, c,
+                                   stream_ptr()), "adsr_rcab_ca_scale")
     _count("rcab_ca_scale", 0.0, _t)

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define ADSR_ABI_VERSION 20
+#define ADSR_ABI_VERSION 21
 
 #define ADSR_OK 0
 #define ADSR_ERR_BAD_SHAPE 1   /* unsupported dimensions (e.g. window size whose N does not tile 64) */
@@ -162,7 +162,7 @@ int adsr_conv3x3_halo_bf16(const void* in, int64_t ld_in, int B, int H, int W, i
                            float* chan_part, int num_sms, void* stream);
 /* mean[b, c] = (sum over the `parts` partial rows of image b) / HW, summed in a fixed order (deterministic).  With w1 != NULL the
  * kernel continues with CALayer's conv_du (src/drn.py:128-133) and writes sigmoid(W2 relu(W1 mean + b1) + b2) into `mean` instead:
- * adsr_rcab_ca_scale then takes that buffer with Cr = 0 (scales given, no per-block MLP). */
+ * adsr_rcab_ca_scale then takes that buffer as its scales. */
 int adsr_channel_mean_parts(const float* chan_part, int B, int parts, int ld_part, int C, int HW, float* mean,
                             const float* w1, const float* b1, const float* w2, const float* b2, int Cr, void* stream);
 
@@ -223,16 +223,17 @@ int adsr_quantize_u8(const float* x_nchw, int B, int nc, int H, int W, float rgb
  *   (src/drn.py:174-175, 243-246); mat = [nc, nc] fp32, bias = [nc].   fp32 NCHW in and out.
  * adsr_conv3x3_small: `head` conv, Cin <= 3 (fp32 NCHW) -> C <= 64 channels NHWC bf16 (src/drn.py:187, 247), written to
  *   out1 and, optionally, to the column slice col2.. of out2 (the skip-connection half of the later torch.cat).
- * adsr_channel_mean: AdaptiveAvgPool2d(1) of CALayer (src/drn.py:126, 137): x [B, HW, ld] bf16 -> mean [B, C] fp32.
- * adsr_rcab_ca_scale: out = res * sigmoid(W2 relu(W1 mean + b1) + b2) + x   (src/drn.py:128-139, 155-158). */
+ * adsr_channel_mean: the pooling partials of CALayer (src/drn.py:126, 137) where the halo conv does not run: x [B, HW, ld] bf16
+ *   (C % 8 == 0, 16-byte aligned rows) -> part[(b * slices + s) * ld_part + c] = column sums of pixel slice s, for
+ *   adsr_channel_mean_parts(part, B, slices, ...): a fixed summation order, so the result does not depend on scheduling or the batch.
+ * adsr_rcab_ca_scale: out = res * scale[b] + x   (src/drn.py:139, 155-158), scale [B, C] from adsr_channel_mean_parts with the MLP. */
 int adsr_bicubic_affine(const float* x_nchw, int B, int nc, int h, int w, int scale, const float* mat,
                         const float* bias, float* out_nchw, void* stream);
 int adsr_conv3x3_small(const float* x_nchw, int B, int nc, int H, int W, const float* weight, const float* bias,
                        int C, void* out1, int64_t ld1, void* out2, int64_t ld2, int col2, void* stream);
-int adsr_channel_mean(const void* x, int64_t ld, int B, int HW, int C, float* mean, void* stream);
+int adsr_channel_mean(const void* x, int64_t ld, int B, int HW, int C, int slices, float* part, int64_t ld_part, void* stream);
 int adsr_rcab_ca_scale(const void* res, int64_t ldr, const void* x, int64_t ldx, void* out, int64_t ldo,
-                       const float* mean, const float* w1, const float* b1, const float* w2, const float* b2,
-                       int B, int HW, int C, int Cr, void* stream);
+                       const float* scale, int B, int HW, int C, void* stream);
 
 /* ---- per-image anomaly scores ---------------------------------------------------------------------------------
  * replaces ssim_numpy (src/metrics.py:26-67) for every window size of the sweep (src/evaluate.py:233-248),

@@ -2,7 +2,8 @@
 
 Covers the fused attention half (csrc/swin_attn.cu), the standalone window attention (csrc/attention*.cu), the fused
 Swin MLP with its three epilogues (csrc/swin_mlp.cu) and the GEMM kernels with or without the folded LayerNorm
-(csrc/tc_gemm*.cu).
+(csrc/tc_gemm*.cu), the 3x3 convs on every dispatch branch (csrc/conv_halo.cu and the implicit GEMM) and DRN's CALayer / RCAB
+kernels (csrc/drn_ops.cu).
 
 Every weight comes from the packed images (unpack_* below invert pack._swizzle_slab / pack._swizzle_tiles), so the
 reference uses the kernels' own gamma fold and its bf16 rounding, colsum from the bf16 weights, GELU's 0.5 in fc2, the
@@ -274,6 +275,116 @@ def gemm(a, k, pw, *, act="none", slope=0.0, alpha=1.0, res=None, stats=None, sl
     return v
 
 
+# ------------------------------------------------------------------------------------------------ convolutions (DRCT, DRN)
+def unpack_conv(pw, compact: bool = False) -> torch.Tensor:
+    """Inverse of pack.pack_conv3x3_weight -> fp64 [Cout, Cin, 3, 3].  The tiled implicit-GEMM image has K = tap * round64(Cin) + c;
+    the `compact` halo twin (csrc/conv_halo.cu) K = tap * round16(Cin) + c in one N tile of round16(Cout) rows."""
+    cout, cin = pw.N, pw.K
+    src = pw.compact if compact else pw
+    step = (cin + 15) // 16 * 16 if compact else (cin + 63) // 64 * 64
+    w = unpack_tiles(src)[:cout, :9 * step].reshape(cout, 9, step)[:, :, :cin]
+    return w.permute(0, 2, 1).reshape(cout, cin, 3, 3)
+
+
+def conv_input(x: torch.Tensor, B: int, H: int, W: int, cin: int, dt=F64) -> torch.Tensor:
+    """NHWC rows [B*H*W, >= cin] -> NCHW."""
+    return x[:, :cin].to(dt).reshape(B, H, W, cin).permute(0, 3, 1, 2)
+
+
+def rows_of(t: torch.Tensor) -> torch.Tensor:
+    """NCHW -> NHWC rows [B*H*W, C]."""
+    return t.permute(0, 2, 3, 1).reshape(-1, t.shape[1])
+
+
+def act_fn(v: torch.Tensor, act: str, slope: float) -> torch.Tensor:
+    if act == "relu":
+        return torch.clamp_min(v, 0.0)
+    if act == "lrelu":
+        return torch.where(v > 0, v, v * slope)
+    return v
+
+
+def conv_pre(xin: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, stride: int = 1, noise: bool = False) -> torch.Tensor:
+    """conv + bias, zero padding 1, NCHW.  noise=True: fp32, accumulated tap by tap (tap-major, then channel) like the kernels."""
+    if not noise:
+        return torch.nn.functional.conv2d(xin.to(F64), w.to(F64), bias.to(F64), stride=stride, padding=1)
+    xp = torch.nn.functional.pad(xin.float(), (1, 1, 1, 1))
+    B, _, H, W = xin.shape
+    Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
+    acc = torch.zeros(B, w.shape[0], Ho, Wo)
+    for ky in range(3):
+        for kx in range(3):
+            tap = xp[:, :, ky:ky + stride * (Ho - 1) + 1:stride, kx:kx + stride * (Wo - 1) + 1:stride]
+            acc = acc + torch.einsum("bchw,oc->bohw", tap, w[:, :, ky, kx].float())
+    return acc + bias.float()[None, :, None, None]
+
+
+def conv_epilogue(pre, *, act="none", slope=0.0, alpha=1.0, res=None, ps=False) -> torch.Tensor:
+    """alpha * act(pre) (+ res rows) -> output rows; `ps`: PixelShuffle(2) rows [B*2Ho*2Wo, N/4].  The manual epilogue
+    (tc_gemm_manual.cu) rounds alpha * act(.) to bf16 before it adds the residual, the TMA epilogue (tc_gemm.cu) adds it in fp32:
+    `compare(..., rounded_branch=True)` charges the first rounding."""
+    v = act_fn(pre, act, slope) * alpha
+    if ps:
+        return rows_of(torch.nn.functional.pixel_shuffle(v, 2))
+    v = rows_of(v)
+    if res is not None:
+        v = v + res[:, :v.shape[1]].to(v.dtype)
+    return v
+
+
+def conv3x3(x, B, H, W, cin, pw, *, stride=1, act="none", slope=0.0, alpha=1.0, res=None, ps=False, compact=False,
+            noise=False) -> torch.Tensor:
+    """adsr_conv3x3_igemm_bf16 / adsr_conv3x3_halo_bf16 from the packed image: alpha * act(conv(x) + b) (+ res), fp64 (noise:
+    fp32 tap-major accumulation), output rows before their bf16 rounding."""
+    w = unpack_conv(pw, compact).to(x.device)
+    bias = (pw.compact if compact else pw).bias[:pw.N].to(x.device)
+    pre = conv_pre(conv_input(x, B, H, W, cin, torch.float32 if noise else F64), w, bias, stride, noise)
+    return conv_epilogue(pre, act=act, slope=slope, alpha=alpha, res=res, ps=ps)
+
+
+def conv3x3_small(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
+    """adsr_conv3x3_small (DRN head): fp32 NCHW input and weights -> rows [B*H*W, C] before the bf16 rounding."""
+    return rows_of(conv_pre(x, w, b))
+
+
+def channel_mean(t: torch.Tensor, B: int, HW: int, C: int) -> torch.Tensor:
+    """AdaptiveAvgPool2d(1) of NHWC rows [B*HW, >= C] -> fp64 [B, C]."""
+    return t[:, :C].to(F64).reshape(B, HW, C).mean(1)
+
+
+def ca_scale(mean: torch.Tensor, w1, b1, w2, b2) -> torch.Tensor:
+    """CALayer's squeeze-excite: sigmoid(W2 relu(W1 mean + b1) + b2), fp64 [B, C]."""
+    h = torch.clamp_min(mean.to(F64) @ w1.to(F64).t() + b1.to(F64), 0.0)
+    return torch.sigmoid(h @ w2.to(F64).t() + b2.to(F64))
+
+
+def channel_mean_parts(part: torch.Tensor, B: int, parts: int, C: int, HW: int, mlp=None) -> torch.Tensor:
+    """adsr_channel_mean_parts: [B*parts, >= C] fp32 partial sums -> the means, or with mlp = (w1, b1, w2, b2) the CA scales."""
+    mean = part[:, :C].to(F64).reshape(B, parts, C).sum(1) / HW
+    return mean if mlp is None else ca_scale(mean, *mlp)
+
+
+def rcab_ca_scale(t2: torch.Tensor, x: torch.Tensor, scale: torch.Tensor, B: int, HW: int, C: int) -> torch.Tensor:
+    """adsr_rcab_ca_scale: x + t2 * s per image, rows before the bf16 rounding."""
+    t = t2[:, :C].to(F64).reshape(B, HW, C)
+    return (x[:, :C].to(F64).reshape(B, HW, C) + t * scale.to(F64)[:, None, :]).reshape(B * HW, C)
+
+
+def rcab(x, B, H, W, c1, c2, mlp, *, noise=False, pool_hw=None, scale_fn=None):
+    """One RCAB of DRN: t1 = bf16(ReLU(c1 x)), t2 = bf16(c2 t1), s = CA(mean(t2)), x + t2 * s before the bf16 rounding.
+    The pooled mean is taken from t2 before its rounding (the halo epilogue's partial sums); the fallback pools the bf16 t2,
+    the same to ~ulp / sqrt(HW).  pool_hw / scale_fn state CA defects: the mean's divisor and the map from means to scales."""
+    C = c1.N
+    t1 = bf16(conv3x3(x, B, H, W, C, c1, act="relu", noise=noise))
+    t2p = conv3x3(t1, B, H, W, C, c2, noise=noise)
+    t2 = bf16(t2p)
+    mean = t2p.to(F64).reshape(B, H * W, C).sum(1) / (H * W if pool_hw is None else pool_hw)
+    s = ca_scale(mean, *mlp) if scale_fn is None else scale_fn(mean)
+    if noise:
+        s = s.float().double()
+    return rcab_ca_scale(t2, x, s, B, H * W, C)
+
+
 # ------------------------------------------------------------------------------------------------ comparator
 def ulp_bf16(t: torch.Tensor) -> torch.Tensor:
     """Spacing of bf16 numbers at |t| (8 significant bits); 0 at 0."""
@@ -298,17 +409,19 @@ class Verdict:
                 f"in units of rms(branch)")
 
 
-def compare(got, ref, shortcut=None, *, b, rms_b, a=1.0) -> Verdict:
+def compare(got, ref, shortcut=None, *, b, rms_b, a=1.0, rounded_branch=False) -> Verdict:
     """Per element |got - ref| <= a ulp_bf16(ref) + b rms(branch), branch = ref - shortcut (the whole output without a
     shortcut), and the RMS error net of the output rounding's mean square ulp^2 / 12 <= rms_b rms(branch).  `ref` is the
-    output before its bf16 rounding; `got` what the kernel stored."""
+    output before its bf16 rounding; `got` what the kernel stored.  rounded_branch: the kernel rounded the branch to bf16
+    before it added the shortcut, charged like the output rounding (half an ulp of the branch, mean square ulp^2 / 12)."""
     ref = ref.to(F64)
     err = got.to(F64) - ref
     branch = ref if shortcut is None else ref - shortcut.to(F64)
     scale = float(branch.square().mean().sqrt().clamp_min(1e-30))
     ulp = ulp_bf16(ref)
-    mx = float((err.abs() - a * ulp).max()) / scale
-    ms = float(err.square().mean() - ulp.square().mean() / 12.0)
+    ulp_b = ulp_bf16(branch) if rounded_branch else torch.zeros_like(ulp)
+    mx = float((err.abs() - a * ulp - 0.5 * ulp_b).max()) / scale
+    ms = float(err.square().mean() - ulp.square().mean() / 12.0 - ulp_b.square().mean() / 12.0)
     return Verdict(mx, math.sqrt(max(ms, 0.0)) / scale, b, rms_b)
 
 
@@ -454,6 +567,40 @@ def ln_gemm_case(M, K, N, seed, *, rows=False, mean_std=None):
     return dict(a=a, stats=st, pw=pw, raw=dict(w=w, b=b, gamma=gm, beta=bt))
 
 
+def conv_case(B, H, W, Cin, Cout, seed, *, res=False, ld=None, fill=0.0):
+    """bf16 NHWC rows [B*H*W, ld] (columns >= Cin hold `fill`, the 8-channel K tail zeros), weights ~ N(0, 0.05^2), bias ~ N(0, 1),
+    and for `res` bf16 residual rows; Ho, Wo at stride 1 (the caller sizes a stride-2 residual itself)."""
+    from importlib import import_module
+    pack = import_module("anomaly-detection-super-resolution_b200.pack")
+    g = _gen(seed)
+    ld = (Cin + 15) // 16 * 16 if ld is None else ld
+    x = torch.full((B * H * W, ld), fill, dtype=torch.bfloat16)
+    x[:, :Cin] = torch.randn(B * H * W, Cin, generator=g).to(torch.bfloat16)
+    x[:, Cin:(Cin + 7) // 8 * 8] = 0
+    w = torch.randn(Cout, Cin, 3, 3, generator=g) * 0.05
+    bias = torch.randn(Cout, generator=g)
+    r = (torch.randn(B * H * W, (Cout + 15) // 16 * 16, generator=g)).to(torch.bfloat16) if res else None
+    return dict(x=x, w=w, bias=bias, pw=pack.pack_conv3x3_weight(w, bias), res=r)
+
+
+def rcab_case(B, H, W, C, seed):
+    """One RCAB's inputs: bf16 x rows [B*H*W, round16(C)], c1 / c2 packed with DRN's init scale, CALayer weights (C // 16 hidden)."""
+    from importlib import import_module
+    pack = import_module("anomaly-detection-super-resolution_b200.pack")
+    g = _gen(seed)
+    ld = (C + 15) // 16 * 16
+    x = torch.zeros(B * H * W, ld, dtype=torch.bfloat16)
+    off = torch.randn(B, 1, C, generator=g) * 1.5                 # per-image channel offsets: images differ in their CA scales
+    x[:, :C] = (torch.randn(B, H * W, C, generator=g) * 2.0 + off).reshape(-1, C).to(torch.bfloat16)
+    s = (9 * C) ** -0.5
+    c1 = pack.pack_conv3x3_weight(torch.randn(C, C, 3, 3, generator=g) * s, torch.randn(C, generator=g) * 0.2)
+    c2 = pack.pack_conv3x3_weight(torch.randn(C, C, 3, 3, generator=g) * s, torch.randn(C, generator=g) * 0.5)
+    cr = C // 16
+    mlp = (torch.randn(cr, C, generator=g), torch.randn(cr, generator=g) * 0.1,
+           torch.randn(C, cr, generator=g), torch.randn(C, generator=g) * 0.1)
+    return dict(x=x, c1=c1, c2=c2, mlp=mlp, B=B, H=H, W=W, C=C)
+
+
 # ------------------------------------------------------------------------------------------------ tolerances
 # (b, rms_b) of `compare` per kernel, in units of rms(branch); a = 1 ulp everywhere.  Bounded from below by the largest
 # error measured on a B200 (1000 W power limit) over the seeded GPU cases and by the simulated kernel noise (`noise=True`),
@@ -462,11 +609,15 @@ def ln_gemm_case(M, K, N, seed, *, rows=False, mean_std=None):
 #   attention  measured max 0.017 / rms 0.0017;                                   softmax scale +1 % gives rms 0.0098
 #   swin_mlp   measured max 0.0085 / rms 0.0016 (mean/std 100);                  colsum from fp32 weights gives 0.079
 #   gemm       measured max 0.0016 / rms 0.00032;                                 LayerNorm eps 1e-3 gives > 0.01
+#   conv       measured within 1 ulp, rms <= 0.00094 (double-rounded residual);   ReLU for LeakyReLU(0.01) gives 0.067 / 0.011
+#   rcab       measured max 0.0137 / rms 0.00029;                                 pad columns pooled gives 0.046 / 0.0045 (64 px)
 TOL = {
     "swin_attn": (0.045, 0.005),      # q | k | v and O are bf16 operands: their rounding flips are the noise floor
     "attention": (0.03, 0.004),
     "swin_mlp": (0.012, 0.003),       # one bf16 intermediate: the GELU activations, from a GELU approximation good to 8.6e-5
     "gemm": (0.003, 0.0008),          # fp32 accumulation only
+    "conv": (0.003, 0.0008),          # exact bf16 inputs and weights: fp32 accumulation order only
+    "rcab": (0.02, 0.003),            # bf16 t1 and t2 between the stages: a rounding flip of t2 shows as ulp(t2) * s
 }
 # Logits about 10 apart: where two keys nearly tie, O moves by p (1 - p) |v1 - v2| per unit of logit error, so the fp32
 # logits' rounding shows in single elements (simulated noise 0.035, B200 0.074 on C = 244); the RMS limit is unchanged.

@@ -1,12 +1,11 @@
-"""GPU parity of the tcgen05 GEMM kernels (csrc/tc_gemm.cu, the row-tile csrc/tc_gemm_rows.cu) against the fp64 reference of
-oracle/hotpath_oracle.py on the packed weights, with the comparator in units of the GEMM output; the implicit-GEMM convs
-against fp32 torch on bf16-rounded inputs."""
+"""GPU parity of the tcgen05 GEMM kernels (csrc/tc_gemm.cu, the row-tile csrc/tc_gemm_rows.cu) and of the 3x3 convs (the
+implicit GEMM on its three branches, the halo-tile csrc/conv_halo.cu) against the fp64 reference of oracle/hotpath_oracle.py on
+the packed weights, with the comparator in units of the output (of the conv branch when a residual is added)."""
 import pytest
 import torch
-import torch.nn.functional as F
 
 from oracle import hotpath_oracle as R
-from gpu_common import bf16_round, mod, rel_err
+from gpu_common import mod
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -98,37 +97,62 @@ def test_gemm_rows_kernel_epilogues():
     _gemm_case(700, 276, 276, act="relu", res=True, seed=20, rows=True)
 
 
-def _conv_case(B, H, W, Cin, Cout, stride=1, act="none", res=False, ps=False, seed=0):
-    ops, pack = mod("ops"), mod("pack")
-    torch.manual_seed(seed)
-    ld = (Cin + 15) // 16 * 16
-    x = torch.zeros(B * H * W, ld, device=DEV, dtype=torch.bfloat16)
-    x[:, :Cin] = torch.randn(B * H * W, Cin, device=DEV).to(torch.bfloat16)
-    w = torch.randn(Cout, Cin, 3, 3, device=DEV) * 0.05
-    bias = torch.randn(Cout, device=DEV)
-    pw = pack.pack_conv3x3_weight(w, bias)
+CONV_TOL = R.TOL["conv"]
+# conv dispatch (ops.conv3x3 -> conv_halo.cu, tc_gemm.cu): the kernel each branch launches, as torch.profiler names it
+CONV_KERNEL = {"halo": r"conv_halo_kernel", "tma_box": r"tc_gemm_manual_kernel<\d+, 4>", "gather_tma_epi": r"tc_gemm_kernel<",
+               "gather_manual": r"tc_gemm_manual_kernel<\d+, 3>"}
+
+
+def _run_conv(c, B, H, W, Cin, Cout, *, stride=1, act="none", slope=0.01, res=False, ps=False, ocol0=0, n_store=None, ld_out=None,
+              halo=True, chan_part=None):
+    """ops.conv3x3 on the case's bf16 rows into a poisoned output; returns (out, got rows, Ho, Wo)."""
+    ops = mod("ops")
     Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
-    xin = x[:, :Cin].float().view(B, H, W, Cin).permute(0, 3, 1, 2)
-    want = F.conv2d(xin, bf16_round(w), bias, stride=stride, padding=1)
-    code = {"none": ops.ACT_NONE, "lrelu": ops.ACT_LRELU}[act]
-    if act == "lrelu":
-        want = F.leaky_relu(want, 0.01)
-    r = None
-    if res:
-        r = torch.randn(B * Ho * Wo, (Cout + 15) // 16 * 16, device=DEV).to(torch.bfloat16)
-        want = want + r[:, :Cout].float().view(B, Ho, Wo, Cout).permute(0, 3, 1, 2)
-    if ps:
-        want = F.pixel_shuffle(want, 2)
-        out = torch.zeros(B * 4 * Ho * Wo, Cout // 4, device=DEV, dtype=torch.bfloat16)
-        ops.conv3x3(x, B, H, W, Cin, pw, out, out_mode=ops.OUT_PIXEL_SHUFFLE2)
-        got = out.float().view(B, 2 * Ho, 2 * Wo, Cout // 4).permute(0, 3, 1, 2)
-    else:
-        out = torch.zeros(B * Ho * Wo, (Cout + 15) // 16 * 16, device=DEV, dtype=torch.bfloat16)
-        ops.conv3x3(x, B, H, W, Cin, pw, out, stride=stride, act=code, slope=0.01, res=r)
-        got = out[:, :Cout].float().view(B, Ho, Wo, Cout).permute(0, 3, 1, 2)
+    pw = mod("pack").to_device(c["pw"], DEV)
+    x = c["x"].to(DEV)
+    r = c["res"][:B * Ho * Wo].to(DEV) if res else None
+    code = {"none": ops.ACT_NONE, "lrelu": ops.ACT_LRELU, "relu": ops.ACT_RELU}[act]
+    old = ops._HALO_CONV
+    ops._HALO_CONV = halo
+    try:
+        if ps:
+            out = torch.full((B * 4 * Ho * Wo, Cout // 4 + 8), -7.0, device=DEV, dtype=torch.bfloat16)
+            ops.conv3x3(x, B, H, W, Cin, pw, out[:, :Cout // 4], out_mode=ops.OUT_PIXEL_SHUFFLE2, act=code, slope=slope)
+            got = out[:, :Cout // 4]
+        else:
+            ns = (Cout + 15) // 16 * 16 if n_store is None else n_store
+            out = torch.full((B * Ho * Wo, ld_out or ocol0 + ns + 16), -7.0, device=DEV, dtype=torch.bfloat16)
+            ran_halo = ops.conv3x3(x, B, H, W, Cin, pw, out, stride=stride, act=code, slope=slope, res=r, ocol0=ocol0, n_store=n_store,
+                                   chan_part=chan_part)
+            got = out[:, ocol0:ocol0 + Cout]
+    finally:
+        ops._HALO_CONV = old
     torch.cuda.synchronize()
-    err = rel_err(got, want)
-    assert err < 0.012, f"conv B={B} H={H} Cin={Cin} Cout={Cout} s={stride} ps={ps}: rel err {err}"
+    return out, got, Ho, Wo
+
+
+def _conv_case(B, H, W, Cin, Cout, stride=1, act="none", res=False, ps=False, seed=0, slope=0.01, halo=True, branch=None):
+    """Implicit-GEMM / halo conv against the fp64 reference from the packed image.  `branch` names the dispatch branch when a
+    residual is added: the manual epilogue (TMA-box A tiles) rounds the conv branch to bf16 before it adds the residual, and the
+    comparator charges that rounding."""
+    c = R.conv_case(B, H, W, Cin, Cout, seed, res=res)
+    out, got, Ho, Wo = _run_conv(c, B, H, W, Cin, Cout, stride=stride, act=act, slope=slope, res=res, ps=ps, halo=halo)
+    r = c["res"][:B * Ho * Wo] if res else None
+    if branch is None and res:
+        branch = "tma_box" if stride == 1 and W <= 128 and 128 % W == 0 and (H * W) % 128 == 0 else "gather_tma_epi"
+    ref = R.conv3x3(c["x"], B, H, W, Cin, c["pw"], stride=stride, act=act, slope=slope, res=r, ps=ps)
+    tag = f"conv B={B} H={H} W={W} Cin={Cin} Cout={Cout} s={stride} act={act} res={res} ps={ps} halo={halo}"
+    assert bool(torch.isfinite(got.float()).all()), f"{tag}: non-finite output"
+    rounded = res and branch in ("tma_box", "gather_manual")
+    # two roundings in a row are not two independent uniform noises: B200 measured rms 0.00094 on tma_box_res
+    v = R.compare(got.cpu(), ref, r[:, :Cout] if res else None, b=CONV_TOL[0], rms_b=0.0015 if rounded else CONV_TOL[1],
+                  rounded_branch=rounded)
+    print(f"[conv] {tag}: {v}")
+    assert v.ok, f"{tag}: {v}"
+    ns = Cout // 4 if ps else (Cout + 15) // 16 * 16
+    if not ps and ns > Cout:
+        assert float(out[:, Cout:ns].float().abs().max()) == 0.0, "padded columns must be exact zeros"
+    assert bool((out[:, ns:] == -7.0).all()), "wrote past n_store"
 
 
 def test_conv_64_to_64():
@@ -153,20 +177,115 @@ def test_conv_stride2_and_odd_sizes():
     _conv_case(3, 20, 12, 16, 32, seed=6)        # M not a multiple of 128, tiles straddle images
 
 
+# (name, expected branch, shape and epilogue).  The halo kernel takes stride 1 without residual at 8 <= W <= 126 when its weights
+# and halo tile fit in shared memory; the TMA-box implicit GEMM stride-1 convs whose 128-pixel tiles are whole rows; a residual
+# elsewhere the TMA epilogue; everything else the gather producers with the manual epilogue.
+CONV_DISPATCH = [
+    ("halo_w8", "halo", dict(B=3, H=8, W=8, Cin=20, Cout=20, act="relu")),
+    ("halo_w126_h1", "halo", dict(B=4, H=1, W=126, Cin=40, Cout=40, act="lrelu", slope=0.2)),
+    ("halo_tail_panel", "halo", dict(B=5, H=17, W=24, Cin=72, Cout=48, act="lrelu", slope=0.1, seed=72)),
+    ("halo_second_panel", "halo", dict(B=2, H=16, W=40, Cin=100, Cout=48, seed=100)),
+    ("halo_many_tiles", "halo", dict(B=160, H=16, W=16, Cin=96, Cout=32, act="relu")),
+    ("halo_bad_shape", "gather_manual", dict(B=1, H=9, W=126, Cin=128, Cout=48)),             # 110 KB weights + 160 KB halo
+    ("tma_box_w128", "tma_box", dict(B=2, H=3, W=128, Cin=64, Cout=64, halo=False)),
+    ("tma_box_res", "tma_box", dict(B=2, H=24, W=32, Cin=64, Cout=64, act="lrelu", slope=0.2, res=True, seed=24)),
+    ("tma_box_ps", "tma_box", dict(B=2, H=32, W=32, Cin=64, Cout=256, ps=True, seed=3)),
+    ("tma_box_tail_panel", "tma_box", dict(B=2, H=16, W=16, Cin=72, Cout=40, act="lrelu", slope=0.01, halo=False)),
+    ("gather_res_w24", "gather_tma_epi", dict(B=2, H=24, W=24, Cin=64, Cout=64, act="lrelu", slope=0.2, res=True, seed=24)),
+    ("gather_res_w40", "gather_tma_epi", dict(B=3, H=16, W=40, Cin=96, Cout=96, res=True, seed=9)),
+    ("gather_hw_off128", "gather_manual", dict(B=2, H=17, W=32, Cin=100, Cout=64, halo=False)),   # W | 128, H*W % 128 != 0
+    ("gather_stride2_33x17", "gather_manual", dict(B=2, H=33, W=17, Cin=80, Cout=80, stride=2, act="lrelu", slope=0.2, seed=33)),
+    ("gather_ps_w40", "gather_manual", dict(B=2, H=20, W=40, Cin=40, Cout=160, ps=True)),
+    ("gather_many_tiles", "gather_manual", dict(B=40, H=33, W=33, Cin=40, Cout=40, act="relu", halo=False)),
+]
+
+
+def _profile_dispatch():
+    """{case name: names of the CUDA kernels torch.profiler records while the case's conv runs}."""
+    from torch.profiler import ProfilerActivity, profile
+    seen = {}
+    for name, _, kw in CONV_DISPATCH:
+        kw = dict(kw)
+        c = R.conv_case(kw["B"], kw["H"], kw["W"], kw["Cin"], kw["Cout"], kw.pop("seed", 0), res=kw.get("res", False))
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            _run_conv(c, **kw)
+        seen[name] = sorted({e.name for e in prof.events() if "kernel" in e.name})
+    return seen
+
+
+@pytest.fixture(scope="module")
+def dispatch_kernels():
+    """The kernel names of every dispatch case, profiled in a child process: after CUDA activity tracing has run in a process,
+    a later profiling session there can miss kernels (tests/test_gpu_scoring_dispatch.py recorded an empty trace after these
+    sessions), so this module leaves the test process's profiler untouched."""
+    import json
+    import os
+    import subprocess
+    import sys
+    tests = os.path.dirname(os.path.abspath(__file__))
+    code = (f"import json, sys; sys.path[:0] = [{os.path.dirname(tests)!r}, {tests!r}]; import test_gpu_gemm as T; "
+            "print('KERNELS ' + json.dumps(T._profile_dispatch()))")
+    p = subprocess.run([sys.executable, *subprocess._args_from_interpreter_flags(), "-c", code], capture_output=True, text=True,
+                       timeout=900)
+    assert p.returncode == 0, p.stderr[-4000:]
+    line = [ln for ln in p.stdout.splitlines() if ln.startswith("KERNELS ")][-1]
+    return json.loads(line[len("KERNELS "):])
+
+
+@pytest.mark.parametrize("name,branch,kw", CONV_DISPATCH, ids=[c[0] for c in CONV_DISPATCH])
+def test_conv_dispatch_branches(dispatch_kernels, name, branch, kw):
+    """Every conv branch against the reference; torch.profiler confirms the kernel the case names."""
+    import re
+    kw = dict(kw)
+    seed = kw.pop("seed", 0)
+    _conv_case(seed=seed, branch=branch, **kw)
+    names = dispatch_kernels[name]
+    print(f"[conv dispatch] {name}: {names}")
+    if not any(dispatch_kernels.values()):
+        pytest.skip("torch.profiler recorded no CUDA kernels on this runner")
+    hits = {b for b, pat in CONV_KERNEL.items() if any(re.search(pat, n) for n in names)}
+    assert hits == {branch}, (name, branch, names)
+
+
+def test_conv_dispatch_cases_cover_every_branch():
+    assert {c[1] for c in CONV_DISPATCH} == set(CONV_KERNEL)
+
+
+@pytest.mark.parametrize("halo", [True, False])
+def test_drn_conv_shapes_on_both_paths(halo):
+    """DRN's convs on the halo kernel and on the implicit GEMM: 40 -> 40 into columns [40, 80) of an 80-wide buffer, and 80 -> 80
+    with the CALayer partial sums."""
+    ops = mod("ops")
+    B, H, W = 2, 32, 32
+    c = R.conv_case(B, H, W, 40, 40, 40)
+    out, got, _, _ = _run_conv(c, B, H, W, 40, 40, ocol0=40, n_store=40, ld_out=80, halo=halo)
+    v = R.compare(got.cpu(), R.conv3x3(c["x"], B, H, W, 40, c["pw"]), b=CONV_TOL[0], rms_b=CONV_TOL[1])
+    print(f"[conv] DRN 40->40 slice halo={halo}: {v}")
+    assert v.ok and bool((out[:, :40] == -7.0).all())
+    c = R.conv_case(B, H, W, 80, 80, 80)
+    n_parts = ops.halo_parts(H, W)
+    parts = torch.full((B * n_parts, 80), float("nan"), device=DEV)
+    out, got, _, _ = _run_conv(c, B, H, W, 80, 80, act="relu", halo=halo, chan_part=parts)
+    ref = R.conv3x3(c["x"], B, H, W, 80, c["pw"], act="relu")
+    v = R.compare(got.cpu(), ref, b=CONV_TOL[0], rms_b=CONV_TOL[1])
+    print(f"[conv] DRN 80->80 halo={halo}: {v}")
+    assert v.ok
+    if halo:
+        mean = R.channel_mean_parts(parts.cpu(), B, n_parts, 80, H * W)
+        assert float((mean - R.channel_mean(ref, B, H * W, 80)).abs().max()) < 1e-5
+
+
 @pytest.mark.parametrize("B,H,W,Cin,Cout,act", [(3, 32, 32, 80, 80, "relu"), (2, 64, 64, 80, 80, "none"), (5, 17, 24, 40, 48, "lrelu"),
                                                 (1, 9, 126, 128, 16, "none"), (150, 16, 16, 64, 64, "relu"), (2, 8, 8, 20, 20, "none")])
 def test_conv_halo_tile_kernel(B, H, W, Cin, Cout, act):
     """Halo-tile conv with resident weights (csrc/conv_halo.cu), called directly: every tap offset / tile phase / image border,
-    poison in the untouched output columns, and equality with the streaming implicit GEMM on the same inputs."""
-    ops, pack, abi = mod("ops"), mod("pack"), mod("_abi")
-    torch.manual_seed(B * 131 + W)
+    poison in the untouched output columns, and the same reference on the streaming implicit GEMM."""
+    ops, abi = mod("ops"), mod("_abi")
     ld = (Cin + 15) // 16 * 16 + 16
-    x = torch.full((B * H * W, ld), 7.0, device=DEV, dtype=torch.bfloat16)      # columns >= Cin must not matter beyond round8
-    x[:, :Cin] = torch.randn(B * H * W, Cin, device=DEV).to(torch.bfloat16)
-    x[:, Cin:(Cin + 7) // 8 * 8] = 0
-    w = torch.randn(Cout, Cin, 3, 3, device=DEV) * 0.05
-    bias = torch.randn(Cout, device=DEV)
-    pw = pack.pack_conv3x3_weight(w, bias)
+    c = R.conv_case(B, H, W, Cin, Cout, B * 131 + W, ld=ld, fill=7.0)   # columns >= Cin must not matter beyond round8
+    x = c["x"].to(DEV)
+    pw = mod("pack").to_device(c["pw"], DEV)
     assert pw.compact is not None
     wc = pw.compact
     code = {"none": ops.ACT_NONE, "lrelu": ops.ACT_LRELU, "relu": ops.ACT_RELU}[act]
@@ -182,39 +301,40 @@ def test_conv_halo_tile_kernel(B, H, W, Cin, Cout, act):
     mean = torch.zeros(B, Cout, device=DEV)
     ops.channel_mean_parts(parts, B, n_parts, Cout, H * W, mean)
     torch.cuda.synchronize()
-    xin = x[:, :Cin].float().view(B, H, W, Cin).permute(0, 3, 1, 2)
-    want = F.conv2d(xin, bf16_round(w), bias, padding=1)
-    want = {"none": lambda t: t, "lrelu": lambda t: F.leaky_relu(t, 0.1), "relu": F.relu}[act](want)
-    got = out[:, 8:8 + Cout].float().view(B, H, W, Cout).permute(0, 3, 1, 2)
-    err = rel_err(got, want)
-    assert err < 0.012, f"halo conv rel err {err}"
+    ref = R.conv3x3(c["x"], B, H, W, Cin, pw, act=act, slope=0.1, compact=True)
+    v = R.compare(out[:, 8:8 + Cout].cpu(), ref, b=CONV_TOL[0], rms_b=CONV_TOL[1])
+    print(f"[conv] halo B={B} H={H} W={W} Cin={Cin} Cout={Cout} act={act}: {v}")
+    assert v.ok, v
     # pooled means from the epilogue's partial sums (fp32 values before the bf16 rounding): AdaptiveAvgPool2d(1) of the output
-    want_mean = want.mean(dim=(2, 3))
-    assert float((mean - want_mean).abs().max()) < 2e-3 * max(1.0, float(want_mean.abs().max())), "pooled mean"
+    want_mean = R.channel_mean(ref, B, H * W, Cout)
+    assert float((mean.cpu() - want_mean).abs().max()) < 1e-5 * max(1.0, float(want_mean.abs().max())), "pooled mean"
     assert bool(torch.isfinite(parts).all())
     # the same kernel continuing with CALayer's squeeze-excite MLP: sigmoid(W2 relu(W1 mean + b1) + b2)   (src/drn.py:128-139)
     cr = max(1, Cout // 16)
-    w1, b1 = torch.randn(cr, Cout, device=DEV) * 0.3, torch.randn(cr, device=DEV) * 0.1
-    w2, b2 = torch.randn(Cout, cr, device=DEV) * 0.3, torch.randn(Cout, device=DEV) * 0.1
+    g = torch.Generator().manual_seed(Cout)
+    mlp = [torch.randn(cr, Cout, generator=g) * 0.3, torch.randn(cr, generator=g) * 0.1, torch.randn(Cout, cr, generator=g) * 0.3,
+           torch.randn(Cout, generator=g) * 0.1]
     scale = torch.zeros(B, Cout, device=DEV)
-    ops.channel_mean_parts(parts, B, n_parts, Cout, H * W, scale, w1, b1, w2, b2, cr)
+    ops.channel_mean_parts(parts, B, n_parts, Cout, H * W, scale, *[t.to(DEV) for t in mlp], cr)
     torch.cuda.synchronize()
-    want_scale = torch.sigmoid(F.relu(mean @ w1.t() + b1) @ w2.t() + b2)
-    assert float((scale - want_scale).abs().max()) < 1e-5
+    assert float((scale.cpu() - R.channel_mean_parts(parts.cpu(), B, n_parts, Cout, H * W, mlp)).abs().max()) < 1e-5
     assert bool((out[:, :8] == -3.0).all()) and bool((out[:, 8 + n_store:] == -3.0).all())
     assert bool((out_g[:32] == -3.0).all()) and bool((out_g[-32:] == -3.0).all())
     assert bool(torch.isnan(parts_g[:8]).all()) and bool(torch.isnan(parts_g[-8:]).all())
     assert bool((out[:, 8 + Cout:8 + n_store] == 0).all())                      # padded output channels: zero weights, zero bias
-    # the streaming kernel computes the same sums in a different K order: equal to bf16 rounding
-    ref = torch.zeros(B * H * W, n_store, device=DEV, dtype=torch.bfloat16)
+    # the streaming kernel: the same reference, its own summation order
+    o2 = torch.full((B * H * W, n_store + 16), -3.0, device=DEV, dtype=torch.bfloat16)
     old = ops._HALO_CONV
     ops._HALO_CONV = False
     try:
-        ops.conv3x3(x, B, H, W, Cin, pw, ref, act=code, slope=0.1)
+        ops.conv3x3(x, B, H, W, Cin, pw, o2, act=code, slope=0.1)
     finally:
         ops._HALO_CONV = old
     torch.cuda.synchronize()
-    assert rel_err(out[:, 8:8 + Cout].float(), ref[:, :Cout].float()) < 0.006
+    v = R.compare(o2[:, :Cout].cpu(), ref, b=CONV_TOL[0], rms_b=CONV_TOL[1])
+    print(f"[conv] igemm B={B} H={H} W={W} Cin={Cin} Cout={Cout} act={act}: {v}")
+    assert v.ok, v
+    assert bool((o2[:, n_store:] == -3.0).all()) and bool((o2[:, Cout:n_store] == 0).all())
 
 
 def _row_stats(t: torch.Tensor, slots: int) -> torch.Tensor:

@@ -423,3 +423,201 @@ def test_one_pass_variance_breaks_down_beyond_the_supported_range():
     ref = _attn(case, True)
     v = _verdict(R.bf16(_attn(case, True, noise=True).double()), ref, case["x"].double(), "swin_attn")
     assert not v.ok
+
+
+# ------------------------------------------------------------------------------------------------ convolutions and the RCAB
+@pytest.mark.parametrize("cin", [3, 20, 40, 64, 72, 80, 96, 128, 180])
+@pytest.mark.parametrize("cout", [16, 20, 40, 64, 80, 256])
+def test_unpack_conv_inverts_pack(cin, cout):
+    g = torch.Generator().manual_seed(cin * 1000 + cout)
+    w = _bfw(cout, cin, 3, 3, g=g)
+    pw = pack.pack_conv3x3_weight(w, None)
+    assert torch.equal(R.unpack_conv(pw), w.double())
+    slabs = (9 * ((cin + 15) // 16 * 16) + 63) // 64
+    fits = cin <= 128 and cout <= 128 and slabs * ((cout + 15) // 16 * 16) * 128 <= 126 * 1024   # halo weights resident in smem
+    assert (pw.compact is not None) == fits
+    if fits:
+        assert torch.equal(R.unpack_conv(pw, compact=True), w.double())
+
+
+def test_conv_references_match_restatement(no_rounding):
+    """Plain F.conv2d / torch restatements from the fp32 parameters (bf16-representable weights, so packing is exact)."""
+    g = torch.Generator().manual_seed(11)
+    B, H, W, C = 2, 12, 20, 40
+    x = torch.randn(B * H * W, C, generator=g).to(torch.bfloat16)
+    w, b = _bfw(C, C, 3, 3, g=g), torch.randn(C, generator=g)
+    pw = pack.pack_conv3x3_weight(w, b)
+    xin = x.double().view(B, H, W, C).permute(0, 3, 1, 2)
+    pre = F.conv2d(xin, w.double(), b.double(), padding=1)
+    rows = lambda t: t.permute(0, 2, 3, 1).reshape(-1, t.shape[1])
+    res = torch.randn(B * H * W, C, generator=g).to(torch.bfloat16)
+    for compact in (False, True):
+        assert torch.allclose(R.conv3x3(x, B, H, W, C, pw, act="lrelu", slope=0.2, compact=compact), rows(F.leaky_relu(pre, 0.2)),
+                              rtol=0, atol=1e-12)
+    assert torch.allclose(R.conv3x3(x, B, H, W, C, pw, alpha=0.5, res=res), rows(0.5 * pre) + res.double(),
+                          rtol=0, atol=1e-12)
+    assert torch.allclose(R.conv3x3(x, B, H, W, C, pw, ps=True), rows(F.pixel_shuffle(pre, 2)), rtol=0, atol=1e-12)
+    s2 = F.conv2d(xin, w.double(), b.double(), stride=2, padding=1)
+    assert torch.allclose(R.conv3x3(x, B, H, W, C, pw, stride=2), rows(s2), rtol=0, atol=1e-12)
+    assert torch.allclose(R.conv_pre(xin, w, b, 2, noise=True).double(), s2, rtol=0, atol=1e-4)
+    xs = torch.randn(B, 3, H, W, generator=g)
+    ws, bs = torch.randn(20, 3, 3, 3, generator=g), torch.randn(20, generator=g)
+    assert torch.allclose(R.conv3x3_small(xs, ws, bs), rows(F.conv2d(xs.double(), ws.double(), bs.double(), padding=1)), rtol=0, atol=1e-12)
+    # the CA chain: AdaptiveAvgPool2d(1) -> 1x1 conv -> ReLU -> 1x1 conv -> sigmoid, then x + t2 * s
+    t2 = torch.randn(B * H * W, C, generator=g).to(torch.bfloat16)
+    mlp = (torch.randn(2, C, generator=g), torch.randn(2, generator=g), torch.randn(C, 2, generator=g), torch.randn(C, generator=g))
+    t2n = t2.double().view(B, H, W, C).permute(0, 3, 1, 2)
+    d = [m.double() for m in mlp]
+    s = torch.sigmoid(F.conv2d(F.relu(F.conv2d(F.adaptive_avg_pool2d(t2n, 1), d[0][:, :, None, None], d[1])), d[2][:, :, None, None], d[3]))
+    parts = t2.float().view(B, 4, H * W // 4, C).sum(2).reshape(B * 4, C)
+    assert torch.allclose(R.channel_mean(t2, B, H * W, C), t2n.mean((2, 3)), rtol=0, atol=1e-12)
+    assert torch.allclose(R.channel_mean_parts(parts, B, 4, C, H * W, mlp), s.view(B, C), rtol=0, atol=1e-6)
+    assert torch.allclose(R.rcab_ca_scale(t2, x, s.view(B, C), B, H * W, C), rows(xin + t2n * s), rtol=0, atol=1e-12)
+
+
+# The GPU conv cases of tests/test_gpu_gemm.py (shape, seed, epilogue) that carry a conv defect.
+CONV_CASES = {
+    "before_upsample": dict(B=2, H=32, W=32, Cin=180, Cout=64, seed=2, act="lrelu", slope=0.01),
+    "downblock": dict(B=2, H=33, W=17, Cin=80, Cout=80, seed=33, act="lrelu", slope=0.2, stride=2),
+    "tail_panel": dict(B=5, H=17, W=24, Cin=72, Cout=48, seed=72, act="lrelu", slope=0.1),
+    "second_panel": dict(B=2, H=16, W=40, Cin=100, Cout=48, seed=100),
+    "pixel_shuffle": dict(B=2, H=32, W=32, Cin=64, Cout=256, seed=3, ps=True),
+    "res_lrelu": dict(B=2, H=24, W=24, Cin=64, Cout=64, seed=24, act="lrelu", slope=0.2, res=True),
+}
+
+
+def _conv_ref(case, kw, *, w=None, bias=None, xin=None, pre=None, mutate_pre=None, **over):
+    kw = dict(kw, **over)
+    B, H, W, cin, stride = kw["B"], kw["H"], kw["W"], kw["Cin"], kw.get("stride", 1)
+    if pre is None:
+        w = R.unpack_conv(case["pw"]) if w is None else w
+        bias = case["pw"].bias[:kw["Cout"]] if bias is None else bias
+        pre = R.conv_pre(R.conv_input(case["x"], B, H, W, cin) if xin is None else xin, w, bias, stride)
+    if mutate_pre is not None:
+        pre = mutate_pre(pre)
+    return R.conv_epilogue(pre, act=kw.get("act", "none"), slope=kw.get("slope", 0.0), res=case["res"], ps=kw.get("ps", False))
+
+
+def _conv_defect(case, kw, defect):
+    B, H, W, cin = kw["B"], kw["H"], kw["W"], kw["Cin"]
+    w, xin = R.unpack_conv(case["pw"]), R.conv_input(case["x"], B, H, W, cin)
+    if defect == "ReLU for LeakyReLU":
+        return _conv_ref(case, kw, act="relu")
+    if defect == "slope 0.2 -> 0.22":
+        return _conv_ref(case, kw, slope=0.22)
+    if defect == "tap dropped on the last column":
+        w2 = w.clone()
+        w2[:, :, 1, 0] = 0.0                                      # the left neighbour: inside the image
+        drop = R.conv_pre(xin, w2, case["pw"].bias[:kw["Cout"]], kw.get("stride", 1))
+
+        def m(pre):
+            pre = pre.clone()
+            pre[..., -1] = drop[..., -1]
+            return pre
+        return _conv_ref(case, kw, mutate_pre=m)
+    if defect == "replicate padding on the left border":
+        xp = F.pad(xin, (1, 1, 1, 1))
+        xp[..., 1:-1, 0] = xp[..., 1:-1, 1]
+        pre = F.conv2d(xp, w, case["pw"].bias[:kw["Cout"]].double(), stride=kw.get("stride", 1))
+        return _conv_ref(case, kw, pre=pre)
+    if defect == "tail panel dropped for one tap":
+        w2 = w.clone()
+        w2[:, 64:80, 0, 0] = 0.0
+        return _conv_ref(case, kw, w=w2)
+    if defect == "last channel of the second panel dropped":
+        w2 = w.clone()
+        w2[:, cin - 1] = 0.0
+        return _conv_ref(case, kw, w=w2)
+    if defect == "bias missing on one channel":
+        b = case["pw"].bias[:kw["Cout"]].clone()
+        b[-1] = 0.0
+        return _conv_ref(case, kw, bias=b)
+    if defect == "pixel-shuffle sub-pixels transposed":
+        n = kw["Cout"]
+        perm = torch.arange(n).view(n // 4, 2, 2).transpose(1, 2).reshape(-1)
+        return _conv_ref(case, kw, mutate_pre=lambda pre: pre[:, perm])
+    if defect == "stride-2 phase off by one":
+        pre = F.conv2d(F.pad(xin, (0, 1, 0, 1)), w, case["pw"].bias[:kw["Cout"]].double(), padding=1)[..., 1::2, 1::2]
+        return _conv_ref(case, kw, pre=pre)
+    if defect == "residual added before the activation":
+        pre = R.conv_pre(xin, w, case["pw"].bias[:kw["Cout"]])
+        r = case["res"][:, :kw["Cout"]].double().view(B, H, W, -1).permute(0, 3, 1, 2)
+        return R.conv_epilogue(pre + r, act=kw["act"], slope=kw["slope"])
+    raise KeyError(defect)
+
+
+CONV_TABLE = [
+    ("before_upsample", "ReLU for LeakyReLU"), ("before_upsample", "bias missing on one channel"),
+    ("before_upsample", "tap dropped on the last column"), ("before_upsample", "replicate padding on the left border"),
+    ("downblock", "slope 0.2 -> 0.22"), ("downblock", "stride-2 phase off by one"), ("downblock", "tap dropped on the last column"),
+    ("tail_panel", "tail panel dropped for one tap"), ("tail_panel", "replicate padding on the left border"),
+    ("second_panel", "last channel of the second panel dropped"), ("pixel_shuffle", "pixel-shuffle sub-pixels transposed"),
+    ("res_lrelu", "residual added before the activation"), ("res_lrelu", "slope 0.2 -> 0.22"),
+]
+
+
+def _conv_case(which):
+    kw = CONV_CASES[which]
+    case = R.conv_case(kw["B"], kw["H"], kw["W"], kw["Cin"], kw["Cout"], kw["seed"], res=kw.get("res", False))
+    return case, kw
+
+
+def _conv_shortcut(case, kw):
+    return None if case["res"] is None else case["res"][:, :kw["Cout"]]
+
+
+@pytest.mark.parametrize("which,defect", CONV_TABLE)
+def test_conv_defect_fails(which, defect):
+    case, kw = _conv_case(which)
+    ref = _conv_ref(case, kw)
+    v = _verdict(_conv_defect(case, kw, defect), ref, _conv_shortcut(case, kw), "conv")
+    assert not v.ok, f"{which}: '{defect}' passes the comparator: {v}"
+
+
+def test_relu_for_leaky_relu_passed_the_old_bound():
+    """At the conv_before_upsample shape the old bound (1.2 % of max|y|) took a ReLU for LeakyReLU(0.01)."""
+    case, kw = _conv_case("before_upsample")
+    ref, bad = _conv_ref(case, kw), R.bf16(_conv_defect(case, kw, "ReLU for LeakyReLU"))
+    assert float((bad - ref).abs().max() / ref.abs().max()) < 0.012
+    assert not _verdict(bad, ref, None, "conv").ok
+
+
+@pytest.mark.parametrize("which", list(CONV_CASES))
+def test_conv_kernel_noise_passes(which):
+    case, kw = _conv_case(which)
+    args = (case["x"], kw["B"], kw["H"], kw["W"], kw["Cin"], case["pw"])
+    ep = dict(stride=kw.get("stride", 1), act=kw.get("act", "none"), slope=kw.get("slope", 0.0), res=case["res"], ps=kw.get("ps", False))
+    got = R.bf16(R.conv3x3(*args, noise=True, **ep).double())
+    v = _verdict(got, R.conv3x3(*args, **ep), _conv_shortcut(case, kw), "conv")
+    assert v.ok, f"{which}: simulated kernel noise fails: {v}"
+
+
+RCAB_CASES = {"halo_64": (4, 64, 64, 40), "halo_32": (4, 32, 32, 80), "fallback_128": (2, 128, 128, 40)}
+
+
+def _rcab(which, **kw):
+    B, H, W, C = RCAB_CASES[which]
+    case = R.rcab_case(B, H, W, C, H + C)
+    return case, R.rcab(case["x"], B, H, W, case["c1"], case["c2"], case["mlp"], **kw)
+
+
+@pytest.mark.parametrize("which,defect", [(w, d) for w in RCAB_CASES for d in ("neighbour's scales", "sigmoid dropped")]
+                         + [("halo_64", "pad columns pooled"), ("halo_32", "pad columns pooled")])
+def test_rcab_defect_fails(which, defect):
+    B, H, W, C = RCAB_CASES[which]
+    case, ref = _rcab(which)
+    mlp = case["mlp"]
+    kw = {"neighbour's scales": dict(scale_fn=lambda m: R.ca_scale(m, *mlp).roll(1, 0)),
+          "sigmoid dropped": dict(scale_fn=lambda m: torch.logit(R.ca_scale(m, *mlp))),
+          "pad columns pooled": dict(pool_hw=H * (W + 2))}[defect]
+    _, got = _rcab(which, **kw)
+    v = _verdict(got, ref, case["x"][:, :C], "rcab")
+    assert not v.ok, f"{which}: '{defect}' passes the comparator: {v}"
+
+
+@pytest.mark.parametrize("which", list(RCAB_CASES))
+def test_rcab_kernel_noise_passes(which):
+    case, ref = _rcab(which)
+    _, got = _rcab(which, noise=True)
+    v = _verdict(R.bf16(got), ref, case["x"][:, :RCAB_CASES[which][3]], "rcab")
+    assert v.ok, f"{which}: simulated kernel noise fails: {v}"
